@@ -2,6 +2,7 @@
 """Benchmark of the B200 coherent-dedispersion hot path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload cfg2]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the fused hot path over one block of synthetic baseband:
   cfg2: DualPolarizationSignal (2^22 samples, 64 channels, 2 pol) complex64, 400-800 MHz,
@@ -21,6 +22,13 @@ oracle (scipy.fft restatement of the reference) on this box's host cores on a bo
 with the astropy/dask stand-ins of oracle/ref_shim -- those packages are not installable here),
 per channel chunk on a thread pool; if no copy of the reference is present it times the oracle
 port and says so (`cpu_baseline.kind`).
+
+`--dump-outputs DIR` (B200 arm) writes, after the timed steps, what the last timed step computed
+(rank 0's block): the array a caller of the timed path receives, as DIR/voltages.npy,
+DIR/intensity.npy or DIR/stokes_i.npy in float32, complex values with a trailing (re, im) axis.
+The inputs are seeded, so two builds run with the same arguments can be compared output for
+output.  A result above 64 MiB is cut to a fixed, seeded sample of its rows (time samples), whose
+row numbers go to DIR/<name>_rows.npy.
 """
 
 import argparse
@@ -104,6 +112,42 @@ def peaks():
         with open(p) as f:
             return float(json.load(f)["hbm_gbs"]), "measured (MEASURED_PEAKS.json hbm_gbs)"
     return 6650.0, "fallback (B200_PROFILING.md)"
+
+
+DUMP_BYTES = 64 << 20      # --dump-outputs writes at most this much
+
+
+def out_name(w):
+    return {None: "voltages", False: "intensity", True: "stokes_i"}[w["stokes"]]
+
+
+def dump_outputs(dirname, name, y, seed=8):
+    """Write the result ``y`` (numpy array or torch tensor, time samples first) as
+    ``dirname/<name>.npy`` in float32 / float64, complex values as a trailing (re, im) axis.
+    Above DUMP_BYTES only a fixed, seeded sample of its rows is written, and their row numbers
+    (as float64) to ``<name>_rows.npy``."""
+    os.makedirs(dirname, exist_ok=True)
+    is_np = isinstance(y, np.ndarray)
+    n = y.shape[0]
+    itemsize = y.itemsize if is_np else y.element_size()
+    row_bytes = max(1, itemsize * int(np.prod(y.shape[1:])))
+    rows = None
+    if n * row_bytes > DUMP_BYTES:
+        keep = DUMP_BYTES // (row_bytes + 8)
+        rows = np.sort(np.random.default_rng(seed).choice(n, keep, replace=False))
+        if is_np:
+            y = y[rows]
+        else:
+            import torch
+            y = y[torch.as_tensor(rows, device=y.device)]
+    a = y if is_np else y.cpu().numpy()
+    if np.iscomplexobj(a):
+        a = np.stack([a.real, a.imag], axis=-1)
+    if a.dtype not in (np.float32, np.float64):
+        a = a.astype(np.float64)
+    np.save(os.path.join(dirname, name + ".npy"), a)
+    if rows is not None:
+        np.save(os.path.join(dirname, name + "_rows.npy"), rows.astype(np.float64))
 
 
 def chan_freqs(w):
@@ -405,6 +449,11 @@ def run_b200(args, w):
     t_begin = time.perf_counter()
     ms_local = k_steps()
     t_end = time.perf_counter()
+    if args.dump_outputs and rank == 0:
+        # the last timed step's result as the caller sees it: (rows, channels[, pols])
+        odt = torch.complex64 if out_kind == L.OUT_C64 else torch.float32
+        oshape = (plan.out_rows, C) if out_kind == L.OUT_STOKES_I else (plan.out_rows, C, P)
+        dump_outputs(args.dump_outputs, out_name(w), out[:out_bytes].view(odt).reshape(oshape))
     ms_total = max_over_ranks(ms_local)
     # per-launch durations for the roofline: the same K steps once more with a CUDA event between
     # the launches (plan.profile) -- an event between two kernels serialises them, so this pass
@@ -961,7 +1010,12 @@ def main():
                     help="run the sharded-workload extras (cfg4 fold + all-reduce, cfg3 / cfg5 "
                          "shards) also at N = 1; they always run at N > 1")
     ap.add_argument("--no-extras", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        # the reference arm sizes its block by a timed calibration, so its input is not fixed
+        ap.error("--dump-outputs needs --impl b200")
     claim_stdout()
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     w = WORKLOADS[args.workload]

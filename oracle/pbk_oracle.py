@@ -14,14 +14,13 @@ here 1.18.1) and numpy ufuncs -- which ARE available, so the oracle calls exactl
 the reference's argument order.  astropy's contribution to the numbers on this path reduces
 to the constant 1/2.41e-4, powers of ten between Hz and MHz, and cycle->rad = 2*pi.
 
-Pinning, part 1 (tests/test_ref_golden.py): OUTPUTS OF THE REFERENCE ITSELF.  The hot-path source
-files of /root/reference are executed here, unmodified and where they lie, by oracle/ref_run.py
-(unit bookkeeping on the stand-ins of oracle/ref_shim, since astropy/dask cannot be installed);
+Pinning, part 1 (tests/test_ref_golden.py): OUTPUTS OF THE REFERENCE ITSELF.  The reference's
+hot-path source files were executed, unmodified and where they lie, by oracle/ref_run.py (unit
+bookkeeping on the stand-ins of oracle/ref_shim, since astropy/dask cannot be installed);
 oracle/make_ref_golden.py froze their outputs for seeded inputs into tests/golden/ref_golden.npz
 (coherent dedispersion in seven geometries, the chirp at BASELINE sizes, the crops of configs
 1/2/3/5, stft/istft, intensity/Stokes/pol basis, time_shift, freq_shift, incoherent
-dedispersion, real_to_complex).  This oracle reproduces all of them, and the live re-run is
-compared with the frozen file bit for bit whenever /root/reference is present.
+dedispersion, real_to_complex).  This oracle reproduces all of them.
 
 Pinning, part 2 (tests/test_oracle_*.py): every known-answer test the reference holds for the
 path is reproduced against this oracle --

@@ -14,10 +14,9 @@ and ``isinstance`` checks, so this loader
   ``phase.py`` needs astropy's Angle machinery; the predictor only hands ``pb.Phase`` the two
   parts it computed, so a two-field record stands in).
 
-Nothing is copied; /root/reference is read, never written.  Used by oracle/make_ref_golden.py to
-freeze reference outputs into tests/golden/ref_golden.npz, and by tests/test_ref_golden.py to
-compare the oracle restatement with the live reference whenever /root/reference is present (it
-is absent on the GPU box, where the frozen vectors stand in)."""
+Nothing is copied; the reference is read, never written.  Used by oracle/make_ref_golden.py to
+freeze reference outputs into tests/golden/ref_golden.npz, and by ``bench.py --impl reference``;
+the tests compare with the frozen vectors only."""
 
 import importlib
 import os

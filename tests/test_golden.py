@@ -1,20 +1,35 @@
 """Frozen vectors (tests/golden/golden_small.npz, written by tests/golden/make_golden.py): the
-oracle must keep reproducing them (CPU), and the CUDA path must match them (GPU)."""
+oracle must keep reproducing them (CPU), and the CUDA path must match them (GPU).  The seeded
+inputs are drawn again by make_golden.inputs() and must match the digests kept in the file."""
 
+import importlib.util
+import json
 import os
 
 import numpy as np
 import pytest
 
 from oracle import pbk_oracle as orc
+from oracle.make_ref_golden import digest
 
-G = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "golden_small.npz"))
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+_spec = importlib.util.spec_from_file_location("make_golden",
+                                               os.path.join(GOLDEN, "make_golden.py"))
+make_golden = importlib.util.module_from_spec(_spec)
+_spec.loader.exec_module(make_golden)
+G = dict(np.load(os.path.join(GOLDEN, "golden_small.npz")))
+G.update(make_golden.inputs())
 
 
 def relerr(a, b):
     a = np.asarray(a).astype(np.complex128 if np.iscomplexobj(a) else np.float64)
     b = np.asarray(b).astype(a.dtype).reshape(a.shape)
     return np.linalg.norm((a - b).ravel()) / np.linalg.norm(b.ravel())
+
+
+def test_regenerated_inputs_match_the_frozen_digests():
+    want = json.loads(str(G["digests_json"]))
+    assert {k: digest(a) for k, a in make_golden.inputs().items()} == want
 
 
 def test_oracle_reproduces_golden():

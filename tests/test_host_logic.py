@@ -198,3 +198,31 @@ def test_bench_reference_arm_prints_exactly_one_json_line():
     assert line["impl"] == "reference" and line["unit"] == "Gsamples/s" and line["value"] > 0
     assert line["cpu_baseline"]["kind"] in ("reference", "port")
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["e2e"]["d2h_bytes_per_step"] == 0
+
+
+def test_bench_dump_outputs_format_and_size_limit(tmp_path, monkeypatch):
+    # --dump-outputs: float32 / float64 arrays, complex as a trailing (re, im) axis; above the
+    # size limit a fixed, seeded sample of rows with their row numbers, the same on every call
+    import subprocess
+    import sys
+
+    import torch
+
+    import bench
+    y = (np.arange(24000, dtype=np.float32).reshape(4000, 3, 2) * (1 + 2j)).astype(np.complex64)
+    bench.dump_outputs(str(tmp_path / "full"), "voltages", y)
+    v = np.load(tmp_path / "full" / "voltages.npy")
+    assert v.dtype == np.float32 and np.array_equal(v[..., 0] + 1j * v[..., 1], y)
+    assert not (tmp_path / "full" / "voltages_rows.npy").exists()
+    monkeypatch.setattr(bench, "DUMP_BYTES", 1 << 14)
+    for sub, arr in (("a", y), ("b", torch.from_numpy(y))):
+        bench.dump_outputs(str(tmp_path / sub), "voltages", arr)
+    va, ra = np.load(tmp_path / "a" / "voltages.npy"), np.load(tmp_path / "a" / "voltages_rows.npy")
+    assert va.nbytes + ra.nbytes <= 1 << 14 and ra.dtype == np.float64
+    assert np.array_equal(va[..., 0] + 1j * va[..., 1], y[ra.astype(np.int64)])
+    assert np.array_equal(va, np.load(tmp_path / "b" / "voltages.npy"))
+    assert np.array_equal(ra, np.load(tmp_path / "b" / "voltages_rows.npy"))
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference",
+                        "--dump-outputs", str(tmp_path / "ref")], capture_output=True, text=True,
+                       timeout=120, cwd=ROOT)
+    assert r.returncode != 0 and "--dump-outputs needs --impl b200" in r.stderr
