@@ -155,10 +155,12 @@ int pbk_fft_plan_create(int64_t outer, int64_t n, int64_t inner, int32_t inverse
  *   inverse:  in (nseg, nchan_out*nperseg, npol) -> out (nseg*nperseg, nchan_out, npol)
  * Any nperseg >= 2 (the reference's tests use 33).  The input is never modified (the reference's
  * istft scales its input in place, misc.py:82-83).  A forward plan for ONE single-polarisation
- * channel with a power-of-two nperseg >= 2^14 is built on the (nperseg/2, 2) even / odd view of the
- * stream and recombined in the last pass (pbk_plan_describe shows ":evenodd"; PBK_NO_SPLIT=1
+ * channel whose nperseg is a power of two with a two-level half-length plan (2^14 .. 2^22 and
+ * possibly longer; 2 .. 2^13 have a one-level half) is built on the (nperseg/2, 2) even / odd view
+ * of the stream and recombined in the last pass (pbk_plan_describe shows ":evenodd"; PBK_NO_SPLIT=1
  * disables it) -- same input, same output, the compile-time-shaped kernels instead of the
- * run-time-shaped ones.
+ * run-time-shaped ones.  Every other nperseg runs the full-length plan (Bluestein when it is not a
+ * power of two).
  */
 int pbk_stft_plan_create(int64_t nseg, int64_t nperseg, int64_t nchan, int64_t npol,
                          int32_t inverse, int32_t device, pbk_plan** plan);
@@ -172,8 +174,11 @@ int pbk_stft_plan_create(int64_t nseg, int64_t nperseg, int64_t nchan, int64_t n
  *       (nseg, nperseg/freq_sum)       float32   out_kind STOKES_I (npol 2)
  * with out[s, c', p] = sum_{f < freq_sum} |stft(in)[s, c'*freq_sum + f, p]|^2, fftshift and 1/n
  * scale of the reference's stft included.  One channel only, a power-of-two segment length that
- * the plan splits into two levels (2^13 .. 2^24) and a power-of-two freq_sum that divides the first
- * level; other shapes return PBK_ERR_UNSUPPORTED (use pbk_stft_plan_create + pbk_detect_scrunch).
+ * the plan splits into two levels (of the lengths tested: npol 2 from 2^13 to 2^20, npol 1 --
+ * planned at half length -- from 2^14 to 2^22; not 2^22 with npol 2, not 2^24) and a power-of-two
+ * freq_sum that divides the first level in whole
+ * last-pass tiles; other shapes, any length that is not a power of two among them, return
+ * PBK_ERR_UNSUPPORTED (use pbk_stft_plan_create + pbk_detect_scrunch).
  * Executed with pbk_fft_exec_device / pbk_fft_exec_host. */
 int pbk_stft_detect_plan_create(int64_t nseg, int64_t nperseg, int64_t nchan, int64_t npol,
                                 int32_t out_kind, int64_t freq_sum, int32_t device,

@@ -1334,6 +1334,11 @@ static int build_fft_plan(long long O, long long n, long long C, long long P, bo
   const int ln = ilog2_exact(n);
   if (ln < 1) {
     if (n < 2) return fail(PBK_ERR_UNSUPPORTED, "transform length %lld is too short", (long long)n);
+    // the even / odd recombination and the detecting epilogue live in the last tile pass: the
+    // Bluestein plan has neither, so the caller takes its plain path
+    if (det)
+      return fail(PBK_ERR_UNSUPPORTED, "length %lld is not a power of two: no even / odd or "
+                  "detecting last pass", (long long)n);
     // not a power of two: Bluestein on top of the power-of-two passes (pbk_blue.cuh)
     return blue_fft_plan_create(O, n, C, P, inverse, in, outm, scale, shift_out, shift_in, device,
                                 out, in_kind);
@@ -1736,10 +1741,13 @@ static int stft_plan_create(int64_t nseg, int64_t nperseg, int64_t nchan, int64_
     return fail(PBK_ERR_INVALID, "packed input needs an even nchan * npol, got %lld",
                 (long long)(nchan * npol));
   const long long n = nperseg, C = nchan, P = npol;
-  if (!inverse && in_dtype == PBK_C64 && C == 1 && P == 1 && n % 2 == 0 && !getenv("PBK_NO_SPLIT")) {
+  if (!inverse && in_dtype == PBK_C64 && C == 1 && P == 1 && n % 2 == 0 &&
+      ilog2_exact(n / 2) >= 1 && !getenv("PBK_NO_SPLIT")) {
     // one single-pol column has no lane pair; its even and odd samples do (see
     // pbk_stft_detect_plan_create): half-length plan on the (n/2, 2) view, recombined in the
-    // last pass.  Shapes it does not cover fall through to the plan below (generic kernels).
+    // last pass.  Only power-of-two halves have that last pass (a Bluestein plan would return
+    // the two half-length spectra unrecombined).  Shapes it does not cover fall through to the
+    // plan below (generic kernels).
     DetectSpec det;
     det.split = det.volt = true;
     const long long h = n / 2;
