@@ -116,6 +116,27 @@ int pbk_dedisp_out_shape(const pbk_plan* plan, int64_t* rows, int64_t* row_elems
 int pbk_dedisp_exec_host(pbk_plan* plan, const void* in, void* out, const void* chirp);
 int pbk_dedisp_exec_device(pbk_plan* plan, const void* d_in, void* d_out, const void* d_chirp,
                            void* stream);
+/* coherent dedispersion -> detection -> time sum -> fold (row F) as one execution of a dedispersion
+ * plan whose out_kind is INTENSITY or STOKES_I (and no explicit chirp): the time-summed power of
+ * output row j is ADDED to profile[bin(j), :] (float32 (nbin, row_elems), caller-zeroed or carrying
+ * earlier blocks) and counts[bin(j)] += 1 (int64 (nbin,)), bin(j) from the phase polynomial at
+ * t = (n0 + j) / sample_rate_hz exactly as pbk_fold, where sample_rate_hz is the OUTPUT-ROW rate
+ * (input rate / downsample).  Device pointers, enqueued on `stream`; nothing is written to a
+ * voltage or intensity array of the caller.
+ * When the plan sums time in the epilogue of its last inverse pass (pbk_plan_describe shows
+ * ":timesum"), the intensity (out_rows x row_elems floats) is at least 256 MiB and there are at
+ * most 512 rows per bin, the bins are computed first and that pass adds its group sums straight
+ * into the profile, so the intensity never reaches HBM; otherwise (smaller intensities stay in L2
+ * between two steps, and many rows per bin serialise the atomics) the plan's normal execution
+ * writes a plan-owned float32 buffer of out_rows x row_elems (allocated at the first such
+ * execution and counted in pbk_plan_info's workspace bytes), which is then folded.  Bins and counts are exact on both
+ * routes; the fused profile collects many float atomics per row in any order, so it is
+ * reproducible to rounding, not bit for bit.  ncoef in [1, 16], finite coefficients, finite
+ * sample_rate_hz > 0, nbin > 0; a C64 plan returns PBK_ERR_INVALID; an empty crop returns PBK_OK
+ * and touches nothing.  A later pbk_dedisp_exec_device of the same plan is unaffected. */
+int pbk_dedisp_fold_exec_device(pbk_plan* plan, const void* d_in, void* d_profile, void* d_counts,
+                                const double* coeffs, int32_t ncoef, double sample_rate_hz,
+                                int64_t n0, int32_t nbin, void* stream);
 
 /* ---- FFT-domain phase ramp / band mask ("next" rows: time_shift, freq_shift) ------------------
  * Replaces the core of transforms/transforms.py:268-271 (time_shift) and :348-361 (freq_shift):

@@ -17,7 +17,7 @@ EXPORTS = [
     "pbk_version", "pbk_last_error", "pbk_status_string", "pbk_device_count",
     "pbk_device_pci_bus_id", "pbk_device_mem_info", "pbk_phase_predict",
     "pbk_dedisp_plan_create", "pbk_dedisp_out_shape", "pbk_dedisp_exec_host",
-    "pbk_dedisp_exec_device", "pbk_fft_plan_create", "pbk_stft_plan_create", "pbk_stft_plan_create_raw",
+    "pbk_dedisp_exec_device", "pbk_dedisp_fold_exec_device", "pbk_fft_plan_create", "pbk_stft_plan_create", "pbk_stft_plan_create_raw",
     "pbk_stft_detect_plan_create", "pbk_stft_fold_exec_device",
     "pbk_dedisp_c128", "pbk_fft_c128", "pbk_stft_c128", "pbk_detect_c128",
     "pbk_fft_exec_host", "pbk_fft_exec_device", "pbk_detect", "pbk_detect_scrunch", "pbk_shift_channels", "pbk_downsample", "pbk_fold",
@@ -84,6 +84,8 @@ def lib():
         L.pbk_dedisp_out_shape.argtypes = [vp] + [ctypes.POINTER(i64)] * 3
         L.pbk_dedisp_exec_host.argtypes = [vp, vp, vp, vp]
         L.pbk_dedisp_exec_device.argtypes = [vp, vp, vp, vp, vp]
+        L.pbk_dedisp_fold_exec_device.argtypes = [vp, vp, vp, vp, ctypes.POINTER(dbl), i32, dbl,
+                                                  i64, i32, vp]
         L.pbk_fft_plan_create.argtypes = [i64, i64, i64, i32, i32, ctypes.POINTER(vp)]
         L.pbk_stft_plan_create.argtypes = [i64, i64, i64, i64, i32, i32, ctypes.POINTER(vp)]
         L.pbk_stft_plan_create_raw.argtypes = [i64, i64, i64, i64, i32, i32, ctypes.POINTER(vp)]
@@ -255,6 +257,15 @@ class DedispPlan(Plan):
     def exec_device(self, d_in, d_out, d_chirp=None, stream=0):
         check(lib().pbk_dedisp_exec_device(self.handle, ptr(d_in), ptr(d_out), ptr(d_chirp),
                                            ctypes.c_void_p(stream)))
+
+    def fold_device(self, d_in, d_profile, d_counts, coeffs, sample_rate_hz, n0, nbin, stream=0):
+        """Dedisperse, detect, time-sum and fold one block (pbk_dedisp_fold_exec_device);
+        ``sample_rate_hz`` is the output-row rate."""
+        c = np.ascontiguousarray(coeffs, dtype=np.float64)
+        check(lib().pbk_dedisp_fold_exec_device(
+            self.handle, ptr(d_in), ptr(d_profile), ptr(d_counts),
+            c.ctypes.data_as(ctypes.POINTER(ctypes.c_double)), len(c), float(sample_rate_hz),
+            int(n0), int(nbin), ctypes.c_void_p(stream)))
 
 
 class RampPlan(Plan):

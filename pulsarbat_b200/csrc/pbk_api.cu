@@ -144,8 +144,11 @@ struct pbk_plan {
   // channelizer plans with a detected output (pbk_stft_detect_plan_create)
   long long det_nseg = 0, det_cells = 0;
   int det_pq = 0;
-  int* d_segbins = nullptr;          // phase bin per segment of the current folded execution
-  const int* exec_segbins = nullptr; // non-null while pbk_stft_fold_exec_device runs the passes
+  int* d_segbins = nullptr;          // phase bin per segment (channelizer) or output row
+                                     // (dedispersion) of the current folded execution
+  const int* exec_segbins = nullptr; // non-null while a fold execution runs the passes
+  void* d_foldbuf = nullptr;         // dedispersion fold on the unfused route: the plan's output
+  size_t fold_bytes = 0;             // lazily allocated d_segbins + d_foldbuf of a dedispersion plan
   bool split_column = false;    // single column run as its even / odd samples (see plan creation)
   bool split_ragged = false;    // ... with an odd crop edge: passes write d_tmpf, then a D2D copy
   size_t split_skip = 0;
@@ -1141,6 +1144,7 @@ static int launch_one(pbk_plan* pl, const Pass& ps, const void* d_in, void* d_ou
   p.a.chirp_arr = reinterpret_cast<const float2*>(d_chirp);
   p.a.tile0 = tile0;
   if (p.a.fsum_log2 > 0) p.a.fsum_bins = pl->exec_segbins;
+  if (p.a.tsum_log2 > 0) p.a.tsum_bins = pl->exec_segbins;
   const bool aligned = (((uintptr_t)p.a.in | (uintptr_t)p.a.out) & 15) == 0;
   cudaError_t e;
   CUtensorMap tm;
@@ -1281,6 +1285,79 @@ extern "C" int pbk_dedisp_exec_device(pbk_plan* pl, const void* d_in, void* d_ou
 static int ensure_buf(void** p, size_t bytes) {
   if (*p || bytes == 0) return PBK_OK;
   CUDA_TRY(cudaMalloc(p, bytes));
+  return PBK_OK;
+}
+
+// Coherent dedispersion -> detection -> time sum -> fold.  Fused route (the time sum runs in the
+// epilogue of the last inverse pass, large intermediate, few rows per bin): the phase bin of every
+// output row is computed first, and the last pass adds its group sums to profile[bin] instead of
+// out[row], so the intensity never reaches HBM.  Otherwise the plan's normal execution writes a
+// plan-owned buffer and pbk_fold's kernel folds it.
+extern "C" int pbk_dedisp_fold_exec_device(pbk_plan* pl, const void* d_in, void* d_profile,
+                                           void* d_counts, const double* coeffs, int32_t ncoef,
+                                           double sample_rate_hz, int64_t n0, int32_t nbin,
+                                           void* stream) {
+  if (!pl || pl->kind != PLAN_DEDISP) return fail(PBK_ERR_INVALID, "not a dedispersion plan");
+  if (pl->desc.out_kind != PBK_OUT_INTENSITY && pl->desc.out_kind != PBK_OUT_STOKES_I)
+    return fail(PBK_ERR_INVALID, "folding needs a plan with out_kind INTENSITY or STOKES_I");
+  if (pl->desc.explicit_chirp) return fail(PBK_ERR_INVALID, "folding takes no explicit chirp");
+  if (!d_in || !d_profile || !d_counts || !coeffs) return fail(PBK_ERR_INVALID, "NULL pointer");
+  if (nbin <= 0) return fail(PBK_ERR_INVALID, "nbin must be positive");
+  if (ncoef < 1 || ncoef > kFoldMaxCoef)
+    return fail(PBK_ERR_INVALID, "ncoef must be in [1, %d]", kFoldMaxCoef);
+  if (!(sample_rate_hz > 0) || !std::isfinite(sample_rate_hz))
+    return fail(PBK_ERR_INVALID, "sample_rate_hz must be finite and > 0");
+  for (int i = 0; i < ncoef; ++i)
+    if (!std::isfinite(coeffs[i]))
+      return fail(PBK_ERR_INVALID, "phase coefficient %d is not finite", i);
+  if (pl->out_rows == 0) return PBK_OK;   // empty crop: nothing to fold
+  CUDA_TRY(cudaSetDevice(pl->device));
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  FoldArgs fa;
+  memset(&fa, 0, sizeof(fa));
+  for (int i = 0; i < ncoef; ++i) fa.coef[i] = coeffs[i];
+  fa.ncoef = ncoef;
+  fa.sample_rate = sample_rate_hz;
+  fa.n0 = n0;
+  fa.nbin = nbin;
+  fa.nsamp = pl->out_rows;
+  fa.row_elems = pl->row_elems;
+  fold_args_finish(fa);
+  fa.counts = reinterpret_cast<unsigned long long*>(d_counts);
+  // The fused route saves the intermediate's round trip, which only costs HBM traffic once it is
+  // well beyond the 126 MB L2, but it sends every group sum of a profile cell to the same address.
+  // MEASURED (B200 1000 W, cfg2 geometry, scripts/dedisp_fold_bw.py, profiles/r03_dedisp_fold.log):
+  // per-pol x8 / 1024 bins (256 MiB, 512 rows per bin) 0.987x the two steps, x4 (1024 rows per
+  // bin) 0.96x; Stokes I x4 (256 MiB, 1024 rows per bin) 1.017x, x64 (16 MiB) 1.005x, 16 bins up
+  // to 1.23x.  So: fused only for an intermediate of >= 256 MiB with <= 512 rows per bin.
+  const bool fuse = pl->fused_tsum &&
+                    (size_t)pl->out_rows * pl->row_elems * 4 >= ((size_t)256 << 20) &&
+                    pl->out_rows <= 512ll * nbin;
+  if (fuse) {
+    if (!pl->d_segbins) {
+      const size_t b = (size_t)pl->out_rows * sizeof(int);
+      CUDA_TRY(cudaMalloc(&pl->d_segbins, b));
+      pl->fold_bytes += b;
+    }
+    const unsigned blocks = (unsigned)std::min<long long>((pl->out_rows + 255) / 256, 148 * 4);
+    fold_bins_kernel<<<blocks, 256, 0, st>>>(fa, pl->d_segbins);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return fail(PBK_ERR_CUDA, "fold bins launch: %s", cudaGetErrorString(e));
+    pl->exec_segbins = pl->d_segbins;
+    const int rc = run_passes(pl, d_in, d_profile, nullptr, st);   // no memset: it accumulates
+    pl->exec_segbins = nullptr;
+    return rc;
+  }
+  if (!pl->d_foldbuf) {
+    CUDA_TRY(cudaMalloc(&pl->d_foldbuf, pl->out_bytes));
+    pl->fold_bytes += pl->out_bytes;
+  }
+  const int rc = pbk_dedisp_exec_device(pl, d_in, pl->d_foldbuf, nullptr, stream);
+  if (rc != PBK_OK) return rc;
+  fa.in = reinterpret_cast<const float*>(pl->d_foldbuf);
+  fa.profile = reinterpret_cast<float*>(d_profile);
+  cudaError_t e = launch_fold(fa, st);
+  if (e != cudaSuccess) return fail(PBK_ERR_CUDA, "fold launch: %s", cudaGetErrorString(e));
   return PBK_OK;
 }
 
@@ -1932,6 +2009,7 @@ extern "C" void pbk_plan_destroy(pbk_plan* pl) {
   cudaFree(pl->d_ramp_zero);
   cudaFree(pl->d_tmpf);
   cudaFree(pl->d_segbins);
+  cudaFree(pl->d_foldbuf);
   cudaFree(pl->d_l2sync);
   cudaFree(pl->h_din);
   cudaFree(pl->h_dout);
@@ -1944,7 +2022,7 @@ extern "C" int pbk_plan_info(const pbk_plan* pl, int32_t* launches, int64_t* wor
   if (!pl) return fail(PBK_ERR_INVALID, "plan is NULL");
   if (launches) *launches = pl->launches;
   if (workspace_bytes) *workspace_bytes =
-      (int64_t)(pl->scratch_bytes * (pl->scratch2 ? 2 : 1) + pl->tmpf_bytes);
+      (int64_t)(pl->scratch_bytes * (pl->scratch2 ? 2 : 1) + pl->tmpf_bytes + pl->fold_bytes);
   if (levels) *levels = pl->nlevels;
   if (level_log2)
     for (int i = 0; i < 3; ++i) level_log2[i] = pl->level_log2[i];

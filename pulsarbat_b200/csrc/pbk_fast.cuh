@@ -619,7 +619,16 @@ __device__ __forceinline__ void inv_last_sum(const FastTile& T, float4* tile, co
 // time n = (r << log2nmul) + nrest and lands in output row (n - crop_start) >> tsum_log2.  A group
 // receives at most two contributions (a CTA's run of tiles is at least two groups long and run
 // boundaries avoid the groups that straddle the wrap of the inner offset), so the float atomics
-// give the same result in either order.
+// give the same result in either order.  With p.tsum_bins (the fold) the row is tsum_bins[row] and
+// a profile row collects the groups of every row in its phase bin in any order: reproducible to
+// rounding, not bit for bit.  Only sums of rows inside the crop are non-zero, so the bin array is
+// read for rows [0, out_rows) only.
+__device__ __forceinline__ char* tsum_row(const PassArgs& p, char* colbase, long long n,
+                                          long long out_row_bytes) {
+  const long long row = (n - p.crop_start) >> p.tsum_log2;
+  return colbase + (p.tsum_bins ? (long long)p.tsum_bins[row] : row) * out_row_bytes;
+}
+
 template <class C, int EPI>
 __device__ __forceinline__ void tsum_flush(const PassArgs& p, TsumAcc<C, EPI>& acc, char* colbase,
                                            unsigned nrest, int tid, long long out_row_bytes) {
@@ -630,12 +639,16 @@ __device__ __forceinline__ void tsum_flush(const PassArgs& p, TsumAcc<C, EPI>& a
 #pragma unroll
     for (int i = 0; i < R; ++i) {
       const long long n = ((long long)(b + i * S) << p.log2nmul) + nrest;
-      char* a = colbase + ((n - p.crop_start) >> p.tsum_log2) * out_row_bytes;
       if constexpr (EPI == EPI_STOKES_I) {
-        if (acc.a[it][i] != 0.f) atomicAdd(reinterpret_cast<float*>(a), acc.a[it][i]);
+        if (acc.a[it][i] != 0.f)
+          atomicAdd(reinterpret_cast<float*>(tsum_row(p, colbase, n, out_row_bytes)), acc.a[it][i]);
       } else {
-        if (acc.a[it][i].x != 0.f) atomicAdd(reinterpret_cast<float*>(a), acc.a[it][i].x);
-        if (acc.a[it][i].y != 0.f) atomicAdd(reinterpret_cast<float*>(a) + 1, acc.a[it][i].y);
+        const float2 v = acc.a[it][i];
+        if (v.x != 0.f || v.y != 0.f) {
+          float* a = reinterpret_cast<float*>(tsum_row(p, colbase, n, out_row_bytes));
+          if (v.x != 0.f) atomicAdd(a, v.x);
+          if (v.y != 0.f) atomicAdd(a + 1, v.y);
+        }
       }
     }
   }

@@ -141,6 +141,8 @@ struct PassArgs {
   int tsum_log2;      // fast final INV pass: > 0 = sum 2^tsum_log2 consecutive time rows of the
                       // detected output in the epilogue (row R fused; see fast_pass_kernel TSUM)
   int tsum_q;         // ... with groups of tsum_q adjacent CTAs covering adjacent column groups
+  const int* tsum_bins;   // fold fused behind the time sum (pbk_dedisp_fold_exec_device): phase bin
+                          // of every output row; group sums are ADDED to out[bin] instead of out[row]
   // fast FWD-last pass of a channelizer plan with a DETECTED output (pbk_stft_detect_plan_create):
   // |z|^2 summed over 2^fsum_log2 adjacent fine channels in the epilogue, so the channelized
   // voltages never reach HBM; see pbk_fast.cuh (FSUM).

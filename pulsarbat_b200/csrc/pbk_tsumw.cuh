@@ -186,17 +186,20 @@ tsum_warp_kernel(const __grid_constant__ PassArgs p, const __grid_constant__ CUt
     }
   };
   // tile row b + 16 i at inner offset nrest is time n = (row << log2nmul) + nrest and lands in
-  // output row (n - crop_start) >> tsum_log2 (see tsum_flush in pbk_fast.cuh)
+  // output row (n - crop_start) >> tsum_log2, or its phase bin (see tsum_flush in pbk_fast.cuh)
   auto flush = [&](char* colbase, unsigned nrest) {
 #pragma unroll
     for (int i = 0; i < 16; ++i) {
       const long long n = ((long long)(b + 16 * i) << p.log2nmul) + nrest;
-      char* a = colbase + ((n - p.crop_start) >> p.tsum_log2) * ts_rowbytes;
       if constexpr (EPI == EPI_STOKES_I) {
-        if (acc[i] != 0.f) atomicAdd(reinterpret_cast<float*>(a), acc[i]);
+        if (acc[i] != 0.f)
+          atomicAdd(reinterpret_cast<float*>(tsum_row(p, colbase, n, ts_rowbytes)), acc[i]);
       } else {
-        if (acc[i].x != 0.f) atomicAdd(reinterpret_cast<float*>(a), acc[i].x);
-        if (acc[i].y != 0.f) atomicAdd(reinterpret_cast<float*>(a) + 1, acc[i].y);
+        if (acc[i].x != 0.f || acc[i].y != 0.f) {
+          float* a = reinterpret_cast<float*>(tsum_row(p, colbase, n, ts_rowbytes));
+          if (acc[i].x != 0.f) atomicAdd(a, acc[i].x);
+          if (acc[i].y != 0.f) atomicAdd(a + 1, acc[i].y);
+        }
       }
     }
     acc_clear();

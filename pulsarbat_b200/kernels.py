@@ -23,7 +23,8 @@ from . import _lib as L
 from .device import DeviceArray
 
 __all__ = ["default_device", "dedisperse", "chirp", "detect", "shift_channels", "phase_ramp", "mix", "analytic_decimate", "stokes", "pol_basis",
-           "downsample", "fft", "stft", "istft", "stft_detect", "stft_fold", "fold", "predict_phase", "clear_plan_cache",
+           "downsample", "fft", "stft", "istft", "stft_detect", "stft_fold", "fold",
+           "dedisperse_fold", "predict_phase", "clear_plan_cache",
            "pinned_results"]
 
 
@@ -272,41 +273,139 @@ def dedisperse(data, *, dm, sample_rate_hz, chan_freq_hz, ref_freq_hz, crop=None
     """
     if int8 and raw is None:
         raw = "int8"
-    if raw is not None and raw not in _RAW_KINDS:
-        raise ValueError(f"raw must be one of {sorted(_RAW_KINDS)}, got {raw!r}")
-    int8 = raw is not None            # below: "the input is raw bytes"
-    shape = tuple(data.shape)
-    if raw == "u2":
-        if raw_shape is None:
-            raise ValueError('raw="u2" needs raw_shape=(nchan, ...)')
-        body = (shape[0],) + tuple(int(v) for v in raw_shape)
-        if int(np.prod(body[1:])) != 2 * int(np.prod(shape[1:])):
-            raise ValueError(f"raw_shape {raw_shape} does not match rows of {shape[1:]} bytes")
-    else:
-        body = shape[:-1] if raw == "int8" else shape
-    nsamp, nchan = body[0], body[1]
-    trailing = body[2:]
-    npol = int(np.prod(trailing)) if trailing else 1
-    in_dtype, raw_np = _RAW_KINDS[raw] if raw is not None else (L.PBK_C64, None)
-    start, stop = (0, nsamp) if crop is None else (int(crop[0]), int(crop[1]))
-    if stop <= start:
-        start, stop = 0, 0
-    freqs = np.ascontiguousarray(chan_freq_hz, dtype=np.float64)
+    g = _DedispGeometry(data, raw, raw_shape, crop)
     dev = (data.device if _is_dev(data) else (default_device() if device is None else device))
     if raw is None and _is_c128(data):
-        return _dedisperse_c128(data, nsamp, nchan, npol, trailing, dm, sample_rate_hz, freqs,
-                                ref_freq_hz, start, stop, out_kind, downsample, chirp_array, dev)
-    key = ("dedisp", nsamp, nchan, npol, raw, int(out_kind), float(dm),
-           float(sample_rate_hz), float(ref_freq_hz), freqs.tobytes(), start, stop,
-           int(downsample), chirp_array is not None, dev)
-    ctx = _use_plan(key, lambda: L.DedispPlan(
-        nsamp=nsamp, nchan=nchan, npol=npol, dm=dm, sample_rate_hz=sample_rate_hz,
-        ref_freq_hz=ref_freq_hz, chan_freq_hz=freqs, crop=(start, stop),
-        in_dtype=in_dtype, out_kind=out_kind, downsample=downsample,
-        explicit_chirp=chirp_array is not None, device=dev))
+        return _dedisperse_c128(data, g.nsamp, g.nchan, g.npol, g.trailing, dm, sample_rate_hz,
+                                g.freqs(chan_freq_hz), ref_freq_hz, g.start, g.stop, out_kind,
+                                downsample, chirp_array, dev)
+    ctx = g.plan(dm=dm, sample_rate_hz=sample_rate_hz, chan_freq_hz=chan_freq_hz,
+                 ref_freq_hz=ref_freq_hz, out_kind=out_kind, downsample=downsample,
+                 explicit_chirp=chirp_array is not None, dev=dev)
     with ctx as plan:
-        return _dedisperse_with(ctx, plan, data, nsamp, nchan, trailing, out_kind, chirp_array,
-                                int8, raw_np, dev)
+        return _dedisperse_with(ctx, plan, data, g.nsamp, g.nchan, g.trailing, out_kind,
+                                chirp_array, raw is not None, g.raw_np, dev)
+
+
+class _DedispGeometry:
+    """Shape, input kind and crop of a dedispersion call (``raw`` / ``raw_shape`` / ``crop`` as in
+    :func:`dedisperse`), and the cached plan for it."""
+
+    def __init__(self, data, raw, raw_shape, crop):
+        if raw is not None and raw not in _RAW_KINDS:
+            raise ValueError(f"raw must be one of {sorted(_RAW_KINDS)}, got {raw!r}")
+        shape = tuple(data.shape)
+        if raw == "u2":
+            if raw_shape is None:
+                raise ValueError('raw="u2" needs raw_shape=(nchan, ...)')
+            body = (shape[0],) + tuple(int(v) for v in raw_shape)
+            if int(np.prod(body[1:])) != 2 * int(np.prod(shape[1:])):
+                raise ValueError(f"raw_shape {raw_shape} does not match rows of {shape[1:]} bytes")
+        else:
+            body = shape[:-1] if raw == "int8" else shape
+        self.raw = raw
+        self.nsamp, self.nchan = body[0], body[1]
+        self.trailing = body[2:]
+        self.npol = int(np.prod(self.trailing)) if self.trailing else 1
+        self.in_dtype, self.raw_np = _RAW_KINDS[raw] if raw is not None else (L.PBK_C64, None)
+        start, stop = (0, self.nsamp) if crop is None else (int(crop[0]), int(crop[1]))
+        self.start, self.stop = (0, 0) if stop <= start else (start, stop)
+
+    @staticmethod
+    def freqs(chan_freq_hz):
+        return np.ascontiguousarray(chan_freq_hz, dtype=np.float64)
+
+    def plan(self, *, dm, sample_rate_hz, chan_freq_hz, ref_freq_hz, out_kind, downsample,
+             explicit_chirp, dev):
+        freqs = self.freqs(chan_freq_hz)
+        key = ("dedisp", self.nsamp, self.nchan, self.npol, self.raw, int(out_kind), float(dm),
+               float(sample_rate_hz), float(ref_freq_hz), freqs.tobytes(), self.start, self.stop,
+               int(downsample), bool(explicit_chirp), dev)
+        return _use_plan(key, lambda: L.DedispPlan(
+            nsamp=self.nsamp, nchan=self.nchan, npol=self.npol, dm=dm,
+            sample_rate_hz=sample_rate_hz, ref_freq_hz=ref_freq_hz, chan_freq_hz=freqs,
+            crop=(self.start, self.stop), in_dtype=self.in_dtype, out_kind=out_kind,
+            downsample=downsample, explicit_chirp=explicit_chirp, device=dev))
+
+
+def _check_acc(a, name, dtype, want_shape, on_device):
+    """Accumulator given by the caller: raw pointers go to the kernel, so a wrong dtype, shape or
+    placement would corrupt memory silently."""
+    if a is None:
+        return
+    if np.dtype(a.dtype) != np.dtype(dtype) or tuple(a.shape) != tuple(want_shape):
+        raise ValueError(f"{name} must be {np.dtype(dtype).name} of shape {tuple(want_shape)}, "
+                         f"got {np.dtype(a.dtype).name} {tuple(a.shape)}")
+    if on_device != _is_dev(a):
+        raise ValueError(f"{name} must live where the data lives (host array / DeviceArray)")
+    if not _is_dev(a) and not a.flags["C_CONTIGUOUS"]:
+        raise ValueError(f"{name} must be C-contiguous")
+
+
+def dedisperse_fold(data, *, dm, sample_rate_hz, chan_freq_hz, ref_freq_hz, crop, coeffs, nbin,
+                    n0=0, out_kind=L.OUT_INTENSITY, downsample=1, raw=None, raw_shape=None,
+                    profile=None, counts=None):
+    """``fold(dedisperse(data, ..., out_kind=out_kind, downsample=downsample), coeffs,
+    sample_rate_hz / downsample, nbin, n0)`` for a device-resident block: coherent dedispersion,
+    detection (``OUT_INTENSITY`` per pol or ``OUT_STOKES_I``), time sum and fold into phase bins.
+    ``n0`` is the index of the block's first OUTPUT row in the stream, as in :func:`fold`.
+
+    complex64 and raw (``raw="int8" | "u4" | "u2"``, see :func:`dedisperse`) blocks run as one
+    library call on the block's dedispersion plan (the one :func:`dedisperse` caches for the same
+    arguments): where the plan sums time in its last inverse pass, that pass adds its sums straight
+    into the profile and the intensity never reaches HBM.  complex128 runs the FP64
+    :func:`dedisperse` and :func:`fold`.  ``profile`` (nbin, nchan[, npol...]) float32 and
+    ``counts`` (nbin,) int64 DeviceArrays are accumulated into when given.  Returns
+    (profile, counts)."""
+    if not _is_dev(data):
+        raise TypeError("dedisperse_fold takes a DeviceArray (host streams: "
+                        "pulsar.dedisperse_fold, or dedisperse + fold)")
+    if out_kind not in (L.OUT_INTENSITY, L.OUT_STOKES_I):
+        raise ValueError("dedisperse_fold needs out_kind OUT_INTENSITY or OUT_STOKES_I")
+    import torch
+    g = _DedispGeometry(data, raw, raw_shape, crop)
+    dev = data.device
+    nbin = int(nbin)
+    if nbin <= 0:
+        raise ValueError("nbin must be positive")
+    c = np.ascontiguousarray(coeffs, dtype=np.float64)
+    if c.ndim != 1 or not np.all(np.isfinite(c)):
+        raise ValueError("coeffs must be a 1-D array of finite numbers")
+    cells = (g.nchan,) if out_kind == L.OUT_STOKES_I else (g.nchan,) + tuple(g.trailing)
+    _check_acc(profile, "profile", np.float32, (nbin,) + cells, True)
+    _check_acc(counts, "counts", np.int64, (nbin,), True)
+    if profile is None:
+        profile = DeviceArray(torch.zeros((nbin,) + cells, dtype=torch.float32,
+                                          device=f"cuda:{dev}"))
+    if counts is None:
+        counts = DeviceArray(torch.zeros((nbin,), dtype=torch.int64, device=f"cuda:{dev}"))
+    profile, counts = profile.contiguous(), counts.contiguous()
+    rate = float(sample_rate_hz) / int(downsample)
+    if raw is None and _is_c128(data):
+        y = dedisperse(data, dm=dm, sample_rate_hz=sample_rate_hz, chan_freq_hz=chan_freq_hz,
+                       ref_freq_hz=ref_freq_hz, crop=(g.start, g.stop), out_kind=out_kind,
+                       downsample=downsample)
+        if y.shape[0] == 0:
+            return profile, counts
+        return fold(y, c, rate, nbin, n0=n0, profile=profile, counts=counts)
+    ctx = g.plan(dm=dm, sample_rate_hz=sample_rate_hz, chan_freq_hz=chan_freq_hz,
+                 ref_freq_hz=ref_freq_hz, out_kind=out_kind, downsample=downsample,
+                 explicit_chirp=False, dev=dev)
+    with ctx as plan:
+        x = data.contiguous()
+        if raw is None and x.dtype != np.complex64:
+            x = x.astype(np.complex64)
+        with ctx.lock:
+            plan.fold_device(x.ptr, profile.ptr, counts.ptr, c, rate, n0, nbin, _stream())
+            _recount(ctx.ent)
+    return profile, counts
+
+
+def _recount(ent):
+    """A fold execution may have allocated plan-owned buffers: the cache's byte cap must see them."""
+    b = int(ent.plan.info()["workspace_bytes"])
+    with _cache_lock:
+        ent.bytes = b
 
 
 def _dedisperse_c128(data, nsamp, nchan, npol, trailing, dm, sample_rate_hz, freqs, ref_freq_hz,
@@ -831,19 +930,8 @@ def fold(data, coeffs, sample_rate_hz, nbin, n0=0, profile=None, counts=None, wa
         raise ValueError("coeffs must be a 1-D array of finite numbers")
     cp = c.ctypes.data_as(ctypes.POINTER(ctypes.c_double))
 
-    def check_acc(a, name, dtype, want_shape):
-        # raw pointers go to the kernel: a wrong dtype or shape would corrupt memory silently
-        if a is None:
-            return
-        if np.dtype(a.dtype) != np.dtype(dtype) or tuple(a.shape) != tuple(want_shape):
-            raise ValueError(f"{name} must be {np.dtype(dtype).name} of shape {tuple(want_shape)}, "
-                             f"got {np.dtype(a.dtype).name} {tuple(a.shape)}")
-        if _is_dev(data) != _is_dev(a):
-            raise ValueError(f"{name} must live where the data lives (host array / DeviceArray)")
-        if not _is_dev(a) and not a.flags["C_CONTIGUOUS"]:
-            raise ValueError(f"{name} must be C-contiguous")
-    check_acc(profile, "profile", np.float32, (int(nbin),) + shape[1:])
-    check_acc(counts, "counts", np.int64, (int(nbin),))
+    _check_acc(profile, "profile", np.float32, (int(nbin),) + shape[1:], _is_dev(data))
+    _check_acc(counts, "counts", np.int64, (int(nbin),), _is_dev(data))
     if _is_dev(data):
         x = data.contiguous()
         if x.dtype != np.float32:

@@ -1,6 +1,6 @@
 """Pulsar timing helpers on the fold path (reference: pulsarbat/pulsar/)."""
 
-from .folding import fold  # noqa: F401
+from .folding import dedisperse_fold, fold  # noqa: F401
 from .predictor import PhasePredictor, PolycoEntry  # noqa: F401
 
-__all__ = ["PolycoEntry", "PhasePredictor", "fold"]
+__all__ = ["PolycoEntry", "PhasePredictor", "fold", "dedisperse_fold"]

@@ -88,6 +88,19 @@ def dedisperse_blocks(blocks, *, dm, sample_rate_hz, chan_freq_hz, ref_freq_hz, 
     (no extra host copy); by default a fresh array is returned.  ``raw`` / ``raw_shape`` select
     packed raw input exactly as in :func:`kernels.dedisperse` (``int8=True`` is ``raw="int8"``).
     """
+    yield from _stream_blocks(blocks, dm=dm, sample_rate_hz=sample_rate_hz,
+                              chan_freq_hz=chan_freq_hz, ref_freq_hz=ref_freq_hz, crop=crop,
+                              out_kind=out_kind, downsample=downsample, int8=int8, raw=raw,
+                              raw_shape=raw_shape, device=device, pinned_out=pinned_out)
+
+
+def _stream_blocks(blocks, *, dm, sample_rate_hz, chan_freq_hz, ref_freq_hz, crop, out_kind,
+                   downsample, int8=False, raw=None, raw_shape=None, device=None,
+                   pinned_out=False, run=None):
+    """The pipeline behind :func:`dedisperse_blocks`.  With ``run`` the blocks are only uploaded:
+    ``run(i, plan, d_in, stream)`` enqueues whatever block i needs on the compute stream (the
+    device input buffer ``d_in`` is free for the next upload once that work is done), there is no
+    device output buffer and no download leg, and the generator yields nothing."""
     import torch
     dev = kernels.default_device() if device is None else device
     tdev = torch.device(f"cuda:{dev}")
@@ -129,27 +142,29 @@ def dedisperse_blocks(blocks, *, dm, sample_rate_hz, chan_freq_hz, ref_freq_hz, 
                             downsample=downsample, device=dev)
         out_trailing = (nchan,) if out_kind == L.OUT_STOKES_I else (nchan,) + tuple(trailing)
         out_shape = (plan.out_rows,) + out_trailing
+        nout = 0 if run is not None else 2
         with torch.cuda.device(tdev):
             return _State(plan,
                           [torch.empty(shape, dtype=in_t, device=tdev) for _ in range(2)],
-                          [torch.empty(out_shape, dtype=out_t, device=tdev) for _ in range(2)],
-                          [torch.empty(out_shape, dtype=out_t, pin_memory=True) for _ in range(2)],
+                          [torch.empty(out_shape, dtype=out_t, device=tdev) for _ in range(nout)],
+                          [torch.empty(out_shape, dtype=out_t, pin_memory=True)
+                           for _ in range(nout)],
                           torch.cuda.Stream(tdev), torch.cuda.Stream(tdev), torch.cuda.Stream(tdev),
                           [torch.cuda.Event() for _ in range(6)])
 
     key = (shape, raw, body, float(dm), float(sample_rate_hz), float(ref_freq_hz),
-           freqs.tobytes(), start, stop, int(out_kind), int(downsample), dev)
+           freqs.tobytes(), start, stop, int(out_kind), int(downsample), dev, run is not None)
     state = _checkout(key, make)      # owned by this generator until the finally below
     try:
         state.quiesce()               # a previous owner may have been abandoned mid-stream
-        yield from _run_stream(state, first, it, shape, dev, tdev, pinned_out)
+        yield from _run_stream(state, first, it, shape, dev, tdev, pinned_out, run)
     finally:
         # runs on exhaustion, on .close() and when an abandoned generator is collected
         state.quiesce()
         _checkin(key, state)
 
 
-def _run_stream(state, first, it, shape, dev, tdev, pinned_out):
+def _run_stream(state, first, it, shape, dev, tdev, pinned_out, run=None):
     import torch
     plan, d_in, d_out, h_out = state.plan, state.d_in, state.d_out, state.h_out
     s_copy, s_comp, s_down, ev = state.s_copy, state.s_comp, state.s_down, state.ev
@@ -167,8 +182,12 @@ def _run_stream(state, first, it, shape, dev, tdev, pinned_out):
         copied[slot].record(s_copy)
         return hb                                             # keeps the host block alive
 
-    def compute(slot, reuse):
+    def compute(i, slot, reuse):
         s_comp.wait_event(copied[slot])
+        if run is not None:
+            run(i, plan, d_in[slot], s_comp)
+            consumed[slot].record(s_comp)
+            return
         if reuse:
             s_comp.wait_event(done[slot])      # the previous result of this slot has left the device
         plan.exec_device(d_in[slot].data_ptr(), d_out[slot].data_ptr(), None, s_comp.cuda_stream)
@@ -185,6 +204,7 @@ def _run_stream(state, first, it, shape, dev, tdev, pinned_out):
         return r if pinned_out else r.copy()
 
     with torch.cuda.device(tdev):
+        s_comp.wait_stream(torch.cuda.current_stream(tdev))   # e.g. a zeroed accumulator of `run`
         keep = [upload(first, 0, False), None]
         i = 0
         nxt = next(it, None)
@@ -192,13 +212,14 @@ def _run_stream(state, first, it, shape, dev, tdev, pinned_out):
             slot = i & 1
             # kernels of block i are queued before block i+1 is uploaded: a pageable block is
             # copied by host threads inside upload() (csrc/pbk_hostcopy.h), which then overlaps them
-            compute(slot, i >= 2)
+            compute(i, slot, i >= 2)
             if nxt is not None:
                 keep[slot ^ 1] = upload(nxt, slot ^ 1, i >= 1)
-            if i >= 1:
+            if run is None and i >= 1:
                 yield result(slot ^ 1)
             if nxt is None:
-                yield result(slot)
+                if run is None:
+                    yield result(slot)
                 break
             i += 1
             nxt = next(it, None)

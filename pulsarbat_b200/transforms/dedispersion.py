@@ -98,12 +98,13 @@ def _as_dm(x):
     return x if isinstance(x, DispersionMeasure) else DispersionMeasure(x)
 
 
-def crop_range(z, dm, ref_freq):
-    """(start, stop) exactly as dedispersion.py:127-131."""
+def crop_range(z, dm, ref_freq, nsamp=None):
+    """(start, stop) exactly as dedispersion.py:127-131, for a block of ``nsamp`` samples of ``z``
+    (default: all of it)."""
     d_top = dm.sample_delay(z.max_freq, ref_freq, z.sample_rate)
     d_bot = dm.sample_delay(z.min_freq, ref_freq, z.sample_rate)
     start = math.ceil(-min(0, d_top, d_bot))
-    stop = len(z) - math.ceil(+max(0, d_top, d_bot))
+    stop = (len(z) if nsamp is None else nsamp) - math.ceil(+max(0, d_top, d_bot))
     return start, stop
 
 
