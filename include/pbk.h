@@ -18,11 +18,20 @@
  *    stream) and do not synchronise.  A plan owns its scratch arrays (one, or two of N*C*P*8
  *    bytes each when that is at most 1/5 of the device memory; pbk_plan_info reports the total):
  *    executions of the same plan must be ordered on the device (same stream, or events between
- *    streams).  A *_device execution only enqueues kernels (and a memset of a summed output):
- *    it can be captured into a CUDA graph.  The passes of one execution are chained with
+ *    streams).  A *_device execution only enqueues kernels (and a memset of a summed output,
+ *    and the device-to-device copies of a staged array, below): it can be captured into a CUDA
+ *    graph once the plan's lazily allocated buffers exist.  The passes of one execution are chained with
  *    programmatic dependent launch (PBK_PDL=0 switches it off); the first pass waits for the
  *    previous kernel of the stream to complete like any kernel, and kernels the caller enqueues
  *    afterwards wait for the last pass.
+ *  - Device pointers need only the alignment of their element type: 8 bytes for complex64 and
+ *    int64, 4 for float32 and int32, 2 for int8 (re, im) pairs, 1 for packed u4 / u2 rows.
+ *    16-byte aligned arrays take the vectorised kernels.  Other arrays give the same result on a
+ *    scalar path, or through a plan-owned 16-byte aligned staging buffer and a device-to-device
+ *    copy where the work needs the vectorised kernels: the output of a plan whose last pass sums
+ *    time, detects or recombines even / odd samples, and the profile of
+ *    pbk_stft_fold_exec_device.  The staging buffer is allocated at the first execution that
+ *    needs it and counted in pbk_plan_info's workspace bytes.
  *  - There is no CPU fallback: without a CUDA device every call fails with PBK_ERR_CUDA.
  */
 #ifndef PBK_H_
@@ -124,8 +133,8 @@ int pbk_dedisp_exec_device(pbk_plan* plan, const void* d_in, void* d_out, const 
  * (input rate / downsample).  Device pointers, enqueued on `stream`; nothing is written to a
  * voltage or intensity array of the caller.
  * When the plan sums time in the epilogue of its last inverse pass (pbk_plan_describe shows
- * ":timesum"), the intensity (out_rows x row_elems floats) is at least 256 MiB and there are at
- * most 512 rows per bin, the bins are computed first and that pass adds its group sums straight
+ * ":timesum"), the intensity (out_rows x row_elems floats) is at least 256 MiB, there are at
+ * most 512 rows per bin and d_profile is 16-byte aligned, the bins are computed first and that pass adds its group sums straight
  * into the profile, so the intensity never reaches HBM; otherwise (smaller intensities stay in L2
  * between two steps, and many rows per bin serialise the atomics) the plan's normal execution
  * writes a plan-owned float32 buffer of out_rows x row_elems (allocated at the first such
@@ -208,7 +217,9 @@ int pbk_stft_detect_plan_create(int64_t nseg, int64_t nperseg, int64_t nchan, in
  * to profile[bin(s), :, :] (float32 (nbin, nperseg/freq_sum[, npol]), caller-zeroed or carrying
  * earlier blocks) and counts[bin(s)] += 1 (int64 (nbin,)), bin(s) from the phase polynomial at
  * t = (n0 + s) / sample_rate_hz exactly as pbk_fold (sample_rate_hz is the SEGMENT rate).  `plan`
- * comes from pbk_stft_detect_plan_create; device pointers, enqueued on `stream`. */
+ * comes from pbk_stft_detect_plan_create; device pointers, enqueued on `stream`.  A profile that
+ * is not 16-byte aligned is copied into the plan's staging buffer, accumulated there by the same
+ * launches and copied back. */
 int pbk_stft_fold_exec_device(pbk_plan* plan, const void* d_in, void* d_profile, void* d_counts,
                               const double* coeffs, int32_t ncoef, double sample_rate_hz,
                               int64_t n0, int32_t nbin, void* stream);

@@ -152,6 +152,8 @@ struct pbk_plan {
   bool split_column = false;    // single column run as its even / odd samples (see plan creation)
   bool split_ragged = false;    // ... with an odd crop edge: passes write d_tmpf, then a D2D copy
   size_t split_skip = 0;
+  void* d_stage = nullptr;      // 16-byte aligned stand-in for a caller's array that is not (see
+  size_t stage_bytes = 0;       // stage_ensure); lazily allocated, grown on demand
   // lazily allocated staging buffers for *_host execution
   void* h_din = nullptr;
   void* h_dout = nullptr;
@@ -1130,6 +1132,34 @@ static void* role_ptr(const pbk_plan* pl, int role, const void* uin, void* uout)
   }
 }
 
+static bool misaligned16(const void* p) { return ((uintptr_t)p & 15) != 0; }
+
+// Epilogues that only the compile-time-shaped (fast / TMA / warp-private) kernels implement: the
+// time sum (and the fold behind it), the detection with its frequency sum (and fold), and the even
+// / odd recombination.  The generic pass_kernel would silently skip them and write a differently
+// shaped result, so such a pass never takes it.
+static bool needs_fast_kernel(const Pass& ps) {
+  return ps.a.tsum_log2 > 0 || ps.a.fsum_log2 > 0 || ps.a.fsum_split || ps.a.split;
+}
+
+// The fast kernels move 16-byte vectors, while the C ABI only promises element alignment.  When the
+// last pass needs them and the caller's output is not 16-byte aligned, it writes this plan-owned
+// buffer and the execution copies it out (device to device), as split_ragged does with d_tmpf.
+static bool last_pass_needs_fast(const pbk_plan* pl) {
+  return !pl->passes.empty() && pl->passes.back().out_role == ROLE_USER_OUT &&
+         needs_fast_kernel(pl->passes.back());
+}
+
+static int stage_ensure(pbk_plan* pl, size_t bytes) {
+  if (pl->stage_bytes >= bytes) return PBK_OK;
+  cudaFree(pl->d_stage);   // waits for the work queued on the old buffer
+  pl->d_stage = nullptr;
+  pl->stage_bytes = 0;
+  CUDA_TRY(cudaMalloc(&pl->d_stage, bytes));
+  pl->stage_bytes = bytes;
+  return PBK_OK;
+}
+
 static int launch_one(pbk_plan* pl, const Pass& ps, const void* d_in, void* d_out,
                       const void* d_chirp, long long tile0, long long tile_end, cudaStream_t st,
                       int idx = 0) {
@@ -1146,6 +1176,12 @@ static int launch_one(pbk_plan* pl, const Pass& ps, const void* d_in, void* d_ou
   if (p.a.fsum_log2 > 0) p.a.fsum_bins = pl->exec_segbins;
   if (p.a.tsum_log2 > 0) p.a.tsum_bins = pl->exec_segbins;
   const bool aligned = (((uintptr_t)p.a.in | (uintptr_t)p.a.out) & 15) == 0;
+  if (needs_fast_kernel(ps) && !(ps.family >= 0 && aligned))
+    return fail(PBK_ERR_UNSUPPORTED, "%s pass with a fused %s epilogue needs the "
+                "compile-time-shaped kernels and 16-byte aligned arrays (in %p, out %p)",
+                ps.mode == MODE_FWD ? "FWD" : ps.mode == MODE_MID ? "MID" : "INV",
+                ps.a.tsum_log2 > 0 ? "time-sum" : ps.a.fsum_log2 > 0 ? "detection" : "even/odd",
+                p.a.in, p.a.out);
   cudaError_t e;
   CUtensorMap tm;
   if (ps.tma && aligned && tile0 == 0 && tile_end < 0 && tma_encode(ps, p.a.in, &tm)) {
@@ -1265,10 +1301,19 @@ extern "C" int pbk_dedisp_exec_device(pbk_plan* pl, const void* d_in, void* d_ou
   CUDA_TRY(cudaSetDevice(pl->device));
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   if (pl->blue) return blue_exec(pl, d_in, d_out, d_chirp, st);
+  void* dst = pl->split_ragged ? pl->d_tmpf : d_out;
+  const bool stage = last_pass_needs_fast(pl) && misaligned16(dst);
+  int rc;
+  if (stage) {
+    if ((rc = stage_ensure(pl, pl->out_bytes)) != PBK_OK) return rc;
+    dst = pl->d_stage;
+  }
   if (pl->fused_tsum)   // the last pass adds its group sums to the output
-    CUDA_TRY(cudaMemsetAsync(d_out, 0, pl->out_bytes, st));
-  int rc = run_passes(pl, d_in, pl->split_ragged ? pl->d_tmpf : d_out, d_chirp, st);
+    CUDA_TRY(cudaMemsetAsync(dst, 0, pl->out_bytes, st));
+  rc = run_passes(pl, d_in, dst, d_chirp, st);
   if (rc != PBK_OK) return rc;
+  if (stage)
+    CUDA_TRY(cudaMemcpyAsync(d_out, pl->d_stage, pl->out_bytes, cudaMemcpyDeviceToDevice, st));
   if (pl->split_ragged)
     CUDA_TRY(cudaMemcpyAsync(d_out, static_cast<const char*>(pl->d_tmpf) + pl->split_skip,
                              pl->out_bytes, cudaMemcpyDeviceToDevice, st));
@@ -1330,9 +1375,11 @@ extern "C" int pbk_dedisp_fold_exec_device(pbk_plan* pl, const void* d_in, void*
   // per-pol x8 / 1024 bins (256 MiB, 512 rows per bin) 0.987x the two steps, x4 (1024 rows per
   // bin) 0.96x; Stokes I x4 (256 MiB, 1024 rows per bin) 1.017x, x64 (16 MiB) 1.005x, 16 bins up
   // to 1.23x.  So: fused only for an intermediate of >= 256 MiB with <= 512 rows per bin.
+  // The fused pass runs on the fast kernels only, which need 16-byte aligned arrays: a profile
+  // aligned only to its float32 elements takes the unfused route.
   const bool fuse = pl->fused_tsum &&
                     (size_t)pl->out_rows * pl->row_elems * 4 >= ((size_t)256 << 20) &&
-                    pl->out_rows <= 512ll * nbin;
+                    pl->out_rows <= 512ll * nbin && !misaligned16(d_profile);
   if (fuse) {
     if (!pl->d_segbins) {
       const size_t b = (size_t)pl->out_rows * sizeof(int);
@@ -1901,7 +1948,14 @@ extern "C" int pbk_fft_exec_device(pbk_plan* pl, const void* d_in, void* d_out, 
   if (pl->blue) return blue_exec(pl, d_in, d_out, nullptr, reinterpret_cast<cudaStream_t>(stream));
   if (d_in == d_out && pl->passes.size() == 1)
     return fail(PBK_ERR_INVALID, "single-pass transforms cannot run in place");
-  return run_passes(pl, d_in, d_out, nullptr, reinterpret_cast<cudaStream_t>(stream));
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  if (!(last_pass_needs_fast(pl) && misaligned16(d_out)))
+    return run_passes(pl, d_in, d_out, nullptr, st);
+  int rc = stage_ensure(pl, pl->out_bytes);   // detecting or even / odd last pass: see stage_ensure
+  if (rc == PBK_OK) rc = run_passes(pl, d_in, pl->d_stage, nullptr, st);
+  if (rc != PBK_OK) return rc;
+  CUDA_TRY(cudaMemcpyAsync(d_out, pl->d_stage, pl->out_bytes, cudaMemcpyDeviceToDevice, st));
+  return PBK_OK;
 }
 
 extern "C" int pbk_stft_fold_exec_device(pbk_plan* pl, const void* d_in, void* d_profile,
@@ -1937,10 +1991,23 @@ extern "C" int pbk_stft_fold_exec_device(pbk_plan* pl, const void* d_in, void* d
   fold_bins_kernel<<<blocks, 256, 0, st>>>(fa, pl->d_segbins);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return fail(PBK_ERR_CUDA, "fold bins launch: %s", cudaGetErrorString(e));
+  // a profile aligned only to its float32 elements is accumulated in the plan's aligned staging
+  // buffer: copied in, added to by the detecting pass, copied back
+  void* prof = d_profile;
+  const size_t prof_bytes = (size_t)nbin * pl->det_cells * pl->det_pq * sizeof(float);
+  if (misaligned16(d_profile)) {
+    int rc = stage_ensure(pl, prof_bytes);
+    if (rc != PBK_OK) return rc;
+    prof = pl->d_stage;
+    CUDA_TRY(cudaMemcpyAsync(prof, d_profile, prof_bytes, cudaMemcpyDeviceToDevice, st));
+  }
   pl->exec_segbins = pl->d_segbins;
-  const int rc = run_passes(pl, d_in, d_profile, nullptr, st);
+  const int rc = run_passes(pl, d_in, prof, nullptr, st);
   pl->exec_segbins = nullptr;
-  return rc;
+  if (rc != PBK_OK) return rc;
+  if (prof != d_profile)
+    CUDA_TRY(cudaMemcpyAsync(d_profile, prof, prof_bytes, cudaMemcpyDeviceToDevice, st));
+  return PBK_OK;
 }
 
 extern "C" int pbk_fft_exec_host(pbk_plan* pl, const void* in, void* out) {
@@ -2010,6 +2077,7 @@ extern "C" void pbk_plan_destroy(pbk_plan* pl) {
   cudaFree(pl->d_tmpf);
   cudaFree(pl->d_segbins);
   cudaFree(pl->d_foldbuf);
+  cudaFree(pl->d_stage);
   cudaFree(pl->d_l2sync);
   cudaFree(pl->h_din);
   cudaFree(pl->h_dout);
@@ -2022,7 +2090,8 @@ extern "C" int pbk_plan_info(const pbk_plan* pl, int32_t* launches, int64_t* wor
   if (!pl) return fail(PBK_ERR_INVALID, "plan is NULL");
   if (launches) *launches = pl->launches;
   if (workspace_bytes) *workspace_bytes =
-      (int64_t)(pl->scratch_bytes * (pl->scratch2 ? 2 : 1) + pl->tmpf_bytes + pl->fold_bytes);
+      (int64_t)(pl->scratch_bytes * (pl->scratch2 ? 2 : 1) + pl->tmpf_bytes + pl->fold_bytes +
+                pl->stage_bytes);
   if (levels) *levels = pl->nlevels;
   if (level_log2)
     for (int i = 0; i < 3; ++i) level_log2[i] = pl->level_log2[i];
@@ -2387,9 +2456,10 @@ extern "C" int pbk_stokes(const void* in, void* out, int64_t npairs, int32_t cir
   if (npairs < 0) return fail(PBK_ERR_INVALID, "bad count");
   return run_elementwise(in, out, (size_t)npairs * 16, (size_t)npairs * 16, on_device, device,
                          stream, [&](const void* i, void* o, cudaStream_t st) {
-                           return launch_1d(stokes_kernel, npairs, st,
-                                            reinterpret_cast<const float4*>(i),
-                                            reinterpret_cast<float4*>(o), (long long)npairs,
+                           return launch_1d(aligned16(i, o) ? stokes_kernel<true>
+                                                            : stokes_kernel<false>,
+                                            npairs, st, reinterpret_cast<const float2*>(i),
+                                            reinterpret_cast<float*>(o), (long long)npairs,
                                             (int)circular);
                          });
 }
@@ -2399,9 +2469,10 @@ extern "C" int pbk_pol_basis(const void* in, void* out, int64_t npairs, int32_t 
   if (npairs < 0) return fail(PBK_ERR_INVALID, "bad count");
   return run_elementwise(in, out, (size_t)npairs * 16, (size_t)npairs * 16, on_device, device,
                          stream, [&](const void* i, void* o, cudaStream_t st) {
-                           return launch_1d(pol_basis_kernel, npairs, st,
-                                            reinterpret_cast<const float4*>(i),
-                                            reinterpret_cast<float4*>(o), (long long)npairs,
+                           return launch_1d(aligned16(i, o) ? pol_basis_kernel<true>
+                                                            : pol_basis_kernel<false>,
+                                            npairs, st, reinterpret_cast<const float2*>(i),
+                                            reinterpret_cast<float2*>(o), (long long)npairs,
                                             (int)to_circular);
                          });
 }

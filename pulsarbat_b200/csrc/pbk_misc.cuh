@@ -64,9 +64,38 @@ static inline cudaError_t launch_downsample(const float* in, float* out, long lo
   return cudaGetLastError();
 }
 
+// one (A, B) pol pair of complex64 as (Are, Aim, Bre, Bim): a 128-bit load when the array is
+// 16-byte aligned (V4), two 64-bit loads when it is only aligned to its complex64 elements
+template <bool V4>
+__device__ __forceinline__ float4 ld_pair(const float2* p) {
+  if (V4) return __ldg(reinterpret_cast<const float4*>(p));
+  const float2 a = __ldg(p), b = __ldg(p + 1);
+  return make_float4(a.x, a.y, b.x, b.y);
+}
+// four floats: one 128-bit store, or four 32-bit stores (a float32 Stokes array may be aligned
+// to 4 bytes only)
+template <bool V4>
+__device__ __forceinline__ void st_pair(float* p, float4 v) {
+  if (V4) {
+    *reinterpret_cast<float4*>(p) = v;
+  } else {
+    p[0] = v.x;
+    p[1] = v.y;
+    p[2] = v.z;
+    p[3] = v.w;
+  }
+}
+
+// pol-pair kernels below take the 128-bit path only for 16-byte aligned arrays (the C ABI promises
+// complex64 alignment, 8 bytes, and nothing more)
+static inline bool aligned16(const void* a, const void* b) {
+  return (((uintptr_t)a | (uintptr_t)b) & 15) == 0;
+}
+
 // power detection with optional time sum.  in (rows*M, CP) complex64.
 //   stokes == 0: out (rows, CP)   = sum_m re^2+im^2
 //   stokes == 1: out (rows, CP/2) = sum_m |A|^2+|B|^2   (pol pairs are adjacent)
+template <bool V4>
 __global__ void __launch_bounds__(256) detect_kernel(const float2* __restrict__ in,
                                                      float* __restrict__ out, long long rows,
                                                      long long CP, int stokes, long long M) {
@@ -78,7 +107,7 @@ __global__ void __launch_bounds__(256) detect_kernel(const float2* __restrict__ 
     float acc = 0.f;
     if (stokes) {
       for (long long m = 0; m < M; ++m) {
-        const float4 v = __ldg(reinterpret_cast<const float4*>(in + (j * M + m) * CP + 2 * e));
+        const float4 v = ld_pair<V4>(in + (j * M + m) * CP + 2 * e);
         // (XX) + (YY), each as re*re + im*im like the reference
         acc += (v.x * v.x + v.y * v.y) + (v.z * v.z + v.w * v.w);
       }
@@ -99,7 +128,11 @@ static inline cudaError_t launch_detect(const float2* in, float* out, long long 
   const long long total = rows * (stokes ? CP / 2 : CP);
   long long blocks = (total + 255) / 256;
   if (blocks > 148ll * 32) blocks = 148ll * 32;
-  detect_kernel<<<(unsigned)blocks, 256, 0, st>>>(in, out, rows, CP, stokes ? 1 : 0, M);
+  // the 128-bit Stokes loads read pol pairs at even complex offsets: a 16-byte aligned base suffices
+  if ((((uintptr_t)in) & 15) == 0)
+    detect_kernel<true><<<(unsigned)blocks, 256, 0, st>>>(in, out, rows, CP, stokes ? 1 : 0, M);
+  else
+    detect_kernel<false><<<(unsigned)blocks, 256, 0, st>>>(in, out, rows, CP, stokes ? 1 : 0, M);
   return cudaGetLastError();
 }
 
@@ -274,36 +307,38 @@ __global__ void __launch_bounds__(256) decimate2_kernel(const float2* __restrict
 // full Stokes [I, Q, U, V] from (A, B) pol pairs (core.py:937-966, PSR/IEEE convention)
 //   linear:   I=AA+BB  Q=AA-BB  U=2Re(A*B)  V=2Im(A*B)
 //   circular: I=AA+BB  Q=2Re(A*B)  U=2Im(A*B)  V=AA-BB          (A*B = conj(A) B)
-__global__ void __launch_bounds__(256) stokes_kernel(const float4* __restrict__ in,
-                                                     float4* __restrict__ out, long long n,
+template <bool V4>
+__global__ void __launch_bounds__(256) stokes_kernel(const float2* __restrict__ in,
+                                                     float* __restrict__ out, long long n,
                                                      int circular) {
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n;
        i += (long long)gridDim.x * blockDim.x) {
-    const float4 v = __ldg(in + i);  // (Are, Aim, Bre, Bim)
+    const float4 v = ld_pair<V4>(in + 2 * i);  // (Are, Aim, Bre, Bim)
     const float aa = v.x * v.x + v.y * v.y;
     const float bb = v.z * v.z + v.w * v.w;
     const float re = v.x * v.z + v.y * v.w;   // Re(conj(A) B)
     const float im = v.x * v.w - v.y * v.z;   // Im(conj(A) B)
-    out[i] = circular ? make_float4(aa + bb, 2.f * re, 2.f * im, aa - bb)
-                      : make_float4(aa + bb, aa - bb, 2.f * re, 2.f * im);
+    st_pair<V4>(out + 4 * i, circular ? make_float4(aa + bb, 2.f * re, 2.f * im, aa - bb)
+                                      : make_float4(aa + bb, aa - bb, 2.f * re, 2.f * im));
   }
 }
 
 // basis change (core.py:882-928): to_circular: [X - iY, X + iY]/sqrt2 ; to_linear: [L + R, i(L - R)]/sqrt2
-__global__ void __launch_bounds__(256) pol_basis_kernel(const float4* __restrict__ in,
-                                                        float4* __restrict__ out, long long n,
+template <bool V4>
+__global__ void __launch_bounds__(256) pol_basis_kernel(const float2* __restrict__ in,
+                                                        float2* __restrict__ out, long long n,
                                                         int to_circular) {
   const float h = 0.70710678118654752440f;
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n;
        i += (long long)gridDim.x * blockDim.x) {
-    const float4 v = __ldg(in + i);
+    const float4 v = ld_pair<V4>(in + 2 * i);
     float4 o;
     if (to_circular) {   // L = X - iY = (Xre + Yim, Xim - Yre); R = X + iY = (Xre - Yim, Xim + Yre)
       o = make_float4((v.x + v.w) * h, (v.y - v.z) * h, (v.x - v.w) * h, (v.y + v.z) * h);
     } else {             // X = L + R ; Y = i (L - R) = (-(Lim - Rim), Lre - Rre)
       o = make_float4((v.x + v.z) * h, (v.y + v.w) * h, -(v.y - v.w) * h, (v.x - v.z) * h);
     }
-    out[i] = o;
+    st_pair<V4>(reinterpret_cast<float*>(out + 2 * i), o);
   }
 }
 
