@@ -147,6 +147,35 @@ int pbk_dedisp_fold_exec_device(pbk_plan* plan, const void* d_in, void* d_profil
                                 const double* coeffs, int32_t ncoef, double sample_rate_hz,
                                 int64_t n0, int32_t nbin, void* stream);
 
+/* Coherent dedispersion of one block at ndm trial DMs (a coherent DM search, or refining the DM of
+ * a known pulsar): the forward transform of the input runs once per execution, and the chirp pass
+ * and every pass after it run once per trial.  `desc` means what it means for
+ * pbk_dedisp_plan_create, except that desc->dm is ignored: trial k uses dms[k] (any finite value,
+ * 0 and negative DMs included).  All trials share one crop, one downsample and one out_kind; raw
+ * int8 / u4 / u2 input works.  explicit_chirp, ndm < 1, a NULL dms and a non-finite DM return
+ * PBK_ERR_INVALID.  Each trial computes bit for bit what a pbk_dedisp_plan_create plan with the
+ * same desc and dm = dms[k] computes.
+ * Execute with pbk_dedisp_exec_device / pbk_dedisp_exec_host: out is a contiguous
+ * (ndm, rows, row_elems) array, trial k at out + k * rows * row_elems * elem_bytes, where
+ * pbk_dedisp_out_shape reports the shape of ONE trial.  A trial slab that is not 16-byte aligned
+ * is written through the plan's staging buffer.  The plan keeps a second scratch array for the
+ * shared forward result; the per-trial inverse passes run in place in the other one.  When every
+ * per-trial pass runs on the LDG fast kernels and has fewer tiles than the GPU holds CTAs, T > 1
+ * trials run as one launch (gridDim.y = T; the other array then holds T slabs), with T chosen by the
+ * plan for about two waves of CTAs and bounded by the memory of the slabs; otherwise T = 1.  The
+ * L2-blocked schedules ($PBK_L2_CHUNK_MB, $PBK_L2PIPE) are not used.  Lengths that are not powers
+ * of two (Bluestein) run their whole execution once per trial.  pbk_dedisp_fold_exec_device on a
+ * trial plan returns PBK_ERR_UNSUPPORTED.  pbk_plan_describe lists the shared passes, then
+ * "TRIALS:ndm=<ndm>:per_launch=<T>" and the passes run per batch of T trials; pbk_plan_info and
+ * pbk_plan_segments count the shared passes once and the per-trial launches once per batch, so
+ * launches = shared passes + ceil(ndm / T) x per-trial passes.  The last timed segment of a batch
+ * ends where the next batch's first launch starts, so it includes the zeroing of a time-summed
+ * output and the copy out of a staged output between them. */
+int pbk_dedisp_trials_plan_create(const pbk_dedisp_desc* desc, const double* dms, int32_t ndm,
+                                  pbk_plan** plan);
+/* number of trial DMs of a plan: ndm for a trial plan, 1 for every other plan */
+int pbk_plan_trials(const pbk_plan* plan, int32_t* ndm);
+
 /* ---- FFT-domain phase ramp / band mask ("next" rows: time_shift, freq_shift) ------------------
  * Replaces the core of transforms/transforms.py:268-271 (time_shift) and :348-361 (freq_shift):
  *   out[:, col] = ifft(fft(in[:, col]) * H_col),

@@ -17,7 +17,8 @@ EXPORTS = [
     "pbk_version", "pbk_last_error", "pbk_status_string", "pbk_device_count",
     "pbk_device_pci_bus_id", "pbk_device_mem_info", "pbk_phase_predict",
     "pbk_dedisp_plan_create", "pbk_dedisp_out_shape", "pbk_dedisp_exec_host",
-    "pbk_dedisp_exec_device", "pbk_dedisp_fold_exec_device", "pbk_fft_plan_create", "pbk_stft_plan_create", "pbk_stft_plan_create_raw",
+    "pbk_dedisp_exec_device", "pbk_dedisp_fold_exec_device", "pbk_dedisp_trials_plan_create",
+    "pbk_plan_trials", "pbk_fft_plan_create", "pbk_stft_plan_create", "pbk_stft_plan_create_raw",
     "pbk_stft_detect_plan_create", "pbk_stft_fold_exec_device",
     "pbk_dedisp_c128", "pbk_fft_c128", "pbk_stft_c128", "pbk_detect_c128",
     "pbk_fft_exec_host", "pbk_fft_exec_device", "pbk_detect", "pbk_detect_scrunch", "pbk_shift_channels", "pbk_downsample", "pbk_fold",
@@ -81,6 +82,9 @@ def lib():
         L.pbk_phase_predict.argtypes = [vp, i64, dbl, dbl, i64, ctypes.POINTER(dbl), i32, i64, vp,
                                         vp, i32, i32, vp]
         L.pbk_dedisp_plan_create.argtypes = [ctypes.POINTER(DedispDesc), ctypes.POINTER(vp)]
+        L.pbk_dedisp_trials_plan_create.argtypes = [ctypes.POINTER(DedispDesc),
+                                                     ctypes.POINTER(dbl), i32, ctypes.POINTER(vp)]
+        L.pbk_plan_trials.argtypes = [vp, ctypes.POINTER(i32)]
         L.pbk_dedisp_out_shape.argtypes = [vp] + [ctypes.POINTER(i64)] * 3
         L.pbk_dedisp_exec_host.argtypes = [vp, vp, vp, vp]
         L.pbk_dedisp_exec_device.argtypes = [vp, vp, vp, vp, vp]
@@ -233,7 +237,7 @@ class DedispPlan(Plan):
                        int(start), int(stop), int(downsample), int(bool(explicit_chirp)),
                        int(device))
         h = ctypes.c_void_p(0)
-        check(lib().pbk_dedisp_plan_create(ctypes.byref(d), ctypes.byref(h)))
+        self._create(d, h)
         super().__init__(h)
         rows, relems, ebytes = ctypes.c_int64(0), ctypes.c_int64(0), ctypes.c_int64(0)
         check(lib().pbk_dedisp_out_shape(h, ctypes.byref(rows), ctypes.byref(relems),
@@ -243,6 +247,9 @@ class DedispPlan(Plan):
         self.out_rows, self.row_elems, self.elem_bytes = rows.value, relems.value, ebytes.value
         self.explicit_chirp = bool(explicit_chirp)
         self.device = device
+
+    def _create(self, desc, h):
+        check(lib().pbk_dedisp_plan_create(ctypes.byref(desc), ctypes.byref(h)))
 
     def out_array(self, trailing=None):
         dt = np.complex64 if self.out_kind == OUT_C64 else np.float32
@@ -266,6 +273,32 @@ class DedispPlan(Plan):
             self.handle, ptr(d_in), ptr(d_profile), ptr(d_counts),
             c.ctypes.data_as(ctypes.POINTER(ctypes.c_double)), len(c), float(sample_rate_hz),
             int(n0), int(nbin), ctypes.c_void_p(stream)))
+
+
+class DedispTrialsPlan(DedispPlan):
+    """One block dedispersed at ``ndm`` trial DMs (pbk_dedisp_trials_plan_create): the forward
+    transform runs once per execution.  Takes DedispPlan's arguments with ``dms`` in place of
+    ``dm``; executions write (ndm, out_rows, ...) arrays."""
+
+    def __init__(self, *, dms, **kw):
+        self.dms = np.ascontiguousarray(dms, dtype=np.float64).reshape(-1)
+        self.ndm = len(self.dms)
+        super().__init__(dm=0.0, **kw)
+
+    def _create(self, desc, h):
+        check(lib().pbk_dedisp_trials_plan_create(
+            ctypes.byref(desc), self.dms.ctypes.data_as(ctypes.POINTER(ctypes.c_double)),
+            self.ndm, ctypes.byref(h)))
+
+    def out_array(self, trailing=None):
+        one = super().out_array(trailing)
+        return np.empty((self.ndm,) + one.shape, dtype=one.dtype)
+
+    def trials(self):
+        """pbk_plan_trials: the number of trial DMs."""
+        n = ctypes.c_int32(0)
+        check(lib().pbk_plan_trials(self.handle, ctypes.byref(n)))
+        return n.value
 
 
 class RampPlan(Plan):

@@ -171,6 +171,15 @@ struct pbk_plan {
   int l2_chunks = 0;            // 0 = plain pass-after-pass schedule
   long long l2_tiles[3] = {0, 0, 0};   // tiles per chunk of passes 1, 2, 3
   int segments = 0;             // timed segments per execution (pbk_plan_profile_read)
+  // trial plans (pbk_dedisp_trials_plan_create): the forward passes run once per execution, the
+  // MID pass and every pass after it once per trial DM, with that trial's chirp constants
+  bool trials = false;
+  int ndm = 1;
+  int nshared = 0;              // leading passes shared by all trials
+  std::vector<double> trial_D;  // PassArgs::D of each trial; d_chanconst holds ndm tables of 3C
+  long long chanconst_stride = 0;
+  int trials_per_launch = 1;    // T: trials batched along gridDim.y of each per-trial launch
+  size_t work_bytes = 0;        // the per-trial scratch array holds T slabs of scratch_bytes
   // optional per-launch device timing (pbk_plan_profile): ring of event sets, one per execution
   std::vector<std::vector<cudaEvent_t>> prof;
   long long prof_next = 0;
@@ -710,7 +719,7 @@ static int setup_l2pipe(pbk_plan* pl, int nblocks) {
 }
 static void blue_free(BlueState* b);
 static int blue_exec(pbk_plan* pl, const void* d_in, void* d_out, const void* d_chirp,
-                     cudaStream_t st);
+                     cudaStream_t st, int trial = -1);
 
 // scratch arrays are pair-planar ({re0,re1,im0,im1} per 16-byte lane pair) when the innermost
 // extent is even; every pass, generic or fast, reads and writes them through that layout
@@ -742,8 +751,19 @@ static int load_kind_of(int in_dtype) {
   }
 }
 
-static int dedisp_plan_create_impl(const pbk_dedisp_desc* d, const RampSpec* ramp, pbk_plan** out);
+// trial DMs of a trial plan; a single-DM plan passes {&desc->dm, 1, false}
+struct TrialSpec {
+  const double* dms;
+  int ndm;
+  bool trials;
+};
+
+static int dedisp_plan_create_impl(const pbk_dedisp_desc* d, const RampSpec* ramp,
+                                   const TrialSpec& tr, pbk_plan** out);
 static int blue_dedisp_plan_create(const pbk_dedisp_desc* d, const RampSpec* ramp, pbk_plan** out);
+
+// PassArgs::D of the chirp, dedispersion.py:30,46 in Hz^2 s
+static double chirp_D(double dm) { return (1.0 / 2.41e-4) * dm * 1e12; }
 
 // per-column ramp description (shift / N, zeroed band) on the device, owned by the plan
 static int upload_ramp(pbk_plan* pl, const RampSpec* ramp, long long C, long long N) {
@@ -764,7 +784,27 @@ static int upload_ramp(pbk_plan* pl, const RampSpec* ramp, long long C, long lon
 }
 
 extern "C" int pbk_dedisp_plan_create(const pbk_dedisp_desc* d, pbk_plan** out) {
-  return dedisp_plan_create_impl(d, nullptr, out);
+  if (!d) return fail(PBK_ERR_INVALID, "NULL argument");
+  return dedisp_plan_create_impl(d, nullptr, TrialSpec{&d->dm, 1, false}, out);
+}
+
+extern "C" int pbk_dedisp_trials_plan_create(const pbk_dedisp_desc* d, const double* dms,
+                                             int32_t ndm, pbk_plan** out) {
+  if (!d || !out || !dms) return fail(PBK_ERR_INVALID, "NULL argument");
+  *out = nullptr;
+  if (ndm < 1) return fail(PBK_ERR_INVALID, "ndm must be >= 1, got %d", (int)ndm);
+  if (d->explicit_chirp) return fail(PBK_ERR_INVALID, "trial plans generate their chirps");
+  for (int k = 0; k < ndm; ++k)
+    if (!std::isfinite(dms[k])) return fail(PBK_ERR_INVALID, "trial DM %d is not finite", k);
+  pbk_dedisp_desc h = *d;
+  h.dm = dms[0];
+  return dedisp_plan_create_impl(&h, nullptr, TrialSpec{dms, (int)ndm, true}, out);
+}
+
+extern "C" int pbk_plan_trials(const pbk_plan* pl, int32_t* ndm) {
+  if (!pl || !ndm) return fail(PBK_ERR_INVALID, "NULL argument");
+  *ndm = pl->ndm;
+  return PBK_OK;
 }
 
 extern "C" int pbk_ramp_plan_create(int64_t nsamp, int64_t ncols, const double* shift_samples,
@@ -789,10 +829,73 @@ extern "C" int pbk_ramp_plan_create(int64_t nsamp, int64_t ncols, const double* 
   d.downsample = 1;
   d.device = device;
   RampSpec r{shift_samples, zero_lo, zero_hi, flags};
-  return dedisp_plan_create_impl(&d, &r, plan);
+  return dedisp_plan_create_impl(&d, &r, TrialSpec{&d.dm, 1, false}, plan);
 }
 
-static int dedisp_plan_create_impl(const pbk_dedisp_desc* d, const RampSpec* ramp, pbk_plan** out) {
+// Trials per launch.  A per-trial pass of a small block has fewer tiles than the GPU holds CTAs
+// (one 2^20-sample column: 128 tiles on 148 SMs), so T trials that share the forward result run as
+// one launch with gridDim.y = T: just enough for two waves of resident CTAs in every per-trial
+// pass, bounded by the memory of T scratch slabs (the 1/5-of-device rule of the second scratch
+// array).  Only the LDG fast kernels take a trial index; a per-trial pass on the generic, TMA or
+// warp-private kernels, a Bluestein length, a one-level plan (its MID pass reads the caller's
+// input), an output staged through d_tmpf and a slab that is not a multiple of 16 bytes keep T = 1.
+static int choose_trials_per_launch(const pbk_plan* pl) {
+  if (pl->blue || pl->nshared == 0 || pl->split_ragged || pl->out_bytes % 16 ||
+      pl->passes.back().out_role != ROLE_USER_OUT)
+    return 1;
+  long long want = 1;
+  for (size_t i = pl->nshared; i < pl->passes.size(); ++i) {
+    const Pass& ps = pl->passes[i];
+    if (ps.family < 0 || ps.tma || ps.tsumw || ps.ntiles <= 0) return 1;
+    const long long resident = (long long)pl->num_sms * ps.finfo.minb;
+    want = std::max(want, (2 * resident + ps.ntiles - 1) / ps.ntiles);
+  }
+  size_t free_b = 0, total_b = 0;
+  if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) {
+    cudaGetLastError();
+    return 1;
+  }
+  long long T = std::min<long long>(want, pl->ndm);
+  while (T > 1 && (size_t)T * pl->scratch_bytes > total_b / 5) --T;
+  return (int)T;
+}
+
+// the trial fields of a plan whose passes (or Bluestein state) are built: trials per launch, the
+// per-trial scratch slabs, launch and segment counts for the trial schedule (see run_trial_passes)
+static int set_trials(pbk_plan* pl, const TrialSpec& tr) {
+  pl->trials = true;
+  pl->ndm = tr.ndm;
+  pl->trial_D.resize(tr.ndm);
+  for (int k = 0; k < tr.ndm; ++k) pl->trial_D[k] = chirp_D(tr.dms[k]);
+  if (pl->blue) {
+    pl->launches *= tr.ndm;
+    return PBK_OK;
+  }
+  const int ds = (pl->desc.downsample > 1 && !pl->fused_tsum) ? 1 : 0;
+  pl->nshared = pl->nlevels - 1;
+  pl->trials_per_launch = choose_trials_per_launch(pl);
+  if (pl->nshared > 0) {
+    // the per-trial passes work in buffer nshared & 1 of the ping-pong pair
+    void*& work = (pl->nshared & 1) ? pl->scratch2 : pl->scratch;
+    if (pl->work_bytes == 0) pl->work_bytes = pl->scratch_bytes;
+    const size_t need = (size_t)pl->trials_per_launch * pl->scratch_bytes;
+    if (need > pl->work_bytes) {
+      cudaFree(work);
+      work = nullptr;
+      pl->work_bytes = 0;
+      CUDA_TRY(cudaMalloc(&work, need));
+      pl->work_bytes = need;
+    }
+  }
+  const int per = (int)pl->passes.size() - pl->nshared + ds;
+  const int batches = (tr.ndm + pl->trials_per_launch - 1) / pl->trials_per_launch;
+  pl->launches = pl->nshared + batches * per;
+  pl->segments = pl->launches;
+  return PBK_OK;
+}
+
+static int dedisp_plan_create_impl(const pbk_dedisp_desc* d, const RampSpec* ramp,
+                                   const TrialSpec& tr, pbk_plan** out) {
   if (!d || !out) return fail(PBK_ERR_INVALID, "NULL argument");
   *out = nullptr;
   if (d->nsamp <= 0 || d->nchan <= 0 || d->npol <= 0)
@@ -834,7 +937,7 @@ static int dedisp_plan_create_impl(const pbk_dedisp_desc* d, const RampSpec* ram
     h.crop_start = d->crop_start / 2;           // whole (even, odd) rows covering the crop
     h.crop_stop = (d->crop_stop + 1) / 2;
     pbk_plan* pl = nullptr;
-    const int rc = dedisp_plan_create_impl(&h, nullptr, &pl);
+    const int rc = dedisp_plan_create_impl(&h, nullptr, tr, &pl);
     if (rc == PBK_OK) {
       bool all_fast = true;
       for (auto& ps : pl->passes) all_fast = all_fast && ps.family >= 0;
@@ -862,6 +965,11 @@ static int dedisp_plan_create_impl(const pbk_dedisp_desc* d, const RampSpec* ram
           }
           pl->split_ragged = true;
         }
+        int rs;
+        if (tr.trials && (rs = set_trials(pl, tr)) != PBK_OK) {   // again, for this geometry
+          pbk_plan_destroy(pl);
+          return rs;
+        }
         *out = pl;
         return PBK_OK;
       }
@@ -872,7 +980,9 @@ static int dedisp_plan_create_impl(const pbk_dedisp_desc* d, const RampSpec* ram
     // not a power of two (or shorter than 16): Bluestein on top of the power-of-two passes
     if (d->nsamp < 2)
       return fail(PBK_ERR_UNSUPPORTED, "nsamp = %lld is too short", (long long)d->nsamp);
-    return blue_dedisp_plan_create(d, ramp, out);
+    const int rc = blue_dedisp_plan_create(d, ramp, out);
+    if (rc == PBK_OK && tr.trials) set_trials(*out, tr);   // the whole execution runs per trial
+    return rc;
   }
   int l[3] = {0, 0, 0};
   const long long I = d->nchan * d->npol;
@@ -970,7 +1080,7 @@ static int dedisp_plan_create_impl(const pbk_dedisp_desc* d, const RampSpec* ram
       ps.a.df = 1.0 / ((double)N * dt);               // numpy fftfreq: val = 1/(n*d)
       if (std::isinf(d->ref_freq_hz)) { ps.a.fr_sub = 0; ps.a.inv_fr = 0; ps.a.a0 = -1.0; }
       else { ps.a.fr_sub = d->ref_freq_hz; ps.a.inv_fr = 1.0 / d->ref_freq_hz; ps.a.a0 = 0; }
-      ps.a.D = (1.0 / 2.41e-4) * d->dm * 1e12;        // dedispersion.py:30,46 in Hz^2 s
+      ps.a.D = chirp_D(d->dm);
     }
     ps.a.scale = (float)(1.0 / (double)N);
     ps.a.chirp_sk = C;
@@ -1052,16 +1162,21 @@ static int dedisp_plan_create_impl(const pbk_dedisp_desc* d, const RampSpec* ram
                           cudaGetErrorString(e)));
   }
   {
-    // constants of the division-free chirp (pbk_fast.cuh: fast_chirp), in long double on the host
-    std::vector<double> cc((size_t)C * 3);
+    // constants of the division-free chirp (pbk_fast.cuh: fast_chirp), in long double on the host;
+    // a trial plan holds one table per trial DM, each computed as its single-DM plan computes it
+    std::vector<double> cc((size_t)C * 3 * tr.ndm);
     const long double fr = d->ref_freq_hz, df = (long double)d->sample_rate_hz / (long double)N;
-    const long double Dl = (1.0L / 2.41e-4L) * (long double)d->dm * 1e12L;
-    for (long long c = 0; c < C; ++c) {
-      const long double fc = d->chan_freq_hz[c];
-      cc[3 * c + 0] = std::isinf(d->ref_freq_hz) ? -1.0 : (double)((fc - fr) / fr);
-      cc[3 * c + 1] = (double)(df / fc);
-      cc[3 * c + 2] = (double)(Dl / fc);
+    for (int k = 0; k < tr.ndm; ++k) {
+      const long double Dl = (1.0L / 2.41e-4L) * (long double)tr.dms[k] * 1e12L;
+      double* t = cc.data() + (size_t)k * 3 * C;
+      for (long long c = 0; c < C; ++c) {
+        const long double fc = d->chan_freq_hz[c];
+        t[3 * c + 0] = std::isinf(d->ref_freq_hz) ? -1.0 : (double)((fc - fr) / fr);
+        t[3 * c + 1] = (double)(df / fc);
+        t[3 * c + 2] = (double)(Dl / fc);
+      }
     }
+    pl->chanconst_stride = 3 * C;
     cudaError_t e = cudaMalloc(&pl->d_chanconst, cc.size() * sizeof(double));
     if (e == cudaSuccess)
       e = cudaMemcpy(pl->d_chanconst, cc.data(), cc.size() * sizeof(double),
@@ -1079,8 +1194,9 @@ static int dedisp_plan_create_impl(const pbk_dedisp_desc* d, const RampSpec* ram
     ps.a.bd = std::isinf(d->ref_freq_hz) ? 0.0
                                          : (d->sample_rate_hz / (double)N) / d->ref_freq_hz;
   }
-  if (m == 3) setup_l2_blocking(pl, (N >> l[0]) * I * 8, 1 << l[0]);
-  if (m == 3 && (rc = setup_l2pipe(pl, 1 << l[0])) != PBK_OK) return cleanup(rc);
+  // trial plans take the plain schedule: FWD level 2 sits inside the L2-blocked groups
+  if (m == 3 && !tr.trials) setup_l2_blocking(pl, (N >> l[0]) * I * 8, 1 << l[0]);
+  if (m == 3 && !tr.trials && (rc = setup_l2pipe(pl, 1 << l[0])) != PBK_OK) return cleanup(rc);
   // Out-of-place intermediate passes: a pass that reads and writes the same scratch array is
   // 2-3 % slower than one that writes another array (cfg2: 1.505 -> 1.463 ms and 1.476 -> 1.426 ms,
   // profiles/r01_pingpong_scratch.log), so when the scratch is small against the device memory
@@ -1098,6 +1214,15 @@ static int dedisp_plan_create_impl(const pbk_dedisp_desc* d, const RampSpec* ram
       pl->scratch2 = nullptr;
     cudaGetLastError();
   }
+  if (tr.trials && pl->scratch && !pl->scratch2) {
+    // the forward result must survive every trial: the per-trial passes work in the other array
+    cudaError_t e = cudaMalloc(&pl->scratch2, pl->scratch_bytes);
+    if (e != cudaSuccess) {
+      pl->scratch2 = nullptr;
+      return cleanup(fail(PBK_ERR_NOMEM, "second scratch (%zu bytes): %s", pl->scratch_bytes,
+                          cudaGetErrorString(e)));
+    }
+  }
   if (pl->l2_chunks == 0) setup_tma(pl);
   const int ds = (d->downsample > 1 && !pl->fused_tsum) ? 1 : 0;
   if (pl->l2pipe) {
@@ -1110,6 +1235,7 @@ static int dedisp_plan_create_impl(const pbk_dedisp_desc* d, const RampSpec* ram
     pl->launches = (int)pl->passes.size() + ds;
     pl->segments = pl->launches;
   }
+  if (tr.trials && (rc = set_trials(pl, tr)) != PBK_OK) return cleanup(rc);
   *out = pl;
   return PBK_OK;
 }
@@ -1162,11 +1288,14 @@ static int stage_ensure(pbk_plan* pl, size_t bytes) {
 
 static int launch_one(pbk_plan* pl, const Pass& ps, const void* d_in, void* d_out,
                       const void* d_chirp, long long tile0, long long tile_end, cudaStream_t st,
-                      int idx = 0) {
+                      int idx = 0, void* scr_in = nullptr, void* scr_out = nullptr) {
   Pass p = ps;
   p.a.in = role_ptr(pl, ps.in_role, d_in, d_out);
   p.a.out = role_ptr(pl, ps.out_role, d_in, d_out);
-  if (pl->scratch2) {   // pass idx reads buffer (idx-1)&1 and writes buffer idx&1
+  if (scr_in || scr_out) {   // the trial schedule names its scratch arrays (run_trial_passes)
+    if (ps.in_role == ROLE_SCRATCH) p.a.in = scr_in;
+    if (ps.out_role == ROLE_SCRATCH) p.a.out = scr_out;
+  } else if (pl->scratch2) {   // pass idx reads buffer (idx-1)&1 and writes buffer idx&1
     void* buf[2] = {pl->scratch, pl->scratch2};
     if (ps.in_role == ROLE_SCRATCH) p.a.in = buf[(idx + 1) & 1];
     if (ps.out_role == ROLE_SCRATCH) p.a.out = buf[idx & 1];
@@ -1182,6 +1311,9 @@ static int launch_one(pbk_plan* pl, const Pass& ps, const void* d_in, void* d_ou
                 ps.mode == MODE_FWD ? "FWD" : ps.mode == MODE_MID ? "MID" : "INV",
                 ps.a.tsum_log2 > 0 ? "time-sum" : ps.a.fsum_log2 > 0 ? "detection" : "even/odd",
                 p.a.in, p.a.out);
+  if (p.a.trials > 1 && (ps.tma || ps.family < 0 || !aligned))
+    return fail(PBK_ERR_UNSUPPORTED, "a batch of %d trials needs the LDG fast kernels and 16-byte "
+                "aligned arrays", p.a.trials);
   cudaError_t e;
   CUtensorMap tm;
   if (ps.tma && aligned && tile0 == 0 && tile_end < 0 && tma_encode(ps, p.a.in, &tm)) {
@@ -1268,6 +1400,46 @@ static int run_passes(pbk_plan* pl, const void* d_in, void* d_out, const void* d
   return PBK_OK;
 }
 
+// Trial schedule.  The shared forward passes run once, ping-ponging between the two scratch arrays
+// as in the plain schedule; their result stays where the last of them wrote it.  Each batch of up
+// to T trials then runs MID from that result into the other array (slab y of T for trial k0 + y),
+// the inverse passes in place there, and the last pass into its output slabs.  One-level plans
+// share nothing: every trial reads the caller's input.
+static int run_shared_passes(pbk_plan* pl, const void* d_in, cudaStream_t st) {
+  for (int i = 0; i < pl->nshared; ++i) {
+    prof_mark(pl, i, st);
+    const int rc = launch_one(pl, pl->passes[i], d_in, nullptr, nullptr, 0, -1, st, i);
+    if (rc != PBK_OK) return rc;
+  }
+  return PBK_OK;
+}
+
+static int run_trial_passes(pbk_plan* pl, const void* d_in, void* d_out, cudaStream_t st, int k,
+                            int t, int seg) {
+  const int ns = pl->nshared;
+  void* buf[2] = {pl->scratch, pl->scratch2};
+  void* shared = ns > 0 ? buf[(ns - 1) & 1] : nullptr;
+  void* work = ns > 0 ? buf[ns & 1] : nullptr;
+  for (size_t i = ns; i < pl->passes.size(); ++i) {
+    Pass q = pl->passes[i];
+    q.a.D = pl->trial_D[k];
+    q.a.chan_const = pl->d_chanconst + (size_t)k * pl->chanconst_stride;
+    if (t > 1) {   // trials k .. k + t - 1 along gridDim.y (choose_trials_per_launch)
+      q.a.trials = t;
+      q.a.trial_cc = pl->chanconst_stride;
+      q.a.trial_in_bytes = (int)i == ns ? 0 : (long long)pl->scratch_bytes;
+      q.a.trial_out_bytes = q.out_role == ROLE_USER_OUT ? (long long)pl->out_bytes
+                                                        : (long long)pl->scratch_bytes;
+    }
+    prof_mark(pl, seg++, st);
+    const int rc = launch_one(pl, q, d_in, d_out, nullptr, 0, -1, st, (int)i,
+                              (int)i == ns ? shared : work, work);
+    if (rc != PBK_OK) return rc;
+  }
+  prof_mark(pl, seg, st);
+  return PBK_OK;
+}
+
 // decide whether the L2-blocked schedule applies (called once the fast kernels are chosen)
 static void setup_l2_blocking(pbk_plan* pl, long long block_bytes, int nblocks) {
   pl->l2_chunks = 0;
@@ -1291,6 +1463,9 @@ static void setup_l2_blocking(pbk_plan* pl, long long block_bytes, int nblocks) 
   pl->l2_chunks = chunks;
 }
 
+static int exec_dedisp(pbk_plan* pl, const void* d_in, void* d_out, const void* d_chirp,
+                       cudaStream_t st, int trial);
+
 extern "C" int pbk_dedisp_exec_device(pbk_plan* pl, const void* d_in, void* d_out,
                                       const void* d_chirp, void* stream) {
   if (!pl || pl->kind != PLAN_DEDISP) return fail(PBK_ERR_INVALID, "not a dedispersion plan");
@@ -1300,20 +1475,58 @@ extern "C" int pbk_dedisp_exec_device(pbk_plan* pl, const void* d_in, void* d_ou
   if (!d_out) return fail(PBK_ERR_INVALID, "output pointer is NULL");
   CUDA_TRY(cudaSetDevice(pl->device));
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  if (pl->blue) return blue_exec(pl, d_in, d_out, d_chirp, st);
+  if (!pl->trials) {
+    if (pl->blue) return blue_exec(pl, d_in, d_out, d_chirp, st);
+    return exec_dedisp(pl, d_in, d_out, d_chirp, st, -1);
+  }
+  // trial k writes the slab out + k * out_bytes
+  char* out = static_cast<char*>(d_out);
+  int rc;
+  if (pl->blue) {
+    for (int k = 0; k < pl->ndm; ++k)
+      if ((rc = blue_exec(pl, d_in, out + (size_t)k * pl->out_bytes, nullptr, st, k)) != PBK_OK)
+        return rc;
+    return PBK_OK;
+  }
+  prof_begin(pl);
+  if ((rc = run_shared_passes(pl, d_in, st)) != PBK_OK) return rc;
+  const int T = pl->trials_per_launch;
+  for (int b = 0; b * T < pl->ndm; ++b)
+    if ((rc = exec_dedisp(pl, d_in, out + (size_t)b * T * pl->out_bytes, nullptr, st, b)) != PBK_OK)
+      return rc;
+  return PBK_OK;
+}
+
+// One execution of a plan (batch < 0), or batch `batch` of a trial plan whose shared passes have
+// run (trials batch * T .. on), into d_out.
+static int exec_dedisp(pbk_plan* pl, const void* d_in, void* d_out, const void* d_chirp,
+                       cudaStream_t st, int batch) {
+  const int trial = batch < 0 ? -1 : batch * pl->trials_per_launch;
+  const int ntr = batch < 0 ? 1 : std::min(pl->trials_per_launch, pl->ndm - trial);
+  const size_t out_bytes = (size_t)ntr * pl->out_bytes;
   void* dst = pl->split_ragged ? pl->d_tmpf : d_out;
-  const bool stage = last_pass_needs_fast(pl) && misaligned16(dst);
+  // A trial slab is only element-aligned when the slab size is not a multiple of 16 bytes; it is
+  // staged whenever the caller's output would be, so that every trial runs on the kernels an
+  // aligned single-DM execution takes and gives the same bits.
+  const bool stage = misaligned16(dst) &&
+                     (trial < 0 ? last_pass_needs_fast(pl)
+                                : pl->passes.back().out_role == ROLE_USER_OUT);
   int rc;
   if (stage) {
-    if ((rc = stage_ensure(pl, pl->out_bytes)) != PBK_OK) return rc;
+    if ((rc = stage_ensure(pl, out_bytes)) != PBK_OK) return rc;
     dst = pl->d_stage;
   }
   if (pl->fused_tsum)   // the last pass adds its group sums to the output
-    CUDA_TRY(cudaMemsetAsync(dst, 0, pl->out_bytes, st));
-  rc = run_passes(pl, d_in, dst, d_chirp, st);
+    CUDA_TRY(cudaMemsetAsync(dst, 0, out_bytes, st));
+  // timed segments of this execution (or batch): [seg0, seg0 + per)
+  const int batches = (pl->ndm + pl->trials_per_launch - 1) / pl->trials_per_launch;
+  const int per = trial < 0 ? pl->segments : (pl->segments - pl->nshared) / batches;
+  const int seg0 = trial < 0 ? 0 : pl->nshared + batch * per;
+  rc = trial < 0 ? run_passes(pl, d_in, dst, d_chirp, st)
+                 : run_trial_passes(pl, d_in, dst, st, trial, ntr, seg0);
   if (rc != PBK_OK) return rc;
   if (stage)
-    CUDA_TRY(cudaMemcpyAsync(d_out, pl->d_stage, pl->out_bytes, cudaMemcpyDeviceToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(d_out, pl->d_stage, out_bytes, cudaMemcpyDeviceToDevice, st));
   if (pl->split_ragged)
     CUDA_TRY(cudaMemcpyAsync(d_out, static_cast<const char*>(pl->d_tmpf) + pl->split_skip,
                              pl->out_bytes, cudaMemcpyDeviceToDevice, st));
@@ -1322,7 +1535,7 @@ extern "C" int pbk_dedisp_exec_device(pbk_plan* pl, const void* d_in, void* d_ou
                                       reinterpret_cast<float*>(d_out), pl->out_rows,
                                       pl->row_elems, pl->desc.downsample, st);
     if (e != cudaSuccess) return fail(PBK_ERR_CUDA, "downsample launch: %s", cudaGetErrorString(e));
-    prof_mark(pl, pl->segments, st);
+    prof_mark(pl, seg0 + per, st);
   }
   return PBK_OK;
 }
@@ -1343,6 +1556,7 @@ extern "C" int pbk_dedisp_fold_exec_device(pbk_plan* pl, const void* d_in, void*
                                            double sample_rate_hz, int64_t n0, int32_t nbin,
                                            void* stream) {
   if (!pl || pl->kind != PLAN_DEDISP) return fail(PBK_ERR_INVALID, "not a dedispersion plan");
+  if (pl->trials) return fail(PBK_ERR_UNSUPPORTED, "folding a trial plan is not supported");
   if (pl->desc.out_kind != PBK_OUT_INTENSITY && pl->desc.out_kind != PBK_OUT_STOKES_I)
     return fail(PBK_ERR_INVALID, "folding needs a plan with out_kind INTENSITY or STOKES_I");
   if (pl->desc.explicit_chirp) return fail(PBK_ERR_INVALID, "folding takes no explicit chirp");
@@ -1417,8 +1631,9 @@ extern "C" int pbk_dedisp_exec_host(pbk_plan* pl, const void* in, void* out, con
   std::lock_guard<std::mutex> lock(pl->mu);
   CUDA_TRY(cudaSetDevice(pl->device));
   int rc;
+  const size_t out_bytes = pl->out_bytes * pl->ndm;   // a trial plan writes ndm slabs
   if ((rc = ensure_buf(&pl->h_din, pl->in_bytes)) != PBK_OK) return rc;
-  if ((rc = ensure_buf(&pl->h_dout, pl->out_bytes)) != PBK_OK) return rc;
+  if ((rc = ensure_buf(&pl->h_dout, out_bytes)) != PBK_OK) return rc;
   if ((rc = ensure_buf(&pl->h_dchirp, pl->chirp_bytes)) != PBK_OK) return rc;
   cudaStream_t st = cudaStreamPerThread;
   // pageable blocks go through the multi-threaded bounce pipeline (pbk_hostcopy.h)
@@ -1426,7 +1641,7 @@ extern "C" int pbk_dedisp_exec_host(pbk_plan* pl, const void* in, void* out, con
   if (pl->chirp_bytes) CUDA_TRY(host_to_device(pl->h_dchirp, chirp, pl->chirp_bytes, st));
   rc = pbk_dedisp_exec_device(pl, pl->h_din, pl->h_dout, pl->h_dchirp, st);
   if (rc != PBK_OK) return rc;
-  CUDA_TRY(device_to_host(out, pl->h_dout, pl->out_bytes, st));
+  CUDA_TRY(device_to_host(out, pl->h_dout, out_bytes, st));
   return PBK_OK;
 }
 
@@ -1713,8 +1928,9 @@ static int blue_convolve(BlueState* b, bool conj, cudaStream_t st) {
   return run_passes(b->invM, b->B, b->A, nullptr, st);
 }
 
+// (trial >= 0: the chirp of that trial of a trial plan)
 static int blue_exec(pbk_plan* pl, const void* d_in, void* d_out, const void* d_chirp,
-                     cudaStream_t st) {
+                     cudaStream_t st, int trial) {
   BlueState* b = pl->blue;
   const long long total = b->O * b->M * b->I;
   cudaError_t e = launch_grid(blue_pre_kernel, total, st, d_in, b->A, (const float2*)b->w, b->in);
@@ -1724,6 +1940,7 @@ static int blue_exec(pbk_plan* pl, const void* d_in, void* d_out, const void* d_
   if (b->dedisp) {
     PassArgs ch = b->chirp;
     ch.chirp_arr = reinterpret_cast<const float2*>(d_chirp);
+    if (trial >= 0) ch.D = pl->trial_D[trial];
     e = launch_grid(blue_midH_kernel, b->M * b->I, st, b->A, b->n, b->M, b->I, b->P, ch);
     if (e != cudaSuccess) return fail(PBK_ERR_CUDA, "bluestein chirp: %s", cudaGetErrorString(e));
     if ((rc = blue_convolve(b, true, st)) != PBK_OK) return rc;
@@ -1790,7 +2007,7 @@ static int blue_dedisp_plan_create(const pbk_dedisp_desc* d, const RampSpec* ram
   b->chirp.df = 1.0 / ((double)N * (1.0 / d->sample_rate_hz));
   if (std::isinf(d->ref_freq_hz)) { b->chirp.fr_sub = 0; b->chirp.inv_fr = 0; b->chirp.a0 = -1.0; }
   else { b->chirp.fr_sub = d->ref_freq_hz; b->chirp.inv_fr = 1.0 / d->ref_freq_hz; b->chirp.a0 = 0; }
-  b->chirp.D = (1.0 / 2.41e-4) * d->dm * 1e12;
+  b->chirp.D = chirp_D(d->dm);
   b->chirp.scale = 1.0f;
   b->chirp.chirp_sk = C;
   b->chirp.chirp_sc = 1;
@@ -2090,7 +2307,9 @@ extern "C" int pbk_plan_info(const pbk_plan* pl, int32_t* launches, int64_t* wor
   if (!pl) return fail(PBK_ERR_INVALID, "plan is NULL");
   if (launches) *launches = pl->launches;
   if (workspace_bytes) *workspace_bytes =
-      (int64_t)(pl->scratch_bytes * (pl->scratch2 ? 2 : 1) + pl->tmpf_bytes + pl->fold_bytes +
+      (int64_t)(pl->scratch_bytes * (pl->scratch2 ? 2 : 1) +
+                (pl->work_bytes > pl->scratch_bytes ? pl->work_bytes - pl->scratch_bytes : 0) +
+                pl->tmpf_bytes + pl->fold_bytes +
                 pl->stage_bytes);
   if (levels) *levels = pl->nlevels;
   if (level_log2)
@@ -2105,15 +2324,27 @@ extern "C" int pbk_plan_describe(const pbk_plan* pl, char* buf, size_t n) {
   if (pl->blue) {
     snprintf(buf, n, "BLUESTEIN:n=%lld:M=2^%d:lanes=%lld", pl->blue->n, ilog2_exact(pl->blue->M),
              pl->blue->I);
+    if (pl->trials) {
+      off = strlen(buf);
+      snprintf(buf + off, n - off, ":trials=%d:per_launch=%d", pl->ndm, pl->trials_per_launch);
+    }
     return PBK_OK;
   }
   for (size_t i = 0; i < pl->passes.size() && off + 1 < n; ++i) {
     const Pass& ps = pl->passes[i];
     const char* mode = ps.mode == MODE_FWD ? "FWD" : ps.mode == MODE_MID ? "MID" : "INV";
     int w;
+    // a trial plan lists its shared passes, then "TRIALS" and the passes that run per trial
+    if (pl->trials && (int)i == pl->nshared) {
+      w = snprintf(buf + off, n - off, "%sTRIALS:ndm=%d:per_launch=%d", i == 0 ? "" : ";",
+                   pl->ndm, pl->trials_per_launch);
+      if (w < 0 || off + (size_t)w + 1 >= n) break;
+      off += (size_t)w;
+    }
     // segments are separated by ';'; the passes of an L2-blocked group are joined by '+'
     const bool blocked = pl->l2_chunks > 0 || pl->l2pipe;
-    const char* sep = i == 0 ? "" : (blocked && (i == 2 || i == 3)) ? "+" : ";";
+    const bool first = i == 0 && !(pl->trials && pl->nshared == 0);
+    const char* sep = first ? "" : (blocked && (i == 2 || i == 3)) ? "+" : ";";
     if (ps.family >= 0)
       w = snprintf(buf + off, n - off, "%s%s:L=2^%d:%s:W=%d:tiles=%lld:threads=%d%s%s", sep,
                    mode, ps.a.log2L, ps.tsumw ? "tmaw-r16" : ps.tma ? "tma-r16" : "fast-r16",

@@ -335,15 +335,24 @@ __device__ __forceinline__ float2 fast_chirp_value(const PassArgs& p, const doub
 
 // TWOCH: single-polarisation data (P = 1) -- the two lanes of a pair are two adjacent channels,
 // each with its own chirp; otherwise the pair is the two pols of one channel and shares it.
+// Trial index of a batched trial-plan launch (blockIdx.y).  Read where it is used, so that the
+// compiler does not keep it (and the offsets built from it) live across the tile loop.
+__device__ __forceinline__ long long trial_y() {
+  unsigned y;
+  asm volatile("mov.u32 %0, %%ctaid.y;" : "=r"(y));
+  return (long long)y;
+}
+
 template <int R, class C, bool TWOCH>
 __device__ __forceinline__ void fast_chirp(const PassArgs& p, const FastTile& T, c2* v, int klo) {
   const double k0 = (double)((long long)T.klow + ((long long)klo << p.log2Kmul));
   const double Nd = (double)p.N;
   double cc0[3], cc1[3];
+  const double* cc = p.chan_const + trial_y() * p.trial_cc + 3 * T.chan;
 #pragma unroll
   for (int i = 0; i < 3; ++i) {
-    cc0[i] = p.chan_const[3 * T.chan + i];
-    cc1[i] = TWOCH ? p.chan_const[3 * (T.chan + 1) + i] : 0.0;
+    cc0[i] = cc[i];
+    cc1[i] = TWOCH ? cc[3 + i] : 0.0;
   }
   if (TWOCH && p.split) {
     // ONE column of length 2N whose even / odd samples are the two lanes (radix-2 decimation in
@@ -772,6 +781,10 @@ fast_pass_kernel(const __grid_constant__ PassArgs p, const float2* __restrict__ 
       const TileInfo ti = *sinfo;
       T.gin = reinterpret_cast<const char*>(p.in) + ti.bi + off_in;
       T.gout = reinterpret_cast<char*>(p.out) + ti.bo + off_out;
+      if constexpr (MODE != MODE_FWD) {   // trial plans batch the MID and INV passes
+        T.gin += trial_y() * p.trial_in_bytes;
+        T.gout += trial_y() * p.trial_out_bytes;
+      }
       if constexpr (TSUM) {
         // ti.bo = (nrest - crop_start) rows + the column offset; keep the column part only
         char* colbase = T.gout - ((long long)ti.nrest - p.crop_start) * ts_rowbytes;

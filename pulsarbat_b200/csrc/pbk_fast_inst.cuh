@@ -42,7 +42,8 @@ static cudaError_t cfg_launch_variant(const PassArgs& a, const float2* d_tables,
   }
   if (MODE == MODE_FWD && EPI == EPI_INTENSITY)   // whole groups of 2^fsum_g_log2 tiles per CTA
     grid = (unsigned)std::min<long long>(std::max<long long>(1, ntiles >> a.fsum_g_log2), resident);
-  return pdl_launch(kern, dim3(grid), dim3(C::NT), smem, st, a, d_tables, ntiles);
+  return pdl_launch(kern, dim3(grid, std::max(1, a.trials)), dim3(C::NT), smem, st, a, d_tables,
+                    ntiles);
 }
 
 // NARROW (arrays with fewer lanes per row than the tile is wide) is a separate instantiation so

@@ -24,7 +24,7 @@ from .device import DeviceArray
 
 __all__ = ["default_device", "dedisperse", "chirp", "detect", "shift_channels", "phase_ramp", "mix", "analytic_decimate", "stokes", "pol_basis",
            "downsample", "fft", "stft", "istft", "stft_detect", "stft_fold", "fold",
-           "dedisperse_fold", "predict_phase", "clear_plan_cache",
+           "dedisperse_fold", "dedisperse_trials", "predict_phase", "clear_plan_cache",
            "pinned_results"]
 
 
@@ -287,6 +287,44 @@ def dedisperse(data, *, dm, sample_rate_hz, chan_freq_hz, ref_freq_hz, crop=None
                                 chirp_array, raw is not None, g.raw_np, dev)
 
 
+def dedisperse_trials(data, *, dms, sample_rate_hz, chan_freq_hz, ref_freq_hz, crop=None,
+                      out_kind=L.OUT_INTENSITY, downsample=1, raw=None, raw_shape=None,
+                      device=None):
+    """:func:`dedisperse` of one block at every DM of ``dms``, stacked: returns an array shaped
+    (len(dms), rows, nchan, ...) (Stokes I drops the pol axis) whose element k equals
+    ``dedisperse(data, dm=dms[k], ...)`` bit for bit.  The forward transform of the block runs once
+    for all trials (pbk_dedisp_trials_plan_create); all trials share ``crop``, ``out_kind`` and
+    ``downsample``.  ``data``, ``raw`` and ``raw_shape`` are as in :func:`dedisperse`: numpy in
+    gives numpy out, a DeviceArray gives a DeviceArray without a host round trip.  complex128
+    runs the FP64 :func:`dedisperse` once per DM (nothing shared)."""
+    dms = tuple(float(v) for v in np.asarray(dms, dtype=np.float64).reshape(-1))
+    if not dms:
+        raise ValueError("dms must hold at least one DM")
+    g = _DedispGeometry(data, raw, raw_shape, crop)
+    dev = (data.device if _is_dev(data) else (default_device() if device is None else device))
+    if raw is None and _is_c128(data):
+        ys = [_dedisperse_c128(data, g.nsamp, g.nchan, g.npol, g.trailing, dm, sample_rate_hz,
+                               g.freqs(chan_freq_hz), ref_freq_hz, g.start, g.stop, out_kind,
+                               downsample, None, dev) for dm in dms]
+        if _is_dev(data):
+            import torch
+            return DeviceArray(torch.stack([y.tensor for y in ys]))
+        return np.stack(ys)
+    freqs = g.freqs(chan_freq_hz)
+    # keyed by the DM tuple: the cache's byte cap sees the plan's workspace like any other
+    key = ("dedisp_trials", g.nsamp, g.nchan, g.npol, g.raw, int(out_kind), dms,
+           float(sample_rate_hz), float(ref_freq_hz), freqs.tobytes(), g.start, g.stop,
+           int(downsample), dev)
+    ctx = _use_plan(key, lambda: L.DedispTrialsPlan(
+        dms=dms, nsamp=g.nsamp, nchan=g.nchan, npol=g.npol, sample_rate_hz=sample_rate_hz,
+        ref_freq_hz=ref_freq_hz, chan_freq_hz=freqs, crop=(g.start, g.stop),
+        in_dtype=g.in_dtype, out_kind=out_kind, downsample=downsample, device=dev))
+    with ctx as plan:
+        # recount: an execution may have allocated the staging buffer
+        return _dedisperse_with(ctx, plan, data, g.nsamp, g.nchan, g.trailing, out_kind, None,
+                                raw is not None, g.raw_np, dev, lead=(len(dms),), recount=True)
+
+
 class _DedispGeometry:
     """Shape, input kind and crop of a dedispersion call (``raw`` / ``raw_shape`` / ``crop`` as in
     :func:`dedisperse`), and the cached plan for it."""
@@ -444,9 +482,9 @@ def _dedisperse_c128(data, nsamp, nchan, npol, trailing, dm, sample_rate_hz, fre
 
 
 def _dedisperse_with(ent, plan, data, nsamp, nchan, trailing, out_kind, chirp_array, int8, raw_np,
-                     dev):
+                     dev, lead=(), recount=False):
     out_trailing = (nchan,) if out_kind == L.OUT_STOKES_I else (nchan,) + trailing
-    out_shape = (plan.out_rows,) + out_trailing
+    out_shape = lead + (plan.out_rows,) + out_trailing
 
     if _is_dev(data):
         x = data.contiguous()
@@ -461,6 +499,8 @@ def _dedisperse_with(ent, plan, data, nsamp, nchan, trailing, out_kind, chirp_ar
                                      dtype=np.complex64), dev)
         with ent.lock:
             plan.exec_device(x.ptr, out.ptr, None if ch is None else ch.ptr, _stream())
+            if recount:
+                _recount(ent.ent)
         return out
 
     if int8:
@@ -474,6 +514,8 @@ def _dedisperse_with(ent, plan, data, nsamp, nchan, trailing, out_kind, chirp_ar
                                   dtype=np.complex64)
     with ent.lock:
         plan.exec_host(x, out, ch)
+        if recount:
+            _recount(ent.ent)
     if out_kind == L.OUT_C64:
         return out if odt == np.complex64 else out.astype(odt)
     rdt = _real_of(odt)

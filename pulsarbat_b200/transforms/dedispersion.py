@@ -16,7 +16,7 @@ from .. import units as u
 from ..core import BasebandSignal, IntensitySignal, RadioSignal
 
 __all__ = ["DispersionMeasure", "DM", "coherent_dedispersion", "incoherent_dedispersion",
-           "dedisperse_detect", "overlap_save_dedispersion"]
+           "dedisperse_detect", "dedisperse_trials", "overlap_save_dedispersion"]
 
 #: s MHz^2 cm^3 / pc -- dedispersion.py:30
 DISPERSION_CONSTANT = 1.0 / 2.41e-4
@@ -229,6 +229,66 @@ def dedisperse_detect(z, DM, /, *, ref_freq=None, stokes_I=False, downsample=1, 
     if downsample > 1:
         kw["sample_rate"] = z.sample_rate / downsample
     return _cropped_like(IntensitySignal, z, x, max(start, 0), **kw)
+
+
+def as_dm_list(DMs):
+    """A sequence of DM values or DispersionMeasures as a list of DispersionMeasures."""
+    if isinstance(DMs, (str, bytes)) or np.ndim(DMs) != 1:
+        raise TypeError("DMs must be a one-dimensional sequence of dispersion measures")
+    out = [_as_dm(d) for d in DMs]
+    if not out:
+        raise ValueError("DMs must hold at least one dispersion measure")
+    return out
+
+
+def common_crop_range(z, DMs, ref_freq, nsamp=None):
+    """(start, stop) valid for every DM of ``DMs``: the intersection of their :func:`crop_range`,
+    i.e. the latest start and the earliest stop.  ``stop <= start`` when it is empty."""
+    ranges = [crop_range(z, dm, ref_freq, nsamp) for dm in DMs]
+    return max(r[0] for r in ranges), min(r[1] for r in ranges)
+
+
+def dedisperse_trials(z, DMs, /, *, ref_freq=None, detect=True, stokes_I=False, downsample=1,
+                      crop=True):
+    """Coherently dedisperse one block at several trial DMs (a DM search, or refining the DM of a
+    known pulsar), sharing the forward FFT of the block between the trials.
+
+    Returns a list with one signal per DM: ``IntensitySignal`` objects (per-pol power, or Stokes I
+    with ``stokes_I=True``, summed over ``downsample`` samples), or ``type(z)`` voltages with
+    ``detect=False``.  Their data are views of one stacked array.  With ``crop=True`` all trials
+    share one crop, the intersection of every DM's crop (:func:`common_crop_range`), so every row
+    is valid for every trial and all results have the same ``start_time`` and length; element k
+    then equals ``dedisperse_detect(z, DMs[k])`` cut to that crop.  An empty intersection gives
+    zero-row results.  ``z`` may be a ``(raw_int8, template_signal)`` tuple as in
+    :func:`dedisperse_detect`.  Dask input raises ``TypeError``.
+    """
+    raw = None
+    if isinstance(z, tuple):
+        raw, z = z
+    if not isinstance(z, BasebandSignal):
+        raise TypeError("Signal must be a BasebandSignal object.")
+    DMs = as_dm_list(DMs)
+    if not detect and (downsample > 1 or stokes_I):
+        raise ValueError("downsample and stokes_I need detect=True")
+    src = z.data if raw is None else raw
+    if _dask.is_dask(src):
+        raise TypeError("dedisperse_trials takes numpy or DeviceArray blocks (a dask array: "
+                        "compute the block first, or call dedisperse_detect per chunk)")
+    if ref_freq is None:
+        ref_freq = z.center_freq
+    start, stop = common_crop_range(z, DMs, ref_freq) if crop else (0, len(z))
+    kind = (L.OUT_C64 if not detect else L.OUT_STOKES_I if stokes_I else L.OUT_INTENSITY)
+    x = kernels.dedisperse_trials(src, dms=[d.dm for d in DMs], sample_rate_hz=z.sample_rate_hz,
+                                  chan_freq_hz=z.channel_freqs_hz, ref_freq_hz=_hz(ref_freq),
+                                  crop=(start, stop), out_kind=kind, downsample=downsample,
+                                  raw=None if raw is None else "int8")
+    if not detect:
+        start = min(start, len(z)) if stop <= start else start
+        return [_cropped_like(type(z), z, x[k], start) for k in range(len(DMs))]
+    kw = {"chan_bw": z.chan_bw}
+    if downsample > 1:
+        kw["sample_rate"] = z.sample_rate / downsample
+    return [_cropped_like(IntensitySignal, z, x[k], max(start, 0), **kw) for k in range(len(DMs))]
 
 
 def overlap_save_dedispersion(z, DM, block_len, /, *, ref_freq=None):
