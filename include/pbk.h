@@ -176,6 +176,32 @@ int pbk_dedisp_trials_plan_create(const pbk_dedisp_desc* desc, const double* dms
 /* number of trial DMs of a plan: ndm for a trial plan, 1 for every other plan */
 int pbk_plan_trials(const pbk_plan* plan, int32_t* ndm);
 
+/* Overlap-save execution of a pbk_dedisp_plan_create plan over nblocks blocks of one
+ * device-resident stream (builder-defined, SURVEY 8a row O).  With advance = crop_stop - crop_start
+ * and an input row of nchan * npol elements of in_dtype (row bytes = nchan * npol * bits / 8, so
+ * int8, u4 and u2 rows work), block b reads the plan's nsamp rows starting at row b * advance of
+ * d_in and writes the plan's normal output at d_out + b * rows * row_elems * elem_bytes
+ * (pbk_dedisp_out_shape): d_in must hold (nblocks - 1) * advance + nsamp rows and d_out nblocks
+ * output slabs.  Block b is bit for bit what pbk_dedisp_exec_device writes into a 16-byte aligned
+ * buffer from d_in + b * advance * row bytes.  Enqueue only, like pbk_dedisp_exec_device.
+ * nblocks == 0 or an empty crop returns PBK_OK and touches nothing; nblocks < 0 or a NULL pointer
+ * returns PBK_ERR_INVALID; a trial plan or an explicit-chirp plan returns PBK_ERR_UNSUPPORTED.
+ * When d_in, d_out and the block stride (advance * row bytes) are 16-byte aligned and the plan can
+ * batch (pbk_plan_blocks_per_launch > 1), T blocks run as one launch per pass (gridDim.y = T) and
+ * a time-summed output is zeroed once per batch; the last batch may be partial.  The T scratch
+ * slabs of each scratch array are allocated at the first batched execution and counted in
+ * pbk_plan_info's workspace bytes.  Otherwise each block runs the single execution at its pointers,
+ * with an output slab that is not 16-byte aligned written through the staging buffer.
+ * pbk_plan_profile does not time block executions. */
+int pbk_dedisp_exec_blocks_device(pbk_plan* plan, const void* d_in, int64_t nblocks, void* d_out,
+                                  void* stream);
+/* Blocks batched per launch (T) by pbk_dedisp_exec_blocks_device on a 16-byte aligned stream: about
+ * two waves of resident CTAs in every pass, bounded by the memory of T slabs in each scratch array;
+ * 1 when the plan cannot batch (a pass on the generic, TMA or warp-private kernels, a Bluestein
+ * length, a one-level plan, the L2-blocked schedules, an output through the float buffer or a slab
+ * that is not a multiple of 16 bytes), and for trial and ramp plans. */
+int pbk_plan_blocks_per_launch(const pbk_plan* plan, int32_t* T);
+
 /* ---- FFT-domain phase ramp / band mask ("next" rows: time_shift, freq_shift) ------------------
  * Replaces the core of transforms/transforms.py:268-271 (time_shift) and :348-361 (freq_shift):
  *   out[:, col] = ifft(fft(in[:, col]) * H_col),

@@ -18,7 +18,8 @@ EXPORTS = [
     "pbk_device_pci_bus_id", "pbk_device_mem_info", "pbk_phase_predict",
     "pbk_dedisp_plan_create", "pbk_dedisp_out_shape", "pbk_dedisp_exec_host",
     "pbk_dedisp_exec_device", "pbk_dedisp_fold_exec_device", "pbk_dedisp_trials_plan_create",
-    "pbk_plan_trials", "pbk_fft_plan_create", "pbk_stft_plan_create", "pbk_stft_plan_create_raw",
+    "pbk_plan_trials", "pbk_dedisp_exec_blocks_device", "pbk_plan_blocks_per_launch",
+    "pbk_fft_plan_create", "pbk_stft_plan_create", "pbk_stft_plan_create_raw",
     "pbk_stft_detect_plan_create", "pbk_stft_fold_exec_device",
     "pbk_dedisp_c128", "pbk_fft_c128", "pbk_stft_c128", "pbk_detect_c128",
     "pbk_fft_exec_host", "pbk_fft_exec_device", "pbk_detect", "pbk_detect_scrunch", "pbk_shift_channels", "pbk_downsample", "pbk_fold",
@@ -85,6 +86,8 @@ def lib():
         L.pbk_dedisp_trials_plan_create.argtypes = [ctypes.POINTER(DedispDesc),
                                                      ctypes.POINTER(dbl), i32, ctypes.POINTER(vp)]
         L.pbk_plan_trials.argtypes = [vp, ctypes.POINTER(i32)]
+        L.pbk_dedisp_exec_blocks_device.argtypes = [vp, vp, i64, vp, vp]
+        L.pbk_plan_blocks_per_launch.argtypes = [vp, ctypes.POINTER(i32)]
         L.pbk_dedisp_out_shape.argtypes = [vp] + [ctypes.POINTER(i64)] * 3
         L.pbk_dedisp_exec_host.argtypes = [vp, vp, vp, vp]
         L.pbk_dedisp_exec_device.argtypes = [vp, vp, vp, vp, vp]
@@ -264,6 +267,19 @@ class DedispPlan(Plan):
     def exec_device(self, d_in, d_out, d_chirp=None, stream=0):
         check(lib().pbk_dedisp_exec_device(self.handle, ptr(d_in), ptr(d_out), ptr(d_chirp),
                                            ctypes.c_void_p(stream)))
+
+    def exec_blocks_device(self, d_in, nblocks, d_out, stream=0):
+        """Overlap-save execution over ``nblocks`` blocks of one device stream
+        (pbk_dedisp_exec_blocks_device): block b reads the plan's nsamp rows from row
+        b * (crop_stop - crop_start) of ``d_in`` and writes output slab b of ``d_out``."""
+        check(lib().pbk_dedisp_exec_blocks_device(self.handle, ptr(d_in), int(nblocks),
+                                                  ptr(d_out), ctypes.c_void_p(stream)))
+
+    def blocks_per_launch(self):
+        """pbk_plan_blocks_per_launch: blocks batched per launch on a 16-byte aligned stream."""
+        n = ctypes.c_int32(0)
+        check(lib().pbk_plan_blocks_per_launch(self.handle, ctypes.byref(n)))
+        return n.value
 
     def fold_device(self, d_in, d_profile, d_counts, coeffs, sample_rate_hz, n0, nbin, stream=0):
         """Dedisperse, detect, time-sum and fold one block (pbk_dedisp_fold_exec_device);

@@ -180,17 +180,25 @@ struct pbk_plan {
   long long chanconst_stride = 0;
   int trials_per_launch = 1;    // T: trials batched along gridDim.y of each per-trial launch
   size_t work_bytes = 0;        // the per-trial scratch array holds T slabs of scratch_bytes
+  // overlap-save blocks (pbk_dedisp_exec_blocks_device) of a single-DM plan
+  int blocks_per_launch = 1;    // T: blocks batched along gridDim.y (choose_per_launch)
+  // T slabs of scratch_bytes per scratch array the plan uses, allocated at the first batched
+  // execution
+  void* blk_scratch[2] = {nullptr, nullptr};
+  size_t blk_bytes = 0;
   // optional per-launch device timing (pbk_plan_profile): ring of event sets, one per execution
   std::vector<std::vector<cudaEvent_t>> prof;
   long long prof_next = 0;
   int prof_cur = -1;
+  bool prof_off = false;        // block executions are not timed
 };
 
 static void prof_mark(pbk_plan* pl, int idx, cudaStream_t st) {
   if (pl->prof_cur >= 0) cudaEventRecord(pl->prof[pl->prof_cur][idx], st);
 }
 static void prof_begin(pbk_plan* pl) {
-  pl->prof_cur = pl->prof.empty() ? -1 : (int)(pl->prof_next++ % (long long)pl->prof.size());
+  pl->prof_cur = (pl->prof.empty() || pl->prof_off)
+                     ? -1 : (int)(pl->prof_next++ % (long long)pl->prof.size());
 }
 
 static int ilog2_exact(int64_t v) {
@@ -832,19 +840,22 @@ extern "C" int pbk_ramp_plan_create(int64_t nsamp, int64_t ncols, const double* 
   return dedisp_plan_create_impl(&d, &r, TrialSpec{&d.dm, 1, false}, plan);
 }
 
-// Trials per launch.  A per-trial pass of a small block has fewer tiles than the GPU holds CTAs
-// (one 2^20-sample column: 128 tiles on 148 SMs), so T trials that share the forward result run as
-// one launch with gridDim.y = T: just enough for two waves of resident CTAs in every per-trial
-// pass, bounded by the memory of T scratch slabs (the 1/5-of-device rule of the second scratch
-// array).  Only the LDG fast kernels take a trial index; a per-trial pass on the generic, TMA or
-// warp-private kernels, a Bluestein length, a one-level plan (its MID pass reads the caller's
-// input), an output staged through d_tmpf and a slab that is not a multiple of 16 bytes keep T = 1.
-static int choose_trials_per_launch(const pbk_plan* pl) {
-  if (pl->blue || pl->nshared == 0 || pl->split_ragged || pl->out_bytes % 16 ||
-      pl->passes.back().out_role != ROLE_USER_OUT)
+// Executions per launch: the trials of a trial plan, or the overlap-save blocks of a single-DM
+// plan (pbk_dedisp_exec_blocks_device).  A pass of a small block has fewer tiles than the GPU holds
+// CTAs (one 2^20-sample column: 128 tiles on 148 SMs), so T executions of the batched passes
+// [first, end) run as one launch with gridDim.y = T: just enough for two waves of resident CTAs in
+// every batched pass, at most `limit`, and bounded by the memory of T scratch slabs in each of the
+// `nbuf` batched scratch arrays (together within the 1/5-of-device rule of the second scratch
+// array).  Only the LDG fast kernels take a batch index; a batched pass on the generic, TMA or
+// warp-private kernels, the L2-blocked schedules, a Bluestein length, a one-level plan (a trial's
+// MID pass would read the caller's input), an output staged through d_tmpf and a slab that is not
+// a multiple of 16 bytes keep T = 1.
+static int choose_per_launch(const pbk_plan* pl, size_t first, long long limit, int nbuf) {
+  if (pl->blue || pl->nlevels < 2 || pl->l2pipe || pl->l2_chunks > 0 || pl->split_ragged ||
+      pl->out_bytes % 16 || pl->passes.back().out_role != ROLE_USER_OUT)
     return 1;
   long long want = 1;
-  for (size_t i = pl->nshared; i < pl->passes.size(); ++i) {
+  for (size_t i = first; i < pl->passes.size(); ++i) {
     const Pass& ps = pl->passes[i];
     if (ps.family < 0 || ps.tma || ps.tsumw || ps.ntiles <= 0) return 1;
     const long long resident = (long long)pl->num_sms * ps.finfo.minb;
@@ -855,9 +866,15 @@ static int choose_trials_per_launch(const pbk_plan* pl) {
     cudaGetLastError();
     return 1;
   }
-  long long T = std::min<long long>(want, pl->ndm);
-  while (T > 1 && (size_t)T * pl->scratch_bytes > total_b / 5) --T;
+  long long T = std::min<long long>(want, limit);
+  while (T > 1 && (size_t)T * nbuf * pl->scratch_bytes > total_b / 5) --T;
   return (int)T;
+}
+
+// Blocks per launch of a single-DM plan: every pass is batched, in the plan's scratch arrays
+// (both of a ping-pong pair), up to the grid's y limit.
+static void set_blocks_per_launch(pbk_plan* pl) {
+  pl->blocks_per_launch = choose_per_launch(pl, 0, 65535, pl->scratch2 ? 2 : 1);
 }
 
 // the trial fields of a plan whose passes (or Bluestein state) are built: trials per launch, the
@@ -873,7 +890,7 @@ static int set_trials(pbk_plan* pl, const TrialSpec& tr) {
   }
   const int ds = (pl->desc.downsample > 1 && !pl->fused_tsum) ? 1 : 0;
   pl->nshared = pl->nlevels - 1;
-  pl->trials_per_launch = choose_trials_per_launch(pl);
+  pl->trials_per_launch = choose_per_launch(pl, pl->nshared, pl->ndm, 1);
   if (pl->nshared > 0) {
     // the per-trial passes work in buffer nshared & 1 of the ping-pong pair
     void*& work = (pl->nshared & 1) ? pl->scratch2 : pl->scratch;
@@ -970,6 +987,7 @@ static int dedisp_plan_create_impl(const pbk_dedisp_desc* d, const RampSpec* ram
           pbk_plan_destroy(pl);
           return rs;
         }
+        if (!tr.trials) set_blocks_per_launch(pl);             // again, for this geometry
         *out = pl;
         return PBK_OK;
       }
@@ -1236,6 +1254,7 @@ static int dedisp_plan_create_impl(const pbk_dedisp_desc* d, const RampSpec* ram
     pl->segments = pl->launches;
   }
   if (tr.trials && (rc = set_trials(pl, tr)) != PBK_OK) return cleanup(rc);
+  if (!tr.trials && !ramp) set_blocks_per_launch(pl);
   *out = pl;
   return PBK_OK;
 }
@@ -1464,7 +1483,7 @@ static void setup_l2_blocking(pbk_plan* pl, long long block_bytes, int nblocks) 
 }
 
 static int exec_dedisp(pbk_plan* pl, const void* d_in, void* d_out, const void* d_chirp,
-                       cudaStream_t st, int trial);
+                       cudaStream_t st, int batch, bool stage_any = false);
 
 extern "C" int pbk_dedisp_exec_device(pbk_plan* pl, const void* d_in, void* d_out,
                                       const void* d_chirp, void* stream) {
@@ -1498,9 +1517,10 @@ extern "C" int pbk_dedisp_exec_device(pbk_plan* pl, const void* d_in, void* d_ou
 }
 
 // One execution of a plan (batch < 0), or batch `batch` of a trial plan whose shared passes have
-// run (trials batch * T .. on), into d_out.
+// run (trials batch * T .. on), into d_out.  stage_any: stage an output that is not 16-byte aligned
+// whenever the last pass writes it, as batches of trials always do (see below).
 static int exec_dedisp(pbk_plan* pl, const void* d_in, void* d_out, const void* d_chirp,
-                       cudaStream_t st, int batch) {
+                       cudaStream_t st, int batch, bool stage_any) {
   const int trial = batch < 0 ? -1 : batch * pl->trials_per_launch;
   const int ntr = batch < 0 ? 1 : std::min(pl->trials_per_launch, pl->ndm - trial);
   const size_t out_bytes = (size_t)ntr * pl->out_bytes;
@@ -1509,8 +1529,8 @@ static int exec_dedisp(pbk_plan* pl, const void* d_in, void* d_out, const void* 
   // staged whenever the caller's output would be, so that every trial runs on the kernels an
   // aligned single-DM execution takes and gives the same bits.
   const bool stage = misaligned16(dst) &&
-                     (trial < 0 ? last_pass_needs_fast(pl)
-                                : pl->passes.back().out_role == ROLE_USER_OUT);
+                     (trial < 0 && !stage_any ? last_pass_needs_fast(pl)
+                                              : pl->passes.back().out_role == ROLE_USER_OUT);
   int rc;
   if (stage) {
     if ((rc = stage_ensure(pl, out_bytes)) != PBK_OK) return rc;
@@ -1537,6 +1557,101 @@ static int exec_dedisp(pbk_plan* pl, const void* d_in, void* d_out, const void* 
     if (e != cudaSuccess) return fail(PBK_ERR_CUDA, "downsample launch: %s", cudaGetErrorString(e));
     prof_mark(pl, seg0 + per, st);
   }
+  return PBK_OK;
+}
+
+// Overlap-save blocks b0 .. b0 + t - 1 of a stream as one launch per pass (gridDim.y = t): block
+// b0 + y reads the stream at in + y * stride, works in slab y of the block scratch arrays
+// (ping-ponging between them as run_passes does between the plan's own) and writes out + y * slab.
+static int run_block_batch(pbk_plan* pl, const char* in, char* out, int t, size_t stride,
+                           cudaStream_t st) {
+  if (pl->fused_tsum)   // the last pass adds its group sums to the output
+    CUDA_TRY(cudaMemsetAsync(out, 0, (size_t)t * pl->out_bytes, st));
+  void* const* buf = pl->blk_scratch;
+  for (size_t i = 0; i < pl->passes.size(); ++i) {
+    Pass q = pl->passes[i];
+    q.a.trials = t;
+    q.a.trial_in_bytes = q.in_role == ROLE_USER_IN ? (long long)stride
+                                                   : (long long)pl->scratch_bytes;
+    q.a.trial_out_bytes = q.out_role == ROLE_USER_OUT ? (long long)pl->out_bytes
+                                                      : (long long)pl->scratch_bytes;
+    void* scr_in = buf[1] ? buf[(i + 1) & 1] : buf[0];
+    void* scr_out = buf[1] ? buf[i & 1] : buf[0];
+    const int rc = launch_one(pl, q, in, out, nullptr, 0, -1, st, (int)i, scr_in, scr_out);
+    if (rc != PBK_OK) return rc;
+  }
+  return PBK_OK;
+}
+
+// T slabs in each scratch array the plan uses, for batched block executions
+static int blocks_scratch_ensure(pbk_plan* pl) {
+  if (pl->blk_scratch[0]) return PBK_OK;
+  const size_t bytes = (size_t)pl->blocks_per_launch * pl->scratch_bytes;
+  void* b[2] = {nullptr, nullptr};
+  for (int j = 0; j < (pl->scratch2 ? 2 : 1); ++j) {
+    const cudaError_t e = cudaMalloc(&b[j], bytes);
+    if (e != cudaSuccess) {
+      cudaFree(b[0]);
+      return fail(PBK_ERR_NOMEM, "block scratch (%zu bytes): %s", bytes, cudaGetErrorString(e));
+    }
+  }
+  pl->blk_scratch[0] = b[0];
+  pl->blk_scratch[1] = b[1];
+  pl->blk_bytes = bytes;
+  return PBK_OK;
+}
+
+extern "C" int pbk_dedisp_exec_blocks_device(pbk_plan* pl, const void* d_in, int64_t nblocks,
+                                             void* d_out, void* stream) {
+  if (!pl || pl->kind != PLAN_DEDISP) return fail(PBK_ERR_INVALID, "not a dedispersion plan");
+  if (!d_in) return fail(PBK_ERR_INVALID, "input pointer is NULL");
+  if (nblocks < 0)
+    return fail(PBK_ERR_INVALID, "nblocks must be >= 0, got %lld", (long long)nblocks);
+  if (pl->trials)
+    return fail(PBK_ERR_UNSUPPORTED, "block execution of a trial plan is not supported");
+  if (pl->desc.explicit_chirp)
+    return fail(PBK_ERR_UNSUPPORTED, "block execution of an explicit-chirp plan is not supported");
+  if (nblocks == 0 || pl->out_rows == 0) return PBK_OK;
+  if (!d_out) return fail(PBK_ERR_INVALID, "output pointer is NULL");
+  CUDA_TRY(cudaSetDevice(pl->device));
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  const pbk_dedisp_desc& d = pl->desc;
+  const size_t in_row = ((size_t)d.nchan * d.npol * load_bits(load_kind_of(d.in_dtype))) >> 3;
+  const size_t stride = (size_t)(d.crop_stop - d.crop_start) * in_row;
+  const char* in = static_cast<const char*>(d_in);
+  char* out = static_cast<char*>(d_out);
+  const int T = (misaligned16(in) || misaligned16(out) || stride % 16) ? 1 : pl->blocks_per_launch;
+  struct ProfOff {   // pbk_plan_profile times single executions only
+    pbk_plan* pl;
+    explicit ProfOff(pbk_plan* p) : pl(p) { pl->prof_off = true; }
+    ~ProfOff() { pl->prof_off = false; }
+  } prof_off(pl);
+  int rc;
+  if (T == 1) {
+    // the single execution at each block's pointers; an output slab that is not 16-byte aligned
+    // is staged so that every block runs on the kernels of an aligned execution
+    for (int64_t b = 0; b < nblocks; ++b) {
+      const char* bi = in + (size_t)b * stride;
+      char* bo = out + (size_t)b * pl->out_bytes;
+      rc = pl->blue ? blue_exec(pl, bi, bo, nullptr, st)
+                    : exec_dedisp(pl, bi, bo, nullptr, st, -1, true);
+      if (rc != PBK_OK) return rc;
+    }
+    return PBK_OK;
+  }
+  if ((rc = blocks_scratch_ensure(pl)) != PBK_OK) return rc;
+  for (int64_t b0 = 0; b0 < nblocks; b0 += T) {
+    const int t = (int)std::min<int64_t>(T, nblocks - b0);
+    rc = run_block_batch(pl, in + (size_t)b0 * stride, out + (size_t)b0 * pl->out_bytes, t, stride,
+                         st);
+    if (rc != PBK_OK) return rc;
+  }
+  return PBK_OK;
+}
+
+extern "C" int pbk_plan_blocks_per_launch(const pbk_plan* pl, int32_t* T) {
+  if (!pl || !T) return fail(PBK_ERR_INVALID, "NULL argument");
+  *T = pl->blocks_per_launch;
   return PBK_OK;
 }
 
@@ -2285,6 +2400,8 @@ extern "C" void pbk_plan_destroy(pbk_plan* pl) {
   blue_free(pl->blue);
   cudaFree(pl->scratch);
   cudaFree(pl->scratch2);
+  cudaFree(pl->blk_scratch[0]);
+  cudaFree(pl->blk_scratch[1]);
   cudaFree(pl->d_tw);
   cudaFree(pl->d_ftab);
   cudaFree(pl->d_chanfreq);
@@ -2309,6 +2426,7 @@ extern "C" int pbk_plan_info(const pbk_plan* pl, int32_t* launches, int64_t* wor
   if (workspace_bytes) *workspace_bytes =
       (int64_t)(pl->scratch_bytes * (pl->scratch2 ? 2 : 1) +
                 (pl->work_bytes > pl->scratch_bytes ? pl->work_bytes - pl->scratch_bytes : 0) +
+                pl->blk_bytes * ((pl->blk_scratch[0] ? 1 : 0) + (pl->blk_scratch[1] ? 1 : 0)) +
                 pl->tmpf_bytes + pl->fold_bytes +
                 pl->stage_bytes);
   if (levels) *levels = pl->nlevels;

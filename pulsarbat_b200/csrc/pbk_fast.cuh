@@ -335,8 +335,9 @@ __device__ __forceinline__ float2 fast_chirp_value(const PassArgs& p, const doub
 
 // TWOCH: single-polarisation data (P = 1) -- the two lanes of a pair are two adjacent channels,
 // each with its own chirp; otherwise the pair is the two pols of one channel and shares it.
-// Trial index of a batched trial-plan launch (blockIdx.y).  Read where it is used, so that the
-// compiler does not keep it (and the offsets built from it) live across the tile loop.
+// Batch index (blockIdx.y) of a batched launch: the trial of a trial plan, or the overlap-save
+// block of pbk_dedisp_exec_blocks_device.  Read where it is used, so that the compiler does not
+// keep it (and the offsets built from it) live across the tile loop.
 __device__ __forceinline__ long long trial_y() {
   unsigned y;
   asm volatile("mov.u32 %0, %%ctaid.y;" : "=r"(y));
@@ -737,7 +738,19 @@ fast_pass_kernel(const __grid_constant__ PassArgs p, const float2* __restrict__ 
   const long long t_step = (TSUM || FSUM) ? 1 : gridDim.x;
   pdl_trigger();
   for (int i = tid; i < C::TW_TOTAL; i += C::NT) tws[i] = tables[i];
-  if (tid == 0 && t < t_end) fast_tile_info<C, EPI>(p, tile_at(t), *sinfo, in_bits, out_eb);
+  // Batched launches offset each tile by the batch index (trial plans batch the MID and INV
+  // passes, overlap-save blocks every pass).  In FWD kernels thread 0 adds the offsets to the tile
+  // record: added to every thread's pointers, they spill 16 bytes in the 256-point FWD kernels at
+  // the 128-register cap.  MID and INV kernels add them to the pointers (below), which spills less
+  // there than the record does.
+  auto tile_info = [&](long long tile) {
+    fast_tile_info<C, EPI>(p, tile, *sinfo, in_bits, out_eb);
+    if constexpr (MODE == MODE_FWD) {
+      sinfo->bi += trial_y() * p.trial_in_bytes;
+      sinfo->bo += trial_y() * p.trial_out_bytes;
+    }
+  };
+  if (tid == 0 && t < t_end) tile_info(tile_at(t));
   __syncthreads();
   pdl_wait();   // the previous pass's output (and the array this pass overwrites) from here on
 
@@ -781,7 +794,7 @@ fast_pass_kernel(const __grid_constant__ PassArgs p, const float2* __restrict__ 
       const TileInfo ti = *sinfo;
       T.gin = reinterpret_cast<const char*>(p.in) + ti.bi + off_in;
       T.gout = reinterpret_cast<char*>(p.out) + ti.bo + off_out;
-      if constexpr (MODE != MODE_FWD) {   // trial plans batch the MID and INV passes
+      if constexpr (MODE != MODE_FWD) {   // (FWD: in the tile record, see tile_info)
         T.gin += trial_y() * p.trial_in_bytes;
         T.gout += trial_y() * p.trial_out_bytes;
       }
@@ -835,7 +848,7 @@ fast_pass_kernel(const __grid_constant__ PassArgs p, const float2* __restrict__ 
     // the next tile's record, which the end-of-tile barrier publishes
 #define PBK_NEXT_TILE_INFO()                                                        \
   if (tid == 0 && t + t_step < t_end)                                               \
-    fast_tile_info<C, EPI>(p, tile_at(t + t_step), *sinfo, in_bits, out_eb)
+    tile_info(tile_at(t + t_step))
     if (MODE == MODE_INV) PBK_NEXT_TILE_INFO();
 
     if (MODE == MODE_FWD) {

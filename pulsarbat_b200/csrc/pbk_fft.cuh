@@ -159,10 +159,11 @@ struct PassArgs {
   long long fsum_cells;   // output cells per segment (row length of `out` in cells)
   int split;          // fast MID pass, P == 1: the lane pair is the even / odd samples of ONE column
                       // of length 2N (see fast_chirp); N, df and the tables are the half length's
-  // trial plans (pbk_dedisp_trials_plan_create): a launch of the fast kernels with gridDim.y = trials
-  // runs trial blockIdx.y with its input at in + y * trial_in_bytes, its output at
-  // out + y * trial_out_bytes and its chirp constants at chan_const + y * trial_cc.  Zero / one
-  // trial by default: single-DM launches compute what they always did.
+  // batched launches of trial plans (pbk_dedisp_trials_plan_create) and overlap-save blocks
+  // (pbk_dedisp_exec_blocks_device, trial_cc = 0): a launch of the LDG fast kernels with
+  // gridDim.y = trials runs batch element blockIdx.y with its input at in + y * trial_in_bytes, its
+  // output at out + y * trial_out_bytes and its chirp constants at chan_const + y * trial_cc.  Zero
+  // / one by default: single launches compute what they always did.
   long long trial_in_bytes, trial_out_bytes, trial_cc;
   int trials;         // host side: gridDim.y of a fast launch (0 or 1 = one trial)
 };

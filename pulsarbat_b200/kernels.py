@@ -325,11 +325,54 @@ def dedisperse_trials(data, *, dms, sample_rate_hz, chan_freq_hz, ref_freq_hz, c
                                 raw is not None, g.raw_np, dev, lead=(len(dms),), recount=True)
 
 
+def dedisperse_overlap_save(data, *, block_len, dm, sample_rate_hz, chan_freq_hz, ref_freq_hz,
+                            crop, out_kind=L.OUT_C64, downsample=1, raw=None, raw_shape=None):
+    """Overlap-save dedispersion of a device-resident stream: blocks of ``block_len`` rows that
+    advance by ``crop[1] - crop[0]`` rows, each dedispersed as :func:`dedisperse` with that
+    ``crop``, ``out_kind`` and ``downsample``, stacked into one DeviceArray shaped
+    (nblocks * rows, nchan, ...) (Stokes I drops the pol axis), with no host round trip.  Block b
+    starts at row b * advance and equals ``dedisperse(data[b * advance:][:block_len], ...)`` bit for
+    bit; a tail that does not fill a block is dropped.  ``data`` is a complex64 DeviceArray, or raw
+    baseband with ``raw`` / ``raw_shape`` as in :func:`dedisperse`.  All blocks run as one library
+    call (pbk_dedisp_exec_blocks_device) on the plan :func:`dedisperse` caches for one block; small
+    blocks are batched along the grid."""
+    if not _is_dev(data):
+        raise TypeError("dedisperse_overlap_save takes a DeviceArray stream (host streams: "
+                        "streaming.dedisperse_blocks)")
+    if raw is None and np.dtype(data.dtype) != np.complex64:
+        raise TypeError(f"expected a complex64 or raw stream, got {np.dtype(data.dtype)}")
+    block_len = int(block_len)
+    if block_len < 1:
+        raise ValueError("block_len must be >= 1")
+    g = _DedispGeometry(data, raw, raw_shape, crop, nsamp=block_len)
+    advance = g.stop - g.start
+    if advance <= 0:
+        raise ValueError(f"the crop {tuple(crop)} of a block keeps no rows")
+    nstream = int(data.shape[0])
+    nblocks = (nstream - block_len) // advance + 1 if nstream >= block_len else 0
+    dev = data.device
+    ctx = g.plan(dm=dm, sample_rate_hz=sample_rate_hz, chan_freq_hz=chan_freq_hz,
+                 ref_freq_hz=ref_freq_hz, out_kind=out_kind, downsample=downsample,
+                 explicit_chirp=False, dev=dev)
+    with ctx as plan:
+        out_trailing = (g.nchan,) if out_kind == L.OUT_STOKES_I else (g.nchan,) + g.trailing
+        out = DeviceArray.empty((nblocks * plan.out_rows,) + out_trailing,
+                                np.complex64 if out_kind == L.OUT_C64 else np.float32, dev)
+        if nblocks and plan.out_rows:
+            x = data.contiguous()
+            with ctx.lock:
+                plan.exec_blocks_device(x.ptr, nblocks, out.ptr, _stream())
+                # recount: the first batched execution allocates the block scratch slabs
+                _recount(ctx.ent)
+    return out
+
+
 class _DedispGeometry:
     """Shape, input kind and crop of a dedispersion call (``raw`` / ``raw_shape`` / ``crop`` as in
-    :func:`dedisperse`), and the cached plan for it."""
+    :func:`dedisperse`), and the cached plan for it.  ``nsamp`` overrides the block length (the
+    rows of ``data`` by default)."""
 
-    def __init__(self, data, raw, raw_shape, crop):
+    def __init__(self, data, raw, raw_shape, crop, nsamp=None):
         if raw is not None and raw not in _RAW_KINDS:
             raise ValueError(f"raw must be one of {sorted(_RAW_KINDS)}, got {raw!r}")
         shape = tuple(data.shape)
@@ -342,7 +385,7 @@ class _DedispGeometry:
         else:
             body = shape[:-1] if raw == "int8" else shape
         self.raw = raw
-        self.nsamp, self.nchan = body[0], body[1]
+        self.nsamp, self.nchan = (body[0] if nsamp is None else nsamp), body[1]
         self.trailing = body[2:]
         self.npol = int(np.prod(self.trailing)) if self.trailing else 1
         self.in_dtype, self.raw_np = _RAW_KINDS[raw] if raw is not None else (L.PBK_C64, None)

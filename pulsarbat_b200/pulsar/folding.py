@@ -11,6 +11,7 @@ from .. import kernels
 from .. import units as u
 from ..core import BasebandSignal, Signal
 from ..device import DeviceArray
+from ..transforms.dedispersion import _block_schedule
 
 __all__ = ["fold", "fold_segments", "dedisperse_fold"]
 
@@ -73,22 +74,6 @@ def fold(z, predictor, nbin, *, profile=None, counts=None, want_bins=False):
     if want_bins:
         return profile, counts, np.concatenate(bins) if bins else np.empty(0, np.int32)
     return profile, counts
-
-
-def _block_schedule(nsamp, block_len, start, stop, downsample):
-    """Overlap-save blocks of a folded stream: ``(advance, block starts)``.  Blocks of
-    ``block_len`` samples keep the rows ``[start, start + advance)``, where the advance is the
-    valid length ``stop - start`` rounded down to a multiple of ``downsample`` (every summed output
-    row lies inside one block); a tail that does not fill a block is dropped, as
-    ``overlap_save_dedispersion`` drops it."""
-    valid = stop - start
-    if valid <= 0:
-        raise ValueError("block length does not exceed the dispersion sweep")
-    advance = valid // downsample * downsample
-    if advance == 0:
-        raise ValueError(f"the valid length of a block ({valid} samples) is shorter than "
-                         f"downsample={downsample}")
-    return advance, list(range(0, nsamp - block_len + 1, advance))
 
 
 def _block_pieces(nblocks, rows, stretches):

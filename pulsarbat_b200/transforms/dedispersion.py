@@ -291,33 +291,90 @@ def dedisperse_trials(z, DMs, /, *, ref_freq=None, detect=True, stokes_I=False, 
     return [_cropped_like(IntensitySignal, z, x[k], max(start, 0), **kw) for k in range(len(DMs))]
 
 
-def overlap_save_dedispersion(z, DM, block_len, /, *, ref_freq=None):
-    """Dedisperse a long stream in overlapping blocks of ``block_len`` samples (builder-defined,
-    SURVEY.md 8a row O): the result equals the concatenation of ``coherent_dedispersion`` applied
-    to blocks that advance by the valid length, i.e. what the reference gives per block."""
-    if not isinstance(z, BasebandSignal):
-        raise TypeError("Signal must be a BasebandSignal object.")
-    DM = _as_dm(DM)
-    if ref_freq is None:
-        ref_freq = z.center_freq
-    probe = z[:block_len]
-    start, stop = crop_range(probe, DM, ref_freq)
+def _block_schedule(nsamp, block_len, start, stop, downsample):
+    """Overlap-save blocks of a stream: ``(advance, block starts)``.  Blocks of ``block_len``
+    samples keep the rows ``[start, start + advance)``, where the advance is the valid length
+    ``stop - start`` rounded down to a multiple of ``downsample`` (every summed output row lies
+    inside one block); a tail that does not fill a block is dropped."""
     valid = stop - start
     if valid <= 0:
         raise ValueError("block length does not exceed the dispersion sweep")
-    starts = list(range(0, len(z) - block_len + 1, valid))
+    advance = valid // downsample * downsample
+    if advance == 0:
+        raise ValueError(f"the valid length of a block ({valid} samples) is shorter than "
+                         f"downsample={downsample}")
+    return advance, list(range(0, nsamp - block_len + 1, advance))
+
+
+def overlap_save_dedispersion(z, DM, block_len, /, *, ref_freq=None, detect=False, stokes_I=False,
+                              downsample=1):
+    """Dedisperse a long stream in overlapping blocks of ``block_len`` samples (builder-defined,
+    SURVEY.md 8a row O).  The blocks advance by the valid length of a block rounded down to a
+    multiple of ``downsample`` and keep that many rows after the leading crop; the tail that does
+    not fill a block is dropped.
+
+    With ``detect=False`` the result equals the concatenation of ``coherent_dedispersion`` applied
+    to those blocks, i.e. what the reference gives per block.  With ``detect=True`` it is an
+    ``IntensitySignal``: the concatenation of ``dedisperse_detect(block, DM, stokes_I=...,
+    downsample=...)`` over the blocks, which is what ``dedisperse_fold(..., block_len=...)`` folds.
+    ``z`` may be a ``(raw_int8, template_signal)`` tuple as in :func:`dedisperse_detect`.
+
+    A stream on the device (a ``DeviceArray``, complex64 or raw) is dedispersed by one library
+    call for all blocks (:func:`kernels.dedisperse_overlap_save`) and the result stays on the
+    device.  Host complex64 and int8 streams go through the three-stream pipeline (upload, kernels
+    and download of consecutive blocks overlap); complex128 runs the FP64 kernels per block.
+    """
+    raw = None
+    if isinstance(z, tuple):
+        raw, z = z
+    if not isinstance(z, BasebandSignal):
+        raise TypeError("Signal must be a BasebandSignal object.")
+    ds = int(downsample)
+    if ds < 1:
+        raise ValueError("downsample must be >= 1")
+    if not detect and (ds > 1 or stokes_I):
+        raise ValueError("downsample and stokes_I need detect=True")
+    DM = _as_dm(DM)
+    if ref_freq is None:
+        ref_freq = z.center_freq
+    block_len = int(block_len)
+    src = z.data if raw is None else raw
+    start, stop = crop_range(z, DM, ref_freq, nsamp=block_len)
+    advance, starts = _block_schedule(src.shape[0], block_len, start, stop, ds)
+    kind = (L.OUT_C64 if not detect else L.OUT_STOKES_I if stokes_I else L.OUT_INTENSITY)
     kw = dict(dm=DM.dm, sample_rate_hz=z.sample_rate_hz, chan_freq_hz=z.channel_freqs_hz,
-              ref_freq_hz=_hz(ref_freq), crop=(start, stop))
-    if isinstance(z.data, kernels.DeviceArray) or np.asarray(z.data).dtype != np.complex64:
-        pieces = [np.asarray(kernels.dedisperse(z[b:b + block_len].data, **kw)) for b in starts]
-        data = np.concatenate(pieces, axis=0)
+              ref_freq_hz=_hz(ref_freq), crop=(start, start + advance), out_kind=kind,
+              downsample=ds, raw=None if raw is None else "int8")
+    on_dev = isinstance(src, kernels.DeviceArray)
+    if on_dev and (raw is not None or src.dtype == np.complex64):
+        data = kernels.dedisperse_overlap_save(src, block_len=block_len, **kw)
+    elif raw is None and (on_dev or np.asarray(src).dtype != np.complex64):
+        # complex128: the FP64 kernels block by block, on the stream's side of the bus
+        pieces = [kernels.dedisperse(src[b:b + block_len], **kw) for b in starts]
+        if not pieces:
+            shape = (0,) + (tuple(z.shape[1:]) if kind != L.OUT_STOKES_I else (z.nchan,))
+            dt = np.complex128 if kind == L.OUT_C64 else np.float64
+            data = kernels.DeviceArray.empty(shape, dt, src.device) if on_dev else np.empty(shape, dt)
+        elif on_dev:
+            import torch
+            data = kernels.DeviceArray(torch.cat([p.tensor for p in pieces]))
+        else:
+            data = np.concatenate(pieces, axis=0)
     else:
-        # host complex64 stream: the blocks go through the three-stream pipeline (upload of block
-        # i+1, kernels of block i and download of block i-1 overlap) straight into the result
+        # host complex64 or int8 stream: the blocks go through the three-stream pipeline (upload of
+        # block i+1, kernels of block i and download of block i-1 overlap) straight into the result
         from .. import streaming
-        src = np.asarray(z.data)
-        data = np.empty((len(starts) * valid,) + src.shape[1:], np.complex64)
+        src = np.asarray(src)
+        rows = advance // ds
+        trailing = (z.nchan,) if kind == L.OUT_STOKES_I else tuple(z.shape[1:])
+        data = np.empty((len(starts) * rows,) + trailing,
+                        np.complex64 if kind == L.OUT_C64 else np.float32)
         blocks = (src[b:b + block_len] for b in starts)
         for i, y in enumerate(streaming.dedisperse_blocks(blocks, pinned_out=True, **kw)):
-            data[i * valid:(i + 1) * valid] = y
-    return _cropped_like(type(z), z, data, start)
+            data[i * rows:(i + 1) * rows] = y
+    if not detect:
+        return _cropped_like(type(z), z, data, start)
+    kw = {"chan_bw": z.chan_bw}
+    if ds > 1:
+        kw["sample_rate"] = z.sample_rate / ds
+    return _cropped_like(IntensitySignal, z, data, start, **kw)
