@@ -338,6 +338,32 @@ int pbk_shift_channels(const void* in, void* out, int64_t nsamp_in, int64_t nsam
 int pbk_downsample(const void* in, void* out, int64_t nsamp, int64_t row_elems,
                    int64_t factor, int32_t on_device, int32_t device, void* stream);
 
+/* Incoherent dedispersion at ndm trial DMs summed over frequency: a DM x time plane (builder-defined;
+ * trial k is pbk_shift_channels with that trial's delays, summed over channels):
+ *   out[k, j, p] = sum_{c < nchan} in[j + delays[k * nchan + c], c, p],  j < rows,
+ * in (nsamp_in, nchan, npol) float32, out a contiguous (ndm, rows, npol) float32 array.  Channels
+ * are added in ascending order in float32 with no atomics: executions are bit for bit
+ * reproducible, and integer-valued data within float32's exact range sum exactly.  The delays
+ * (host array [ndm * nchan]) are any non-negative values with delay + rows <= nsamp_in; trials may
+ * come in any order and repeat.  pb.incoherent_dedispersion_trials builds them from the reference's
+ * rounded delays (dedispersion.py:164-169) and the intersection of every trial's valid rows.
+ * The plan sorts the trials by sweep, groups them in blocks of KD <= 8 and uploads its tables once
+ * (counted in pbk_plan_info's workspace bytes); one execution is one kernel launch.
+ * ndm < 1, nchan < 1, npol < 1, rows < 0, a NULL pointer, a negative delay or delay + rows >
+ * nsamp_in return PBK_ERR_INVALID; rows, nsamp_in or nchan above INT32_MAX and npol > 256 return
+ * PBK_ERR_UNSUPPORTED.  rows == 0 executes as a no-op.  pbk_plan_describe shows
+ * "INCOH:ndm=..:C=..:P=..:rows=.." and the tile (KD, TT rows, CC channels per staged chunk, shared
+ * bytes, CTAs); pbk_plan_trials reports ndm, pbk_plan_blocks_per_launch 1, pbk_plan_segments 0:
+ * pbk_plan_profile does not time these plans (time them with events around the call).
+ * Execution: device pointers need 4-byte alignment (PBK_ERR_INVALID otherwise); _exec_device only
+ * enqueues one kernel on `stream` and can be captured into a graph; _exec_host copies in, runs,
+ * copies out and synchronises.  The input is never written. */
+int pbk_incoh_trials_plan_create(int64_t nsamp_in, int64_t nchan, int64_t npol, int64_t rows,
+                                 const int64_t* delays, int32_t ndm, int32_t device,
+                                 pbk_plan** plan);
+int pbk_incoh_trials_exec_device(pbk_plan* plan, const void* d_in, void* d_out, void* stream);
+int pbk_incoh_trials_exec_host(pbk_plan* plan, const void* in, void* out);
+
 /* ---- polarisation -------------------------------------------------------------------------
  * pbk_stokes:    (A, B) complex64 pol pairs -> [I, Q, U, V] float32 (core.py:930-966; basis
  *                linear when circular == 0).  npairs = nsamp * nchan.

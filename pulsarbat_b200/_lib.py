@@ -19,6 +19,7 @@ EXPORTS = [
     "pbk_dedisp_plan_create", "pbk_dedisp_out_shape", "pbk_dedisp_exec_host",
     "pbk_dedisp_exec_device", "pbk_dedisp_fold_exec_device", "pbk_dedisp_trials_plan_create",
     "pbk_plan_trials", "pbk_dedisp_exec_blocks_device", "pbk_plan_blocks_per_launch",
+    "pbk_incoh_trials_plan_create", "pbk_incoh_trials_exec_device", "pbk_incoh_trials_exec_host",
     "pbk_fft_plan_create", "pbk_stft_plan_create", "pbk_stft_plan_create_raw",
     "pbk_stft_detect_plan_create", "pbk_stft_fold_exec_device",
     "pbk_dedisp_c128", "pbk_fft_c128", "pbk_stft_c128", "pbk_detect_c128",
@@ -88,6 +89,10 @@ def lib():
         L.pbk_plan_trials.argtypes = [vp, ctypes.POINTER(i32)]
         L.pbk_dedisp_exec_blocks_device.argtypes = [vp, vp, i64, vp, vp]
         L.pbk_plan_blocks_per_launch.argtypes = [vp, ctypes.POINTER(i32)]
+        L.pbk_incoh_trials_plan_create.argtypes = [i64, i64, i64, i64, ctypes.POINTER(i64), i32,
+                                                   i32, ctypes.POINTER(vp)]
+        L.pbk_incoh_trials_exec_device.argtypes = [vp, vp, vp, vp]
+        L.pbk_incoh_trials_exec_host.argtypes = [vp, vp, vp]
         L.pbk_dedisp_out_shape.argtypes = [vp] + [ctypes.POINTER(i64)] * 3
         L.pbk_dedisp_exec_host.argtypes = [vp, vp, vp, vp]
         L.pbk_dedisp_exec_device.argtypes = [vp, vp, vp, vp, vp]
@@ -314,6 +319,48 @@ class DedispTrialsPlan(DedispPlan):
         """pbk_plan_trials: the number of trial DMs."""
         n = ctypes.c_int32(0)
         check(lib().pbk_plan_trials(self.handle, ctypes.byref(n)))
+        return n.value
+
+
+class IncohTrialsPlan(Plan):
+    """Incoherent dedispersion at ndm trial DMs summed over frequency
+    (pbk_incoh_trials_plan_create): ``out[k, j, p] = sum_c in[j + delays[k, c], c, p]`` for
+    (nsamp, nchan, npol) float32 input and a contiguous (ndm, rows, npol) float32 output."""
+
+    def __init__(self, *, nsamp, nchan, npol, rows, delays, device=0):
+        d = np.ascontiguousarray(delays, dtype=np.int64)
+        if d.ndim != 2 or d.shape[1] != nchan:
+            raise ValueError(f"delays must have shape (ndm, {nchan})")
+        h = ctypes.c_void_p(0)
+        check(lib().pbk_incoh_trials_plan_create(
+            int(nsamp), int(nchan), int(npol), int(rows),
+            d.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)), d.shape[0], int(device),
+            ctypes.byref(h)))
+        super().__init__(h)
+        self.nsamp, self.nchan, self.npol, self.rows = int(nsamp), int(nchan), int(npol), int(rows)
+        self.ndm = d.shape[0]
+        self.device = device
+
+    def out_array(self):
+        return np.empty((self.ndm, self.rows, self.npol), dtype=np.float32)
+
+    def exec_host(self, x, out):
+        check(lib().pbk_incoh_trials_exec_host(self.handle, ptr(x), ptr(out)))
+        return out
+
+    def exec_device(self, d_in, d_out, stream=0):
+        check(lib().pbk_incoh_trials_exec_device(self.handle, ptr(d_in), ptr(d_out),
+                                                 ctypes.c_void_p(stream)))
+
+    def trials(self):
+        """pbk_plan_trials: the number of trial DMs."""
+        n = ctypes.c_int32(0)
+        check(lib().pbk_plan_trials(self.handle, ctypes.byref(n)))
+        return n.value
+
+    def blocks_per_launch(self):
+        n = ctypes.c_int32(0)
+        check(lib().pbk_plan_blocks_per_launch(self.handle, ctypes.byref(n)))
         return n.value
 
 

@@ -30,6 +30,7 @@
 #include "pbk_fft.cuh"
 #include "pbk_hostcopy.h"
 #include "pbk_misc.cuh"
+#include "pbk_incoh.cuh"
 
 using namespace pbk;
 
@@ -92,7 +93,7 @@ extern "C" int pbk_device_mem_info(int device, size_t* free_bytes, size_t* total
 // plan
 // ------------------------------------------------------------------------------------------
 enum Role { ROLE_USER_IN = 0, ROLE_SCRATCH = 1, ROLE_USER_OUT = 2, ROLE_TMPF = 3 };
-enum PlanKind { PLAN_DEDISP = 0, PLAN_FFT = 1 };
+enum PlanKind { PLAN_DEDISP = 0, PLAN_FFT = 1, PLAN_INCOH = 2 };
 
 struct Pass {
   int mode = MODE_FWD;
@@ -191,6 +192,13 @@ struct pbk_plan {
   long long prof_next = 0;
   int prof_cur = -1;
   bool prof_off = false;        // block executions are not timed
+  // incoherent trial plans (pbk_incoh_trials_plan_create): one launch of incoh_trials_kernel<KD>
+  pbk_incoh::Args incoh{};      // device pointers into d_incoh; in / out set per execution
+  int incoh_kd = 0;
+  unsigned incoh_grid = 0;
+  size_t incoh_smem = 0;
+  int* d_incoh = nullptr;       // perm, off, lo and ext tables
+  size_t incoh_bytes = 0;
 };
 
 static void prof_mark(pbk_plan* pl, int idx, cudaStream_t st) {
@@ -2413,6 +2421,7 @@ extern "C" void pbk_plan_destroy(pbk_plan* pl) {
   cudaFree(pl->d_foldbuf);
   cudaFree(pl->d_stage);
   cudaFree(pl->d_l2sync);
+  cudaFree(pl->d_incoh);
   cudaFree(pl->h_din);
   cudaFree(pl->h_dout);
   cudaFree(pl->h_dchirp);
@@ -2428,7 +2437,7 @@ extern "C" int pbk_plan_info(const pbk_plan* pl, int32_t* launches, int64_t* wor
                 (pl->work_bytes > pl->scratch_bytes ? pl->work_bytes - pl->scratch_bytes : 0) +
                 pl->blk_bytes * ((pl->blk_scratch[0] ? 1 : 0) + (pl->blk_scratch[1] ? 1 : 0)) +
                 pl->tmpf_bytes + pl->fold_bytes +
-                pl->stage_bytes);
+                pl->stage_bytes + pl->incoh_bytes);
   if (levels) *levels = pl->nlevels;
   if (level_log2)
     for (int i = 0; i < 3; ++i) level_log2[i] = pl->level_log2[i];
@@ -2439,6 +2448,12 @@ extern "C" int pbk_plan_describe(const pbk_plan* pl, char* buf, size_t n) {
   if (!pl || !buf || n == 0) return fail(PBK_ERR_INVALID, "NULL argument");
   size_t off = 0;
   buf[0] = 0;
+  if (pl->kind == PLAN_INCOH) {
+    const pbk_incoh::Args& a = pl->incoh;
+    snprintf(buf, n, "INCOH:ndm=%d:C=%d:P=%d:rows=%d:KD=%d:TT=%d:CC=%d:smem=%zu:tiles=%u", pl->ndm,
+             a.C, a.P, a.rows, pl->incoh_kd, a.TT, a.CC, pl->incoh_smem, pl->incoh_grid);
+    return PBK_OK;
+  }
   if (pl->blue) {
     snprintf(buf, n, "BLUESTEIN:n=%lld:M=2^%d:lanes=%lld", pl->blue->n, ilog2_exact(pl->blue->M),
              pl->blue->I);
@@ -2489,6 +2504,164 @@ extern "C" int pbk_plan_describe(const pbk_plan* pl, char* buf, size_t n) {
 extern "C" int pbk_plan_segments(const pbk_plan* pl, int32_t* segments) {
   if (!pl || !segments) return fail(PBK_ERR_INVALID, "NULL argument");
   *segments = pl->segments;
+  return PBK_OK;
+}
+
+// ------------------------------------------------------------------------------------------
+// incoherent dedispersion at many trial DMs, summed over frequency (pbk_incoh.cuh)
+// ------------------------------------------------------------------------------------------
+// Shared memory of one CTA is at most this much, so that two CTAs fit an SM whatever the span.
+static constexpr size_t kIncohSmemCap = 100 * 1024;
+
+// Block tables of one (KD, CC) choice over the trials in sorted order; returns the shared memory
+// one CTA needs.
+static size_t incoh_tables(const std::vector<int>& order, const int64_t* delays, int ndm, int C,
+                           int P, int KD, int CC, std::vector<int>& tab, int* stride_out) {
+  const int nb = (ndm + KD - 1) / KD, nq = (C + CC - 1) / CC;
+  tab.assign((size_t)nb * KD + (size_t)nb * KD * C + 2 * (size_t)nb * nq, 0);
+  int* perm = tab.data();
+  int* off = perm + (size_t)nb * KD;
+  int* lo = off + (size_t)nb * KD * C;
+  int* ext = lo + (size_t)nb * nq;
+  long long ext_max = 0;
+  for (int b = 0; b < nb; ++b)
+    for (int q = 0; q < nq; ++q) {
+      long long mn = LLONG_MAX, mx = LLONG_MIN;
+      for (int s = b * KD; s < std::min(ndm, (b + 1) * KD); ++s)
+        for (int c = q * CC; c < std::min(C, (q + 1) * CC); ++c) {
+          const long long d = delays[(size_t)order[s] * C + c];
+          mn = std::min(mn, d);
+          mx = std::max(mx, d);
+        }
+      lo[b * nq + q] = (int)mn;
+      ext[b * nq + q] = (int)(mx - mn);
+      ext_max = std::max(ext_max, mx - mn);
+    }
+  for (int s = 0; s < nb * KD; ++s) {
+    perm[s] = s < ndm ? order[s] : -1;
+    for (int c = 0; c < C; ++c)
+      off[(size_t)s * C + c] =
+          s < ndm ? (int)(delays[(size_t)order[s] * C + c] - lo[(s / KD) * nq + c / CC]) : 0;
+  }
+  // a staged channel holds ext + TT rows of P floats; any accumulator index < kFlat stays inside.
+  // The stride is padded so that the staging stores of a warp hit distinct banks: with 16 floats
+  // per staged row (CC * P == 16) a warp stores two rows, which stride = 2P (mod 32) separates.
+  long long stride = ext_max * P + pbk_incoh::kFlat;
+  if (stride > INT_MAX / 2) return SIZE_MAX;
+  const int want = CC * P == 16 ? (2 * P) % 32 : 1;
+  while ((int)(stride % 32) != want) ++stride;
+  *stride_out = (int)stride;
+  return (size_t)stride * CC * sizeof(float);
+}
+
+extern "C" int pbk_incoh_trials_plan_create(int64_t nsamp_in, int64_t nchan, int64_t npol,
+                                            int64_t rows, const int64_t* delays, int32_t ndm,
+                                            int32_t device, pbk_plan** out) {
+  if (!delays || !out) return fail(PBK_ERR_INVALID, "NULL pointer");
+  *out = nullptr;
+  if (ndm < 1 || nchan < 1 || npol < 1 || nsamp_in < 0 || rows < 0)
+    return fail(PBK_ERR_INVALID, "bad shape (ndm, nchan and npol must be >= 1, rows >= 0)");
+  for (int64_t i = 0; i < (int64_t)ndm * nchan; ++i)
+    if (delays[i] < 0 || delays[i] > nsamp_in - rows)
+      return fail(PBK_ERR_INVALID, "delay[%lld][%lld] = %lld reads outside the input of %lld rows",
+                  (long long)(i / nchan), (long long)(i % nchan), (long long)delays[i],
+                  (long long)nsamp_in);
+  if (rows > INT_MAX || nsamp_in > INT_MAX || nchan > INT_MAX)
+    return fail(PBK_ERR_UNSUPPORTED, "rows, delays and channels must fit 32-bit indices");
+  if (npol > pbk_incoh::kMaxP)
+    return fail(PBK_ERR_UNSUPPORTED, "npol = %lld: at most %d floats per cell", (long long)npol,
+                pbk_incoh::kMaxP);
+  const int C = (int)nchan, P = (int)npol;
+  // sorted by sweep (the delay of the first channel less that of the last, monotone in DM for a
+  // fixed reference frequency), so that a block of KD trials spans few rows
+  std::vector<int> order(ndm);
+  for (int k = 0; k < ndm; ++k) order[k] = k;
+  std::stable_sort(order.begin(), order.end(), [&](int x, int y) {
+    const int64_t* dx = delays + (size_t)x * C;
+    const int64_t* dy = delays + (size_t)y * C;
+    const int64_t sx = dx[0] - dx[C - 1], sy = dy[0] - dy[C - 1];
+    return sx != sy ? sx < sy : dx[0] < dy[0];
+  });
+  // the largest tile that fits: KD shrinks first, then CC; KD = CC = 1 stages TT rows of one
+  // channel (ext = 0) and always fits
+  std::vector<int> tab;
+  int KD = 0, CC = 0, stride = 0;
+  size_t smem = 0;
+  for (int cc = std::min(C, std::max(1, 16 / P)); cc >= 1 && !KD; cc = cc > 1 ? cc / 2 : 0)
+    for (int kd = 8; kd >= 1 && !KD; kd /= 2) {
+      if (kd > 1 && ndm <= kd / 2) continue;    // half the warps would idle
+      smem = incoh_tables(order, delays, ndm, C, P, kd, cc, tab, &stride);
+      if (smem <= kIncohSmemCap) KD = kd, CC = cc;
+    }
+  if (!KD) return fail(PBK_ERR_UNSUPPORTED, "no tile fits shared memory");
+  const int TT = pbk_incoh::kFlat / P;
+  const long long nb = (ndm + KD - 1) / KD, ntiles = (rows + TT - 1) / TT;
+  if (nb * ntiles > INT_MAX) return fail(PBK_ERR_UNSUPPORTED, "too many tiles for one launch");
+  CUDA_TRY(cudaSetDevice(device));
+  pbk_plan* pl = new pbk_plan();
+  pl->kind = PLAN_INCOH;
+  pl->device = device;
+  pl->ndm = ndm;
+  auto cleanup = [&](int code) { pbk_plan_destroy(pl); return code; };
+  pl->incoh_bytes = tab.size() * sizeof(int);
+  cudaError_t e = cudaMalloc(&pl->d_incoh, pl->incoh_bytes);
+  if (e == cudaSuccess)
+    e = cudaMemcpy(pl->d_incoh, tab.data(), pl->incoh_bytes, cudaMemcpyHostToDevice);
+  if (e == cudaSuccess)
+    e = cudaFuncSetAttribute(pbk_incoh::kernel_of(KD), cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             (int)kIncohSmemCap);   // the cap, never less: other plans share it
+  if (e != cudaSuccess)
+    return cleanup(fail(e == cudaErrorMemoryAllocation ? PBK_ERR_NOMEM : PBK_ERR_CUDA,
+                        "incoherent trial plan: %s", cudaGetErrorString(e)));
+  pbk_incoh::Args& a = pl->incoh;
+  a.row_elems = (long long)C * P;
+  a.C = C, a.P = P, a.rows = (int)rows, a.TT = TT, a.CC = CC, a.nq = (C + CC - 1) / CC;
+  a.stride = stride;
+  a.nb = (int)nb;
+  a.perm = pl->d_incoh;
+  a.off = a.perm + nb * KD;
+  a.lo = a.off + nb * KD * C;
+  a.ext = a.lo + nb * a.nq;
+  pl->incoh_kd = KD;
+  pl->incoh_grid = (unsigned)(nb * ntiles);
+  pl->incoh_smem = smem;
+  pl->launches = rows > 0 ? 1 : 0;
+  pl->in_bytes = (size_t)nsamp_in * C * P * sizeof(float);
+  pl->out_bytes = (size_t)ndm * rows * P * sizeof(float);
+  *out = pl;
+  return PBK_OK;
+}
+
+extern "C" int pbk_incoh_trials_exec_device(pbk_plan* pl, const void* d_in, void* d_out,
+                                            void* stream) {
+  if (!pl || pl->kind != PLAN_INCOH) return fail(PBK_ERR_INVALID, "not an incoherent-trials plan");
+  if (!d_in || !d_out) return fail(PBK_ERR_INVALID, "NULL data pointer");
+  if (((uintptr_t)d_in | (uintptr_t)d_out) & 3)
+    return fail(PBK_ERR_INVALID, "float32 arrays must be 4-byte aligned");
+  if (pl->incoh.rows == 0) return PBK_OK;
+  CUDA_TRY(cudaSetDevice(pl->device));
+  pbk_incoh::Args a = pl->incoh;
+  a.in = reinterpret_cast<const float*>(d_in);
+  a.out = reinterpret_cast<float*>(d_out);
+  cudaError_t e = pbk_incoh::launch(pl->incoh_kd, a, pl->incoh_grid, pl->incoh_smem,
+                                    reinterpret_cast<cudaStream_t>(stream));
+  if (e != cudaSuccess) return fail(PBK_ERR_CUDA, "incoherent trials launch: %s", cudaGetErrorString(e));
+  return PBK_OK;
+}
+
+extern "C" int pbk_incoh_trials_exec_host(pbk_plan* pl, const void* in, void* out) {
+  if (!pl || pl->kind != PLAN_INCOH) return fail(PBK_ERR_INVALID, "not an incoherent-trials plan");
+  if (!in || !out) return fail(PBK_ERR_INVALID, "NULL data pointer");
+  if (pl->incoh.rows == 0) return PBK_OK;
+  std::lock_guard<std::mutex> lock(pl->mu);
+  CUDA_TRY(cudaSetDevice(pl->device));
+  int rc;
+  if ((rc = ensure_buf(&pl->h_din, pl->in_bytes)) != PBK_OK) return rc;
+  if ((rc = ensure_buf(&pl->h_dout, pl->out_bytes)) != PBK_OK) return rc;
+  cudaStream_t st = cudaStreamPerThread;
+  CUDA_TRY(host_to_device(pl->h_din, in, pl->in_bytes, st));
+  if ((rc = pbk_incoh_trials_exec_device(pl, pl->h_din, pl->h_dout, st)) != PBK_OK) return rc;
+  CUDA_TRY(device_to_host(out, pl->h_dout, pl->out_bytes, st));
   return PBK_OK;
 }
 

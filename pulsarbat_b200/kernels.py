@@ -24,7 +24,7 @@ from .device import DeviceArray
 
 __all__ = ["default_device", "dedisperse", "chirp", "detect", "shift_channels", "phase_ramp", "mix", "analytic_decimate", "stokes", "pol_basis",
            "downsample", "fft", "stft", "istft", "stft_detect", "stft_fold", "fold",
-           "dedisperse_fold", "dedisperse_trials", "predict_phase", "clear_plan_cache",
+           "dedisperse_fold", "dedisperse_trials", "incoherent_trials", "predict_phase", "clear_plan_cache",
            "pinned_results"]
 
 
@@ -659,6 +659,46 @@ def shift_channels(data, delays, nsamp_out, device=None):
     L.check(L.lib().pbk_shift_channels(L.ptr(x), L.ptr(out), nsamp, int(nsamp_out), nchan, cell,
                                        dp, 0, dev, None))
     return out
+
+
+def incoherent_trials(data, delays, rows, device=None):
+    """Incoherent dedispersion at many trial DMs summed over frequency (a DM x time plane):
+    ``out[k, j, ...] = sum_c data[j + delays[k, c], c, ...]`` for ``j < rows``, channels added in
+    ascending order in float32 (pbk_incoh_trials_plan_create).
+
+    ``data`` is (nsamp, nchan, ...) float32, numpy or DeviceArray; ``delays`` is (ndm, nchan)
+    int64 with ``0 <= delays`` and ``delays + rows <= nsamp``.  Returns (ndm, rows, ...) float32
+    on the same side of the bus.  Plans are cached by the whole delay table."""
+    shape = tuple(data.shape)
+    if len(shape) < 2:
+        raise ValueError("incoherent_trials takes (nsamp, nchan, ...) data")
+    if np.dtype(data.dtype) != np.float32:
+        raise TypeError(f"incoherent_trials takes float32 data, got {np.dtype(data.dtype)}")
+    nsamp, nchan = shape[0], shape[1]
+    npol = int(np.prod(shape[2:], dtype=np.int64)) if len(shape) > 2 else 1
+    d = np.ascontiguousarray(delays, dtype=np.int64)
+    if d.ndim != 2 or d.shape[1] != nchan or d.shape[0] < 1:
+        raise ValueError(f"delays must have shape (ndm, {nchan}) with ndm >= 1")
+    rows = int(rows)
+    out_shape = (d.shape[0], rows) + shape[2:]
+    dev = data.device if _is_dev(data) else (default_device() if device is None else device)
+    # the key holds the delay table's bytes: a cache hit compares them exactly
+    key = ("incoh_trials", nsamp, nchan, npol, rows, d.shape, d.tobytes(), dev)
+    ctx = _use_plan(key, lambda: L.IncohTrialsPlan(nsamp=nsamp, nchan=nchan, npol=npol, rows=rows,
+                                                   delays=d, device=dev))
+    with ctx as plan:
+        if _is_dev(data):
+            x = data.contiguous()
+            out = DeviceArray.empty(out_shape, np.float32, x.device)
+            if rows:                       # an empty tensor may have a NULL pointer
+                with ctx.lock:
+                    plan.exec_device(x.ptr, out.ptr, _stream())
+            return out
+        x = np.ascontiguousarray(data)
+        out = _result(out_shape, np.float32)
+        with ctx.lock:
+            plan.exec_host(x, out)
+        return out
 
 
 def phase_ramp(data, shift_samples=None, zero_lo=None, zero_hi=None, device=None):

@@ -16,7 +16,8 @@ from .. import units as u
 from ..core import BasebandSignal, IntensitySignal, RadioSignal
 
 __all__ = ["DispersionMeasure", "DM", "coherent_dedispersion", "incoherent_dedispersion",
-           "dedisperse_detect", "dedisperse_trials", "overlap_save_dedispersion"]
+           "dedisperse_detect", "dedisperse_trials", "incoherent_dedispersion_trials",
+           "overlap_save_dedispersion"]
 
 #: s MHz^2 cm^3 / pc -- dedispersion.py:30
 DISPERSION_CONSTANT = 1.0 / 2.41e-4
@@ -289,6 +290,70 @@ def dedisperse_trials(z, DMs, /, *, ref_freq=None, detect=True, stokes_I=False, 
     if downsample > 1:
         kw["sample_rate"] = z.sample_rate / downsample
     return [_cropped_like(IntensitySignal, z, x[k], max(start, 0), **kw) for k in range(len(DMs))]
+
+
+def incoherent_trial_delays(z, DMs, ref_freq):
+    """``(e, t_lo, rows)`` of :func:`incoherent_dedispersion_trials`: trial k reads input row
+    ``t_lo + j + r_k[c]`` of channel c for its output row j, where ``r_k`` are the reference's
+    rounded delays (:func:`incoherent_delays` without its ``crop_before`` shift) and
+    ``[t_lo, t_lo + rows)`` is the intersection of every trial's valid rows in absolute input rows.
+    ``e`` is the (ndm, nchan) int64 table ``r_k[c] + t_lo``; ``rows`` is 0 when the intersection
+    is empty.  A DM whose sweep exceeds the signal raises ``ValueError``."""
+    tables, lo, hi = [], [], []
+    for dm in as_dm_list(DMs):
+        delays, n_out, crop_before = incoherent_delays(z, dm, ref_freq)
+        if n_out < 0 or int(delays.min()) < 0:
+            raise ValueError("dispersion sweep exceeds the signal length")
+        tables.append(delays - crop_before)
+        lo.append(crop_before)
+        hi.append(crop_before + n_out)
+    t_lo = max(lo)
+    rows = max(0, min(hi) - t_lo)
+    return np.stack(tables) + t_lo, t_lo, rows
+
+
+def incoherent_dedispersion_trials(z, DMs, /, *, ref_freq=None):
+    """Incoherently dedisperse a filterbank at several trial DMs and sum over frequency: a DM x
+    time plane in one GPU call (builder-defined; kernels.incoherent_trials).
+
+    Returns a list with one ``IntensitySignal`` per DM, each of shape ``(rows, 1, ...)``, views
+    of one stacked array on ``z``'s side of the bus.  Element k equals
+    ``incoherent_dedispersion(z, DMs[k]).data`` summed over the frequency axis (in float32,
+    channels in ascending order) and cut to the rows that are valid for every trial
+    (:func:`incoherent_trial_delays`); an empty intersection gives zero-row results.  Each result
+    keeps the sample rate and the band (one channel of ``chan_bw * nchan`` at ``center_freq``,
+    ``freq_align="center"``) and starts ``t_lo`` samples after ``z``.  ``z`` must hold float32
+    data (a filterbank, ``stft_detect`` or ``dedisperse_detect`` output); other dtypes and dask
+    arrays raise ``TypeError``.
+    """
+    if not isinstance(z, RadioSignal):
+        raise TypeError("Signal must be a RadioSignal object.")
+    if _dask.is_dask(z.data):
+        raise TypeError("incoherent_dedispersion_trials takes numpy or DeviceArray data (a dask "
+                        "array: compute it first, or call incoherent_dedispersion per chunk)")
+    if np.dtype(z.dtype) != np.float32:
+        raise TypeError(f"incoherent_dedispersion_trials needs float32 data, got {z.dtype} "
+                        "(complex and float64 signals are not supported)")
+    DMs = as_dm_list(DMs)
+    if ref_freq is None:
+        ref_freq = z.center_freq
+    e, t_lo, rows = incoherent_trial_delays(z, DMs, ref_freq)
+    trailing = tuple(z.shape[2:])
+    if rows:
+        x = kernels.incoherent_trials(z.data, e, rows)
+    elif isinstance(z.data, kernels.DeviceArray):
+        x = kernels.DeviceArray.empty((len(DMs), 0) + trailing, np.float32, z.data.device)
+    else:
+        x = np.empty((len(DMs), 0) + trailing, np.float32)
+    shape = (len(DMs), rows, 1) + trailing
+    if isinstance(x, kernels.DeviceArray):
+        x = kernels.DeviceArray(x.tensor.reshape(shape))
+    else:
+        x = x.reshape(shape)
+    kw = {"chan_bw": z.chan_bw * z.nchan, "center_freq": z.center_freq, "freq_align": "center"}
+    if z.start_time is not None:
+        kw["start_time"] = z.start_time + t_lo / z.sample_rate
+    return [IntensitySignal.like(z, x[k], **kw) for k in range(len(DMs))]
 
 
 def _block_schedule(nsamp, block_len, start, stop, downsample):
