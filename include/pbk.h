@@ -364,6 +364,32 @@ int pbk_incoh_trials_plan_create(int64_t nsamp_in, int64_t nchan, int64_t npol, 
 int pbk_incoh_trials_exec_device(pbk_plan* plan, const void* d_in, void* d_out, void* stream);
 int pbk_incoh_trials_exec_host(pbk_plan* plan, const void* in, void* out);
 
+/* Single-pulse search of a stack of time series (builder-defined): x (nser, rows, ncols) float32,
+ * C-contiguous, series (s, c) = x[s, :, c] -- e.g. the (ndm, rows, 1[*P]) plane of
+ * pbk_incoh_trials_* or the (ndm, rows, nchan[*P]) output of a trial plan.
+ *   stats[s, c] = (mean, std) of the series in float64, population std (ddof 0), (nser, ncols, 2)
+ *       float64: computed (fixed-order partials per chunk of rows, merged in a fixed order) and
+ *       written when stats_given == 0, read when it is 1;
+ *   snr(s, c, t, w) = (sum_{i<w} x[s, t+i, c] - w mean) / (std sqrt(w)) for every t with
+ *       t + w <= rows, at the widths[0 .. nwidths) (host array, strictly increasing, >= 1, at most
+ *       4096 samples); every snr of a series whose std is not > 0 (zero, negative, NaN) is 0;
+ *   window j holds the starts [j window, min((j+1) window, rows)), nwin = ceil(rows / window):
+ *       snr[s, j, c] (float32), start[s, j, c] and width[s, j, c] (int32), each (nser, nwin, ncols),
+ *       are the maximum over the (t, w) of the window, ties to the smallest t, then the smallest w,
+ *       compared in float64; a window with no valid (t, w) gets -inf, -1, -1.
+ * window = 1 gives the best-S/N plane; window = max(widths) a compact per-window maximum.  No
+ * atomics: executions are bit for bit reproducible, and integer-valued data give exact boxcar sums.
+ * nser < 1, ncols < 1, rows < 0, nwidths outside 1..32, widths not strictly increasing or < 1,
+ * window < 1, a NULL pointer when rows > 0, and device arrays not aligned to their element size
+ * (4 bytes, 8 for stats) return PBK_ERR_INVALID; a width above 4096, rows, ncols or nser * ncols
+ * above INT32_MAX and grids beyond one launch return PBK_ERR_UNSUPPORTED.  rows == 0 is a no-op.
+ * on_device = 1 only enqueues on `stream` (the statistics partials are a stream-ordered
+ * allocation); 0 copies in, runs, copies out and synchronises.  The input is never written. */
+int pbk_boxcar_search(const void* in, int64_t nser, int64_t rows, int64_t ncols,
+                      const int32_t* widths, int32_t nwidths, int64_t window, void* stats,
+                      int32_t stats_given, void* snr, void* start, void* width, int32_t on_device,
+                      int32_t device, void* stream);
+
 /* ---- polarisation -------------------------------------------------------------------------
  * pbk_stokes:    (A, B) complex64 pol pairs -> [I, Q, U, V] float32 (core.py:930-966; basis
  *                linear when circular == 0).  npairs = nsamp * nchan.

@@ -20,6 +20,7 @@ EXPORTS = [
     "pbk_dedisp_exec_device", "pbk_dedisp_fold_exec_device", "pbk_dedisp_trials_plan_create",
     "pbk_plan_trials", "pbk_dedisp_exec_blocks_device", "pbk_plan_blocks_per_launch",
     "pbk_incoh_trials_plan_create", "pbk_incoh_trials_exec_device", "pbk_incoh_trials_exec_host",
+    "pbk_boxcar_search",
     "pbk_fft_plan_create", "pbk_stft_plan_create", "pbk_stft_plan_create_raw",
     "pbk_stft_detect_plan_create", "pbk_stft_fold_exec_device",
     "pbk_dedisp_c128", "pbk_fft_c128", "pbk_stft_c128", "pbk_detect_c128",
@@ -119,6 +120,8 @@ def lib():
         L.pbk_downsample.argtypes = [vp, vp, i64, i64, i64, i32, i32, vp]
         L.pbk_fold.argtypes = [vp, i64, i64, ctypes.POINTER(dbl), i32, dbl, i64, i32, vp, vp, vp,
                                i32, i32, vp]
+        L.pbk_boxcar_search.argtypes = [vp, i64, i64, i64, ctypes.POINTER(i32), i32, i64, vp, i32,
+                                        vp, vp, vp, i32, i32, vp]
         L.pbk_stokes.argtypes = [vp, vp, i64, i32, i32, i32, vp]
         L.pbk_pol_basis.argtypes = [vp, vp, i64, i32, i32, i32, vp]
         L.pbk_chirp.argtypes = [i64, i64, dbl, dbl, dbl, ctypes.POINTER(dbl), vp, i32, i32, vp]

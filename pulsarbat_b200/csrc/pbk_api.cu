@@ -31,6 +31,7 @@
 #include "pbk_hostcopy.h"
 #include "pbk_misc.cuh"
 #include "pbk_incoh.cuh"
+#include "pbk_search.cuh"
 
 using namespace pbk;
 
@@ -2865,6 +2866,125 @@ extern "C" int pbk_fold(const void* in, int64_t nsamp, int64_t row_elems, const 
   CUDA_TRY(cudaMemcpyAsync(counts, dc.p, cb, cudaMemcpyDeviceToHost, st));
   if (bins_out) CUDA_TRY(cudaMemcpyAsync(bins_out, db.p, bb, cudaMemcpyDeviceToHost, st));
   CUDA_TRY(cudaStreamSynchronize(st));
+  return PBK_OK;
+}
+
+// ------------------------------------------------------------------------------------------
+// single-pulse search: boxcar S/N at many widths, maximum over windows of starts (pbk_search.cuh)
+// ------------------------------------------------------------------------------------------
+// Shared memory of one boxcar CTA is at most this much, so that two CTAs fit an SM.
+static constexpr size_t kBoxSmemCap = 112 * 1024;
+
+extern "C" int pbk_boxcar_search(const void* in, int64_t nser, int64_t rows, int64_t ncols,
+                                 const int32_t* widths, int32_t nwidths, int64_t window,
+                                 void* stats, int32_t stats_given, void* snr, void* start,
+                                 void* width, int32_t on_device, int32_t device, void* stream) {
+  namespace ps = pbk_search;
+  if (nser < 1 || ncols < 1 || rows < 0)
+    return fail(PBK_ERR_INVALID, "bad shape (nser and ncols must be >= 1, rows >= 0)");
+  if (!widths) return fail(PBK_ERR_INVALID, "widths is NULL");
+  if (nwidths < 1 || nwidths > ps::kMaxWidths)
+    return fail(PBK_ERR_INVALID, "nwidths = %d: 1 to %d widths", nwidths, ps::kMaxWidths);
+  for (int k = 0; k < nwidths; ++k)
+    if (widths[k] < 1 || (k > 0 && widths[k] <= widths[k - 1]))
+      return fail(PBK_ERR_INVALID, "widths must be >= 1 and strictly increasing (widths[%d] = %d)",
+                  k, widths[k]);
+  if (window < 1) return fail(PBK_ERR_INVALID, "window must be >= 1");
+  if (rows == 0) return PBK_OK;
+  if (!in || !stats || !snr || !start || !width) return fail(PBK_ERR_INVALID, "NULL data pointer");
+  if (on_device && ((((uintptr_t)in | (uintptr_t)snr | (uintptr_t)start | (uintptr_t)width) & 3) ||
+                    ((uintptr_t)stats & 7)))
+    return fail(PBK_ERR_INVALID, "device arrays must be aligned to their element size");
+  const int wmax = widths[nwidths - 1];
+  if (wmax > ps::kMaxWidth)
+    return fail(PBK_ERR_UNSUPPORTED, "width %d: at most %d samples", wmax, ps::kMaxWidth);
+  if (rows > INT_MAX || ncols > INT_MAX || nser > INT_MAX || nser * ncols > INT_MAX)
+    return fail(PBK_ERR_UNSUPPORTED, "rows, ncols and nser * ncols must fit 32-bit indices");
+  if (nser * rows > LLONG_MAX / 8 / ncols) return fail(PBK_ERR_UNSUPPORTED, "input too large");
+  const int win = (int)std::min<int64_t>(window, rows);
+  const int nwin = (int)((rows + win - 1) / win);
+  // columns per CTA: the widest power of two <= min(ncols, 32) whose ring fits
+  int CW = 32, lr = 0, R = 0;
+  while (CW > ncols) CW /= 2;
+  for (;; CW /= 2) {
+    const int T = ps::kV * ps::kThreads / CW;
+    lr = (wmax + T - 1) / T * T;
+    for (R = 1; R < lr + T + 1; R *= 2) {}
+    if (CW == 1 || ps::boxcar_smem(CW, R + 1) <= kBoxSmemCap) break;
+  }
+  const size_t smem = ps::boxcar_smem(CW, R + 1);
+  const int ngroups = (int)((ncols + CW - 1) / CW);
+  CUDA_TRY(cudaSetDevice(device));
+  int nsm = 0;
+  CUDA_TRY(cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, device));
+  // runs of windows per series: enough CTAs for several waves, but runs of at least 4 (LR + T)
+  // starts so that the LR samples re-read at the start of a run stay a small share
+  const long long T = ps::kV * ps::kThreads / CW;
+  const long long want = (8LL * nsm + nser * ngroups - 1) / (nser * ngroups);
+  const long long by_halo = std::max<long long>(1, rows / (4 * (lr + T)));
+  long long runs = std::max<long long>(1, std::min(std::min(want, by_halo), (long long)nwin));
+  const long long wpr = (nwin + runs - 1) / runs;
+  runs = (nwin + wpr - 1) / wpr;
+  const long long grid = nser * ngroups * runs;
+  const long long nchunks = (rows + (long long)ps::kThreads / CW * ps::kStatPer - 1) /
+                            ((long long)ps::kThreads / CW * ps::kStatPer);
+  if (grid > INT_MAX || nser * ngroups * nchunks > INT_MAX)
+    return fail(PBK_ERR_UNSUPPORTED, "too many tiles for one launch");
+
+  cudaStream_t st = on_device ? reinterpret_cast<cudaStream_t>(stream) : cudaStreamPerThread;
+  const size_t ib = (size_t)nser * rows * ncols * 4, sb = (size_t)nser * ncols * 16,
+               ob = (size_t)nser * nwin * ncols * 4;
+  DevBuf di, ds, dsnr, dstart, dwidth;
+  const void* x = in;
+  void* d_stats = stats;
+  void* d_snr = snr;
+  void* d_start = start;
+  void* d_width = width;
+  if (!on_device) {
+    CUDA_TRY(cudaMalloc(&di.p, ib));
+    CUDA_TRY(cudaMalloc(&ds.p, sb));
+    CUDA_TRY(cudaMalloc(&dsnr.p, ob));
+    CUDA_TRY(cudaMalloc(&dstart.p, ob));
+    CUDA_TRY(cudaMalloc(&dwidth.p, ob));
+    CUDA_TRY(host_to_device(di.p, in, ib, st));
+    if (stats_given) CUDA_TRY(host_to_device(ds.p, stats, sb, st));
+    x = di.p, d_stats = ds.p, d_snr = dsnr.p, d_start = dstart.p, d_width = dwidth.p;
+  }
+  if (!stats_given) {
+    // the partials live in a stream-ordered allocation, freed behind the kernels
+    ps::StatArgs sa{};
+    sa.x = reinterpret_cast<const float*>(x);
+    sa.stats = reinterpret_cast<double*>(d_stats);
+    sa.rows = rows, sa.ncols = ncols, sa.nseries = nser * ncols;
+    sa.ngroups = ngroups, sa.nchunks = (int)nchunks;
+    void* part = nullptr;
+    CUDA_TRY(cudaMallocAsync(&part, (size_t)nser * ncols * nchunks * 24, st));
+    sa.part = reinterpret_cast<double*>(part);
+    cudaError_t e = ps::launch_stats(CW, sa, st);
+    cudaError_t ef = cudaFreeAsync(part, st);
+    if (e != cudaSuccess) return fail(PBK_ERR_CUDA, "statistics launch: %s", cudaGetErrorString(e));
+    CUDA_TRY(ef);
+  }
+  ps::BoxArgs a{};
+  a.x = reinterpret_cast<const float*>(x);
+  a.stats = reinterpret_cast<const double*>(d_stats);
+  a.snr = reinterpret_cast<float*>(d_snr);
+  a.start = reinterpret_cast<int*>(d_start);
+  a.width = reinterpret_cast<int*>(d_width);
+  a.rows = rows, a.ncols = ncols, a.window = win, a.nwin = nwin;
+  a.ngroups = ngroups, a.runs = (int)runs, a.wpr = (int)wpr;
+  a.nw = nwidths, a.wmax = wmax, a.lr = lr, a.mask = R - 1, a.rs = R + 1;
+  for (int k = 0; k < nwidths; ++k) a.widths[k] = widths[k];
+  CUDA_TRY(cudaFuncSetAttribute(ps::boxcar_kernel_of(CW), cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                (int)kBoxSmemCap));
+  cudaError_t e = ps::launch_boxcar(CW, a, (unsigned)grid, smem, st);
+  if (e != cudaSuccess) return fail(PBK_ERR_CUDA, "boxcar launch: %s", cudaGetErrorString(e));
+  if (!on_device) {
+    CUDA_TRY(device_to_host(snr, d_snr, ob, st));
+    CUDA_TRY(device_to_host(start, d_start, ob, st));
+    CUDA_TRY(device_to_host(width, d_width, ob, st));
+    if (!stats_given) CUDA_TRY(device_to_host(stats, d_stats, sb, st));
+  }
   return PBK_OK;
 }
 

@@ -24,7 +24,8 @@ from .device import DeviceArray
 
 __all__ = ["default_device", "dedisperse", "chirp", "detect", "shift_channels", "phase_ramp", "mix", "analytic_decimate", "stokes", "pol_basis",
            "downsample", "fft", "stft", "istft", "stft_detect", "stft_fold", "fold",
-           "dedisperse_fold", "dedisperse_trials", "incoherent_trials", "predict_phase", "clear_plan_cache",
+           "dedisperse_fold", "dedisperse_trials", "incoherent_trials", "boxcar_search", "predict_phase",
+           "clear_plan_cache",
            "pinned_results"]
 
 
@@ -699,6 +700,78 @@ def incoherent_trials(data, delays, rows, device=None):
         with ctx.lock:
             plan.exec_host(x, out)
         return out
+
+
+def boxcar_search(data, widths, window, stats=None, device=None):
+    """Single-pulse search of a stack of time series (pbk_boxcar_search): boxcar S/N at every
+    width and start, reduced to the best (snr, start, width) in each window of ``window`` starts.
+
+    ``data`` is (nser, rows, ...) float32, numpy or DeviceArray; series (s, c) is
+    ``data[s, :, c]`` with the trailing axes flattened into c.  ``snr(s, c, t, w) = (sum of w
+    samples from t - w * mean) / (std * sqrt(w))`` for ``t + w <= rows``, with the float64 mean and
+    population std of the series (0 where std is not > 0).  ``widths`` are strictly increasing,
+    1 to 32 of them, each 1..4096.  Window j holds the starts ``[j * window, (j + 1) * window)``;
+    ties go to the smallest start, then the smallest width; a window with no valid (start, width)
+    gives ``-inf, -1, -1``.  ``stats`` (nser, ..., 2) float64 ``(mean, std)`` replaces the
+    computed statistics when given.
+
+    Returns ``(snr, start, width, stats)`` on the side of the bus of ``data``: (nser, nwin, ...)
+    float32, int32, int32 with ``nwin = ceil(rows / window)``, and the (nser, ..., 2) float64
+    statistics used."""
+    shape = tuple(data.shape)
+    if len(shape) < 2:
+        raise ValueError("boxcar_search takes (nser, rows, ...) data")
+    if np.dtype(data.dtype) != np.float32:
+        raise TypeError(f"boxcar_search takes float32 data, got {np.dtype(data.dtype)}")
+    nser, rows = shape[0], shape[1]
+    trailing = shape[2:]
+    ncols = int(np.prod(trailing, dtype=np.int64)) if trailing else 1
+    w = np.ascontiguousarray(widths, dtype=np.int32)
+    if w.ndim != 1 or not np.array_equal(w, np.asarray(widths, dtype=np.int64).ravel()):
+        raise ValueError("widths must be a 1-D sequence of integers")
+    window = int(window)
+    if window < 1:
+        raise ValueError("window must be >= 1")
+    nwin = -(-rows // window)
+    out_shape = (nser, nwin) + trailing
+    st_shape = (nser,) + trailing + (2,)
+    wp = w.ctypes.data_as(ctypes.POINTER(ctypes.c_int32))
+    if _is_dev(data):
+        x = data.contiguous()
+        dev = x.device
+        given = stats is not None
+        if given:
+            if not _is_dev(stats) or tuple(stats.shape) != st_shape or stats.dtype != np.float64:
+                raise ValueError(f"stats must be a float64 DeviceArray of shape {st_shape}")
+            st = stats.contiguous()
+        else:                             # no rows: the statistics are undefined
+            st = DeviceArray.empty(st_shape, np.float64, dev)
+            if rows == 0:
+                st.tensor.fill_(float("nan"))
+        snr = DeviceArray.empty(out_shape, np.float32, dev)
+        start = DeviceArray.empty(out_shape, np.int32, dev)
+        width = DeviceArray.empty(out_shape, np.int32, dev)
+        L.check(L.lib().pbk_boxcar_search(L.ptr(x.ptr), nser, rows, ncols, wp, len(w), window,
+                                          L.ptr(st.ptr), int(given), L.ptr(snr.ptr),
+                                          L.ptr(start.ptr), L.ptr(width.ptr), 1, dev,
+                                          ctypes.c_void_p(_stream())))
+        return snr, start, width, st
+    x = np.ascontiguousarray(data)
+    dev = default_device() if device is None else device
+    given = stats is not None
+    if given:
+        st = np.ascontiguousarray(stats, dtype=np.float64)
+        if st.shape != st_shape:
+            raise ValueError(f"stats must have shape {st_shape}")
+    else:
+        st = np.full(st_shape, np.nan) if rows == 0 else np.empty(st_shape, np.float64)
+    snr = _result(out_shape, np.float32)
+    start = _result(out_shape, np.int32)
+    width = _result(out_shape, np.int32)
+    L.check(L.lib().pbk_boxcar_search(L.ptr(x), nser, rows, ncols, wp, len(w), window, L.ptr(st),
+                                      int(given), L.ptr(snr), L.ptr(start), L.ptr(width), 0, dev,
+                                      None))
+    return snr, start, width, st
 
 
 def phase_ramp(data, shift_samples=None, zero_lo=None, zero_hi=None, device=None):
