@@ -162,9 +162,8 @@ int pbk_dedisp_fold_exec_device(pbk_plan* plan, const void* d_in, void* d_profil
  * shared forward result; the per-trial inverse passes run in place in the other one.  When every
  * per-trial pass runs on the LDG fast kernels and has fewer tiles than the GPU holds CTAs, T > 1
  * trials run as one launch (gridDim.y = T; the other array then holds T slabs), with T chosen by the
- * plan for about two waves of CTAs and bounded by the memory of the slabs; otherwise T = 1.  The
- * L2-blocked schedules ($PBK_L2_CHUNK_MB, $PBK_L2PIPE) are not used.  Lengths that are not powers
- * of two (Bluestein) run their whole execution once per trial.  pbk_dedisp_fold_exec_device on a
+ * plan for about two waves of CTAs and bounded by the memory of the slabs; otherwise T = 1.
+ * Lengths that are not powers of two (Bluestein) run their whole execution once per trial.  pbk_dedisp_fold_exec_device on a
  * trial plan returns PBK_ERR_UNSUPPORTED.  pbk_plan_describe lists the shared passes, then
  * "TRIALS:ndm=<ndm>:per_launch=<T>" and the passes run per batch of T trials; pbk_plan_info and
  * pbk_plan_segments count the shared passes once and the per-trial launches once per batch, so
@@ -197,9 +196,9 @@ int pbk_dedisp_exec_blocks_device(pbk_plan* plan, const void* d_in, int64_t nblo
                                   void* stream);
 /* Blocks batched per launch (T) by pbk_dedisp_exec_blocks_device on a 16-byte aligned stream: about
  * two waves of resident CTAs in every pass, bounded by the memory of T slabs in each scratch array;
- * 1 when the plan cannot batch (a pass on the generic, TMA or warp-private kernels, a Bluestein
- * length, a one-level plan, the L2-blocked schedules, an output through the float buffer or a slab
- * that is not a multiple of 16 bytes), and for trial and ramp plans. */
+ * 1 when the plan cannot batch (a pass on the generic or TMA kernels, a Bluestein length, a
+ * one-level plan, an output through the float buffer or a slab that is not a multiple of 16 bytes),
+ * and for trial and ramp plans. */
 int pbk_plan_blocks_per_launch(const pbk_plan* plan, int32_t* T);
 
 /* ---- FFT-domain phase ramp / band mask ("next" rows: time_shift, freq_shift) ------------------
@@ -434,16 +433,14 @@ void pbk_plan_destroy(pbk_plan* plan);
 int pbk_plan_info(const pbk_plan* plan, int32_t* launches, int64_t* workspace_bytes,
                   int32_t* levels, int32_t* level_log2 /* [3] */);
 
-/* human-readable list of the passes of a plan: "FWD:L=2^11:fast-r8:W=4:tiles=65536:threads=512;..."
- * (passes joined by '+' run as one L2-blocked group, see pbk_plan_segments) */
+/* human-readable list of the passes of a plan: "FWD:L=2^11:fast-r8:W=4:tiles=65536:threads=512;..." */
 int pbk_plan_describe(const pbk_plan* plan, char* buf, size_t n);
 
 /* Per-launch device timing for benchmarks.  pbk_plan_profile(plan, nslots) makes every later
  * execution record a CUDA event before each kernel launch and after the last one, on the
  * execution stream, into slot (execution count mod nslots); nslots = 0 switches it off.
  * After synchronising, pbk_plan_profile_read returns the duration in ms of each timed segment of
- * one slot.  A segment is one kernel launch, except that the L2-blocked middle passes of a
- * 3-level plan (many small launches) form one segment; pbk_plan_segments gives their number and
+ * one slot.  A segment is one kernel launch; pbk_plan_segments gives their number and
  * pbk_plan_describe lists them separated by ';' (a trailing time-sum kernel is not listed). */
 int pbk_plan_segments(const pbk_plan* plan, int32_t* segments);
 int pbk_plan_profile(pbk_plan* plan, int32_t nslots);

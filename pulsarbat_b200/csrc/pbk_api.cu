@@ -23,8 +23,6 @@
 #include "../../include/pbk.h"
 #include "pbk_fast_launch.h"
 #include "pbk_tma_launch.h"
-#include "pbk_tsumw_launch.h"
-#include "pbk_l2pipe_launch.h"
 #include "pbk_blue.cuh"
 #include "pbk_f64.cuh"
 #include "pbk_fft.cuh"
@@ -114,8 +112,6 @@ struct Pass {
   // TMA-pipelined variant of the same tile shape (pbk_tma.cuh); decided by setup_tma
   bool tma = false;
   TmaInfo tinfo{};
-  // time-summing last pass on the warp-private kernel (pbk_tsumw.cuh): two swizzled half-tile boxes
-  bool tsumw = false;
 };
 
 struct BlueState;   // arbitrary-length (Bluestein) plans, see below
@@ -165,13 +161,6 @@ struct pbk_plan {
   pbk_dedisp_desc desc{};
   int64_t out_rows = 0, row_elems = 0, elem_bytes = 0, full_rows = 0;
   int launches = 0;
-  // L2-blocked schedule of the three middle passes of a 3-level plan (see run_passes)
-  // the three middle passes as one persistent L2-resident pipeline (pbk_l2pipe.cuh)
-  bool l2pipe = false;
-  unsigned* d_l2sync = nullptr;  // ticket | err | done[nblocks][2]
-  int l2pipe_blocks = 0;
-  int l2_chunks = 0;            // 0 = plain pass-after-pass schedule
-  long long l2_tiles[3] = {0, 0, 0};   // tiles per chunk of passes 1, 2, 3
   int segments = 0;             // timed segments per execution (pbk_plan_profile_read)
   // trial plans (pbk_dedisp_trials_plan_create): the forward passes run once per execution, the
   // MID pass and every pass after it once per trial DM, with that trial's chirp constants
@@ -619,17 +608,6 @@ static bool tma_encode(const Pass& ps, const void* base, CUtensorMap* tm) {
                                    : promo == 128 ? CU_TENSOR_MAP_L2_PROMOTION_L2_128B
                                    : promo == 64  ? CU_TENSOR_MAP_L2_PROMOTION_L2_64B
                                                   : CU_TENSOR_MAP_L2_PROMOTION_NONE;
-  if (ps.tsumw) {
-    // warp-private time sum (pbk_tsumw.cuh): the lane axis split into 128-byte chunks, one box =
-    // 32 floats x 2 chunks x 256 rows with the 128-byte swizzle
-    const cuuint64_t dims[5] = {32, I / 16, RI / I, L, (cuuint64_t)(a.Q / a.RI)};
-    const cuuint64_t strides[4] = {128, I * 8, RI * 8, L * RI * 8};
-    const cuuint32_t box[5] = {32, 2, 1, 256, 1};
-    const cuuint32_t es[5] = {1, 1, 1, 1, 1};
-    return enc(tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 5, const_cast<void*>(base), dims, strides, box,
-               es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, l2p,
-               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-  }
   const cuuint64_t dims[4] = {2 * I, RI / I, L, (cuuint64_t)(a.Q / a.RI)};
   const cuuint64_t strides[3] = {I * 8, RI * 8, L * RI * 8};
   const cuuint32_t box[4] = {(cuuint32_t)(4u << ps.tinfo.log2pw), 1, (cuuint32_t)ps.tinfo.box_rows, 1};
@@ -647,7 +625,6 @@ static void setup_tma(pbk_plan* pl) {
   int idx = -1;
   for (auto& ps : pl->passes) {
     ps.tma = false;
-    ps.tsumw = false;
     ++idx;
     if (only && atoi(only) != idx) continue;
     if (ps.family < 0 || ps.signinv || ps.fast_load_transposed) continue;
@@ -686,12 +663,6 @@ static void setup_tma(pbk_plan* pl) {
     if (!tma_kind_enabled(kind, a.log2L)) continue;
     ps.tma = true;
     ps.tinfo = ti;
-    // PBK_TSUMW=0: keep the thread-group kernel for the time-summing pass
-    // $PBK_TSUMW=1: the time-summing pass on the warp-private kernel (pbk_tsumw.cuh).  Opt-in: it
-    // is bit-identical but slower on B200 (cfg2: 1.13-1.18 ms against 0.95-0.97), see DESIGN.md 5.1e
-    const char* tw = getenv("PBK_TSUMW");
-    ps.tsumw = tsum && tw && tw[0] == '1' && tsumw_supported(a.log2L, ti.log2pw) &&
-               ti.box_rows == 256;
   }
 }
 
@@ -707,33 +678,6 @@ static int upload_tables(pbk_plan* pl, TableSet& ts) {
   return PBK_OK;
 }
 
-static void setup_l2_blocking(pbk_plan* pl, long long block_bytes, int nblocks);
-
-// $PBK_L2PIPE: 1 = run FWD(level 2) -> MID(level 3) -> INV(level 2) of a 3-level plan as the one
-// persistent kernel of pbk_l2pipe.cuh when the shapes are the instantiated ones (2^8 / 2^6 points,
-// wide tiles, generated chirp); unset / 0 = three launches.
-static bool l2pipe_wanted() {
-  const char* e = getenv("PBK_L2PIPE");
-  return e && strcmp(e, "0") != 0;
-}
-static int setup_l2pipe(pbk_plan* pl, int nblocks) {
-  pl->l2pipe = false;
-  if (!l2pipe_wanted() || pl->passes.size() != 5 || pl->l2_chunks > 0) return PBK_OK;
-  const Pass &a = pl->passes[1], &b = pl->passes[2], &c = pl->passes[3];
-  auto plain = [](const Pass& ps) {
-    return ps.family >= 0 && ps.in_role == ROLE_SCRATCH && ps.out_role == ROLE_SCRATCH &&
-           ps.a.load_kind == LOAD_PLANAR && ps.a.store_planar && !ps.a.final_epi && !ps.signinv;
-  };
-  if (!plain(a) || !plain(b) || !plain(c)) return PBK_OK;
-  if (a.mode != MODE_FWD || b.mode != MODE_MID || c.mode != MODE_INV) return PBK_OK;
-  if (a.a.log2L != 8 || c.a.log2L != 8 || b.a.log2L != 6 || b.a.split) return PBK_OK;
-  if (a.finfo.log2pw != 4 || b.finfo.log2pw != 5) return PBK_OK;
-  if (a.a.I % 64 || a.a.I % a.a.P || a.ntiles % nblocks || b.ntiles % (2ll * nblocks)) return PBK_OK;
-  CUDA_TRY(cudaMalloc(&pl->d_l2sync, (size_t)(2 + 2 * nblocks) * sizeof(unsigned)));
-  pl->l2pipe = true;
-  pl->l2pipe_blocks = nblocks;
-  return PBK_OK;
-}
 static void blue_free(BlueState* b);
 static int blue_exec(pbk_plan* pl, const void* d_in, void* d_out, const void* d_chirp,
                      cudaStream_t st, int trial = -1);
@@ -855,18 +799,17 @@ extern "C" int pbk_ramp_plan_create(int64_t nsamp, int64_t ncols, const double* 
 // [first, end) run as one launch with gridDim.y = T: just enough for two waves of resident CTAs in
 // every batched pass, at most `limit`, and bounded by the memory of T scratch slabs in each of the
 // `nbuf` batched scratch arrays (together within the 1/5-of-device rule of the second scratch
-// array).  Only the LDG fast kernels take a batch index; a batched pass on the generic, TMA or
-// warp-private kernels, the L2-blocked schedules, a Bluestein length, a one-level plan (a trial's
-// MID pass would read the caller's input), an output staged through d_tmpf and a slab that is not
-// a multiple of 16 bytes keep T = 1.
+// array).  Only the LDG fast kernels take a batch index; a batched pass on the generic or TMA
+// kernels, a Bluestein length, a one-level plan (a trial's MID pass would read the caller's
+// input), an output staged through d_tmpf and a slab that is not a multiple of 16 bytes keep T = 1.
 static int choose_per_launch(const pbk_plan* pl, size_t first, long long limit, int nbuf) {
-  if (pl->blue || pl->nlevels < 2 || pl->l2pipe || pl->l2_chunks > 0 || pl->split_ragged ||
+  if (pl->blue || pl->nlevels < 2 || pl->split_ragged ||
       pl->out_bytes % 16 || pl->passes.back().out_role != ROLE_USER_OUT)
     return 1;
   long long want = 1;
   for (size_t i = first; i < pl->passes.size(); ++i) {
     const Pass& ps = pl->passes[i];
-    if (ps.family < 0 || ps.tma || ps.tsumw || ps.ntiles <= 0) return 1;
+    if (ps.family < 0 || ps.tma || ps.ntiles <= 0) return 1;
     const long long resident = (long long)pl->num_sms * ps.finfo.minb;
     want = std::max(want, (2 * resident + ps.ntiles - 1) / ps.ntiles);
   }
@@ -1221,16 +1164,13 @@ static int dedisp_plan_create_impl(const pbk_dedisp_desc* d, const RampSpec* ram
     ps.a.bd = std::isinf(d->ref_freq_hz) ? 0.0
                                          : (d->sample_rate_hz / (double)N) / d->ref_freq_hz;
   }
-  // trial plans take the plain schedule: FWD level 2 sits inside the L2-blocked groups
-  if (m == 3 && !tr.trials) setup_l2_blocking(pl, (N >> l[0]) * I * 8, 1 << l[0]);
-  if (m == 3 && !tr.trials && (rc = setup_l2pipe(pl, 1 << l[0])) != PBK_OK) return cleanup(rc);
   // Out-of-place intermediate passes: a pass that reads and writes the same scratch array is
   // 2-3 % slower than one that writes another array (cfg2: 1.505 -> 1.463 ms and 1.476 -> 1.426 ms,
   // profiles/r01_pingpong_scratch.log), so when the scratch is small against the device memory
   // (<= 1/5 of it, and 3x its size still free: a 34 GB cfg5 shard qualifies on a 180 GB part) a
   // second one is allocated and pass i reads
   // buffer (i-1)&1 and writes buffer i&1.  PBK_NO_PINGPONG=1 keeps the passes in place.
-  if (pl->scratch && pl->l2_chunks == 0 && !getenv("PBK_NO_PINGPONG")) {
+  if (pl->scratch && !getenv("PBK_NO_PINGPONG")) {
     bool any = false;
     for (const auto& ps : pl->passes)
       any = any || (ps.in_role == ROLE_SCRATCH && ps.out_role == ROLE_SCRATCH);
@@ -1250,18 +1190,10 @@ static int dedisp_plan_create_impl(const pbk_dedisp_desc* d, const RampSpec* ram
                           cudaGetErrorString(e)));
     }
   }
-  if (pl->l2_chunks == 0) setup_tma(pl);
+  setup_tma(pl);
   const int ds = (d->downsample > 1 && !pl->fused_tsum) ? 1 : 0;
-  if (pl->l2pipe) {
-    pl->launches = 3 + ds;
-    pl->segments = 3 + ds;
-  } else if (pl->l2_chunks > 0) {
-    pl->launches = 2 + 3 * pl->l2_chunks + ds;
-    pl->segments = 3 + ds;
-  } else {
-    pl->launches = (int)pl->passes.size() + ds;
-    pl->segments = pl->launches;
-  }
+  pl->launches = (int)pl->passes.size() + ds;
+  pl->segments = pl->launches;
   if (tr.trials && (rc = set_trials(pl, tr)) != PBK_OK) return cleanup(rc);
   if (!tr.trials && !ramp) set_blocks_per_launch(pl);
   *out = pl;
@@ -1277,10 +1209,22 @@ extern "C" int pbk_dedisp_out_shape(const pbk_plan* pl, int64_t* rows, int64_t* 
   return PBK_OK;
 }
 
-static void* role_ptr(const pbk_plan* pl, int role, const void* uin, void* uout) {
+// the scratch arrays one pass reads (if its input is scratch) and writes (if its output is)
+struct ScratchPair {
+  void* in;
+  void* out;
+};
+
+// Pass i of a schedule that works in the pair of arrays buf: with a second array the passes
+// ping-pong, pass i reading buffer (i-1)&1 and writing buffer i&1; otherwise they work in place.
+static ScratchPair pass_scratch(void* const buf[2], size_t i) {
+  return {buf[1] ? buf[(i + 1) & 1] : buf[0], buf[1] ? buf[i & 1] : buf[0]};
+}
+
+static void* role_ptr(const pbk_plan* pl, int role, const void* uin, void* uout, void* scr) {
   switch (role) {
     case ROLE_USER_IN: return const_cast<void*>(uin);
-    case ROLE_SCRATCH: return pl->scratch;
+    case ROLE_SCRATCH: return scr;
     case ROLE_USER_OUT: return uout;
     default: return pl->d_tmpf;
   }
@@ -1288,10 +1232,10 @@ static void* role_ptr(const pbk_plan* pl, int role, const void* uin, void* uout)
 
 static bool misaligned16(const void* p) { return ((uintptr_t)p & 15) != 0; }
 
-// Epilogues that only the compile-time-shaped (fast / TMA / warp-private) kernels implement: the
-// time sum (and the fold behind it), the detection with its frequency sum (and fold), and the even
-// / odd recombination.  The generic pass_kernel would silently skip them and write a differently
-// shaped result, so such a pass never takes it.
+// Epilogues that only the compile-time-shaped (fast / TMA) kernels implement: the time sum (and the
+// fold behind it), the detection with its frequency sum (and fold), and the even / odd
+// recombination.  The generic pass_kernel would silently skip them and write a differently shaped
+// result, so such a pass never takes it.
 static bool needs_fast_kernel(const Pass& ps) {
   return ps.a.tsum_log2 > 0 || ps.a.fsum_log2 > 0 || ps.a.fsum_split || ps.a.split;
 }
@@ -1315,21 +1259,11 @@ static int stage_ensure(pbk_plan* pl, size_t bytes) {
 }
 
 static int launch_one(pbk_plan* pl, const Pass& ps, const void* d_in, void* d_out,
-                      const void* d_chirp, long long tile0, long long tile_end, cudaStream_t st,
-                      int idx = 0, void* scr_in = nullptr, void* scr_out = nullptr) {
+                      const void* d_chirp, ScratchPair scr, cudaStream_t st) {
   Pass p = ps;
-  p.a.in = role_ptr(pl, ps.in_role, d_in, d_out);
-  p.a.out = role_ptr(pl, ps.out_role, d_in, d_out);
-  if (scr_in || scr_out) {   // the trial schedule names its scratch arrays (run_trial_passes)
-    if (ps.in_role == ROLE_SCRATCH) p.a.in = scr_in;
-    if (ps.out_role == ROLE_SCRATCH) p.a.out = scr_out;
-  } else if (pl->scratch2) {   // pass idx reads buffer (idx-1)&1 and writes buffer idx&1
-    void* buf[2] = {pl->scratch, pl->scratch2};
-    if (ps.in_role == ROLE_SCRATCH) p.a.in = buf[(idx + 1) & 1];
-    if (ps.out_role == ROLE_SCRATCH) p.a.out = buf[idx & 1];
-  }
+  p.a.in = role_ptr(pl, ps.in_role, d_in, d_out, scr.in);
+  p.a.out = role_ptr(pl, ps.out_role, d_in, d_out, scr.out);
   p.a.chirp_arr = reinterpret_cast<const float2*>(d_chirp);
-  p.a.tile0 = tile0;
   if (p.a.fsum_log2 > 0) p.a.fsum_bins = pl->exec_segbins;
   if (p.a.tsum_log2 > 0) p.a.tsum_bins = pl->exec_segbins;
   const bool aligned = (((uintptr_t)p.a.in | (uintptr_t)p.a.out) & 15) == 0;
@@ -1344,15 +1278,14 @@ static int launch_one(pbk_plan* pl, const Pass& ps, const void* d_in, void* d_ou
                 "aligned arrays", p.a.trials);
   cudaError_t e;
   CUtensorMap tm;
-  if (ps.tma && aligned && tile0 == 0 && tile_end < 0 && tma_encode(ps, p.a.in, &tm)) {
-    e = ps.tsumw ? tsumw_launch(p.a, tm, pl->d_ftab + ps.ftab_off, ps.ntiles, pl->num_sms, st)
-                 : tma_launch(ps.a.log2L, ps.mode, p.a, tm, pl->d_ftab + ps.ftab_off, ps.ntiles,
-                              pl->num_sms, st);
+  if (ps.tma && aligned && tma_encode(ps, p.a.in, &tm)) {
+    e = tma_launch(ps.a.log2L, ps.mode, p.a, tm, pl->d_ftab + ps.ftab_off, ps.ntiles, pl->num_sms,
+                   st);
   } else if (ps.family >= 0 && aligned) {
     if (ps.fast_load_transposed)
       p.a.load_kind = ps.a.load_kind == LOAD_PLANAR ? LOAD_TRANSP_PLANAR : LOAD_TRANSP;
-    e = fast_launch(ps.family, ps.a.log2L, ps.mode, p.a, pl->d_ftab + ps.ftab_off,
-                    tile_end < 0 ? ps.ntiles : tile_end, pl->num_sms, st);
+    e = fast_launch(ps.family, ps.a.log2L, ps.mode, p.a, pl->d_ftab + ps.ftab_off, ps.ntiles,
+                    pl->num_sms, st);
   }
   else
     e = launch_pass(p, ps.fast && aligned, st);
@@ -1360,88 +1293,30 @@ static int launch_one(pbk_plan* pl, const Pass& ps, const void* d_in, void* d_ou
   return PBK_OK;
 }
 
-// Pass schedule.  Plain: one launch per pass over the whole array.  L2-blocked (3-level plans on
-// the fast kernels): after the first forward level the array is 2^l1 independent contiguous
-// blocks (one per k1); the three middle passes (FWD level 2, MID level 3, INV level 2) work in
-// place inside a block, so they are launched block-chunk by block-chunk with chunks sized to stay
-// resident in the 126 MB L2: HBM sees one read and one write for the three passes instead of
-// three of each.
+// Passes [0, end) of the plan (every pass when end < 0), one launch each, ping-ponging between
+// the plan's scratch arrays; timed segment i is pass i.  A whole execution also records the closing
+// mark.  A trial plan runs its shared passes here (end = nshared), and the first batch of trials
+// records that mark as its own first one (run_trial_passes).
 static int run_passes(pbk_plan* pl, const void* d_in, void* d_out, const void* d_chirp,
-                      cudaStream_t st) {
+                      cudaStream_t st, int end = -1) {
+  const int np = (int)pl->passes.size();
+  if (end < 0) end = np;
   prof_begin(pl);
-  int seg = 0, rc;
-  const size_t np = pl->passes.size();
-  const bool aligned = ((((uintptr_t)d_in | (uintptr_t)d_out | (uintptr_t)pl->scratch) & 15) == 0);
-  if (pl->l2pipe && aligned) {
-    prof_mark(pl, seg++, st);
-    if ((rc = launch_one(pl, pl->passes[0], d_in, d_out, d_chirp, 0, -1, st, 0)) != PBK_OK) return rc;
-    prof_mark(pl, seg++, st);
-    PassArgs pa[3];
-    for (int j = 0; j < 3; ++j) {      // the pointers launch_one would give passes 1..3
-      const Pass& ps = pl->passes[1 + j];
-      pa[j] = ps.a;
-      void* buf[2] = {pl->scratch, pl->scratch2 ? pl->scratch2 : pl->scratch};
-      pa[j].in = buf[pl->scratch2 ? (j + 2) & 1 : 0];
-      pa[j].out = buf[pl->scratch2 ? (j + 1) & 1 : 0];
-      pa[j].tile0 = 0;
-    }
-    const size_t sync_bytes = (size_t)(2 + 2 * pl->l2pipe_blocks) * sizeof(unsigned);
-    if (cudaMemsetAsync(pl->d_l2sync, 0, sync_bytes, st) != cudaSuccess)
-      return fail(PBK_ERR_CUDA, "l2 pipeline reset: %s", cudaGetErrorString(cudaGetLastError()));
-    L2PipeArgs q;
-    q.nblocks = pl->l2pipe_blocks;
-    q.tiles_a = pl->passes[1].ntiles / q.nblocks;
-    q.tiles_b = pl->passes[2].ntiles / q.nblocks;
-    q.ticket = pl->d_l2sync;
-    q.err = pl->d_l2sync + 1;
-    q.done = pl->d_l2sync + 2;
-    cudaError_t e = l2pipe_launch_l8_l6(pa[0], pa[1], pa[2], pl->d_ftab + pl->passes[1].ftab_off,
-                                        pl->d_ftab + pl->passes[2].ftab_off, q, pl->num_sms, st);
-    if (e != cudaSuccess) return fail(PBK_ERR_CUDA, "l2 pipeline launch: %s", cudaGetErrorString(e));
-    prof_mark(pl, seg++, st);
-    if ((rc = launch_one(pl, pl->passes[4], d_in, d_out, d_chirp, 0, -1, st, 4)) != PBK_OK) return rc;
-    prof_mark(pl, seg, st);
-    return PBK_OK;
-  }
-  if (pl->l2_chunks > 0 && aligned) {
-    prof_mark(pl, seg++, st);
-    if ((rc = launch_one(pl, pl->passes[0], d_in, d_out, d_chirp, 0, -1, st)) != PBK_OK) return rc;
-    prof_mark(pl, seg++, st);
-    for (int c = 0; c < pl->l2_chunks; ++c)
-      for (int j = 0; j < 3; ++j) {
-        const long long t0 = (long long)c * pl->l2_tiles[j];
-        if ((rc = launch_one(pl, pl->passes[1 + j], d_in, d_out, d_chirp, t0,
-                             t0 + pl->l2_tiles[j], st)) != PBK_OK)
-          return rc;
-      }
-    prof_mark(pl, seg++, st);
-    if ((rc = launch_one(pl, pl->passes[4], d_in, d_out, d_chirp, 0, -1, st)) != PBK_OK) return rc;
-    prof_mark(pl, seg, st);
-    return PBK_OK;
-  }
-  for (size_t i = 0; i < np; ++i) {
-    prof_mark(pl, seg++, st);
-    if ((rc = launch_one(pl, pl->passes[i], d_in, d_out, d_chirp, 0, -1, st, (int)i)) != PBK_OK)
-      return rc;
-  }
-  prof_mark(pl, seg, st);
-  return PBK_OK;
-}
-
-// Trial schedule.  The shared forward passes run once, ping-ponging between the two scratch arrays
-// as in the plain schedule; their result stays where the last of them wrote it.  Each batch of up
-// to T trials then runs MID from that result into the other array (slab y of T for trial k0 + y),
-// the inverse passes in place there, and the last pass into its output slabs.  One-level plans
-// share nothing: every trial reads the caller's input.
-static int run_shared_passes(pbk_plan* pl, const void* d_in, cudaStream_t st) {
-  for (int i = 0; i < pl->nshared; ++i) {
+  void* const buf[2] = {pl->scratch, pl->scratch2};
+  for (int i = 0; i < end; ++i) {
     prof_mark(pl, i, st);
-    const int rc = launch_one(pl, pl->passes[i], d_in, nullptr, nullptr, 0, -1, st, i);
+    const int rc = launch_one(pl, pl->passes[i], d_in, d_out, d_chirp, pass_scratch(buf, i), st);
     if (rc != PBK_OK) return rc;
   }
+  if (end == np) prof_mark(pl, np, st);
   return PBK_OK;
 }
 
+// Trial schedule.  The shared forward passes run once (run_passes up to nshared); their result
+// stays where the last of them wrote it.  Each batch of up to T trials then runs MID from that
+// result into the other array (slab y of T for trial k0 + y), the inverse passes in place there,
+// and the last pass into its output slabs.  One-level plans share nothing: every trial reads the
+// caller's input.
 static int run_trial_passes(pbk_plan* pl, const void* d_in, void* d_out, cudaStream_t st, int k,
                             int t, int seg) {
   const int ns = pl->nshared;
@@ -1460,35 +1335,12 @@ static int run_trial_passes(pbk_plan* pl, const void* d_in, void* d_out, cudaStr
                                                         : (long long)pl->scratch_bytes;
     }
     prof_mark(pl, seg++, st);
-    const int rc = launch_one(pl, q, d_in, d_out, nullptr, 0, -1, st, (int)i,
-                              (int)i == ns ? shared : work, work);
+    const int rc =
+        launch_one(pl, q, d_in, d_out, nullptr, {(int)i == ns ? shared : work, work}, st);
     if (rc != PBK_OK) return rc;
   }
   prof_mark(pl, seg, st);
   return PBK_OK;
-}
-
-// decide whether the L2-blocked schedule applies (called once the fast kernels are chosen)
-static void setup_l2_blocking(pbk_plan* pl, long long block_bytes, int nblocks) {
-  pl->l2_chunks = 0;
-  if (pl->passes.size() != 5) return;
-  for (int j = 1; j <= 3; ++j) {
-    const Pass& ps = pl->passes[j];
-    if (ps.family < 0 || ps.in_role != ROLE_SCRATCH || ps.out_role != ROLE_SCRATCH) return;
-  }
-  long long target = 0;   // off by default: on B200 the small launches cost more than the saved HBM traffic
-  if (const char* e = getenv("PBK_L2_CHUNK_MB")) target = atoll(e) << 20;
-  if (target <= 0) return;
-  long long per = std::max<long long>(1, target / block_bytes);   // blocks per chunk
-  while (nblocks % per) --per;
-  const int chunks = (int)(nblocks / per);
-  if (chunks < 2) return;
-  for (int j = 0; j < 3; ++j) {
-    const Pass& ps = pl->passes[1 + j];
-    if (ps.ntiles % chunks) return;
-    pl->l2_tiles[j] = ps.ntiles / chunks;
-  }
-  pl->l2_chunks = chunks;
 }
 
 static int exec_dedisp(pbk_plan* pl, const void* d_in, void* d_out, const void* d_chirp,
@@ -1516,8 +1368,7 @@ extern "C" int pbk_dedisp_exec_device(pbk_plan* pl, const void* d_in, void* d_ou
         return rc;
     return PBK_OK;
   }
-  prof_begin(pl);
-  if ((rc = run_shared_passes(pl, d_in, st)) != PBK_OK) return rc;
+  if ((rc = run_passes(pl, d_in, nullptr, nullptr, st, pl->nshared)) != PBK_OK) return rc;
   const int T = pl->trials_per_launch;
   for (int b = 0; b * T < pl->ndm; ++b)
     if ((rc = exec_dedisp(pl, d_in, out + (size_t)b * T * pl->out_bytes, nullptr, st, b)) != PBK_OK)
@@ -1576,7 +1427,6 @@ static int run_block_batch(pbk_plan* pl, const char* in, char* out, int t, size_
                            cudaStream_t st) {
   if (pl->fused_tsum)   // the last pass adds its group sums to the output
     CUDA_TRY(cudaMemsetAsync(out, 0, (size_t)t * pl->out_bytes, st));
-  void* const* buf = pl->blk_scratch;
   for (size_t i = 0; i < pl->passes.size(); ++i) {
     Pass q = pl->passes[i];
     q.a.trials = t;
@@ -1584,9 +1434,7 @@ static int run_block_batch(pbk_plan* pl, const char* in, char* out, int t, size_
                                                    : (long long)pl->scratch_bytes;
     q.a.trial_out_bytes = q.out_role == ROLE_USER_OUT ? (long long)pl->out_bytes
                                                       : (long long)pl->scratch_bytes;
-    void* scr_in = buf[1] ? buf[(i + 1) & 1] : buf[0];
-    void* scr_out = buf[1] ? buf[i & 1] : buf[0];
-    const int rc = launch_one(pl, q, in, out, nullptr, 0, -1, st, (int)i, scr_in, scr_out);
+    const int rc = launch_one(pl, q, in, out, nullptr, pass_scratch(pl->blk_scratch, i), st);
     if (rc != PBK_OK) return rc;
   }
   return PBK_OK;
@@ -2421,7 +2269,6 @@ extern "C" void pbk_plan_destroy(pbk_plan* pl) {
   cudaFree(pl->d_segbins);
   cudaFree(pl->d_foldbuf);
   cudaFree(pl->d_stage);
-  cudaFree(pl->d_l2sync);
   cudaFree(pl->d_incoh);
   cudaFree(pl->h_din);
   cudaFree(pl->h_dout);
@@ -2475,13 +2322,11 @@ extern "C" int pbk_plan_describe(const pbk_plan* pl, char* buf, size_t n) {
       if (w < 0 || off + (size_t)w + 1 >= n) break;
       off += (size_t)w;
     }
-    // segments are separated by ';'; the passes of an L2-blocked group are joined by '+'
-    const bool blocked = pl->l2_chunks > 0 || pl->l2pipe;
     const bool first = i == 0 && !(pl->trials && pl->nshared == 0);
-    const char* sep = first ? "" : (blocked && (i == 2 || i == 3)) ? "+" : ";";
+    const char* sep = first ? "" : ";";
     if (ps.family >= 0)
       w = snprintf(buf + off, n - off, "%s%s:L=2^%d:%s:W=%d:tiles=%lld:threads=%d%s%s", sep,
-                   mode, ps.a.log2L, ps.tsumw ? "tmaw-r16" : ps.tma ? "tma-r16" : "fast-r16",
+                   mode, ps.a.log2L, ps.tma ? "tma-r16" : "fast-r16",
                    2 << ps.finfo.log2pw, ps.ntiles, ps.tma ? ps.tinfo.threads : ps.finfo.threads,
                    ps.a.tsum_log2 > 0 ? ":timesum" : "",
                    ps.a.split || ps.a.fsum_split ? ":evenodd" : "");
@@ -2491,13 +2336,6 @@ extern "C" int pbk_plan_describe(const pbk_plan* pl, char* buf, size_t n) {
                    ps.grid, kThreads);
     if (w < 0) break;
     off += (size_t)w;
-    if (pl->l2pipe && i == 3 && off + 1 < n) {
-      w = snprintf(buf + off, n - off, ":l2pipe=%d", pl->l2pipe_blocks);
-      if (w > 0) off += (size_t)w;
-    } else if (blocked && i == 3 && off + 1 < n) {
-      w = snprintf(buf + off, n - off, ":l2chunks=%d", pl->l2_chunks);
-      if (w > 0) off += (size_t)w;
-    }
   }
   return PBK_OK;
 }

@@ -71,16 +71,6 @@ __device__ __forceinline__ void tma_load_4d(void* dst, const CUtensorMap* map, i
       "l"(map), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(smem_u32(bar))
       : "memory");
 }
-// rank-5 variant (pbk_tsumw.cuh: the lane axis split into 128-byte chunks so that the box can carry
-// the 128-byte swizzle while a tile row stays one contiguous 256-byte run in global memory)
-__device__ __forceinline__ void tma_load_5d(void* dst, const CUtensorMap* map, int c0, int c1,
-                                            int c2, int c3, int c4, uint64_t* bar) {
-  asm volatile(
-      "cp.async.bulk.tensor.5d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, "
-      "{%2, %3, %4, %5, %6}], [%7];" ::"r"(smem_u32(dst)),
-      "l"(map), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(c4), "r"(smem_u32(bar))
-      : "memory");
-}
 // orders this thread's earlier generic-proxy accesses to shared memory before later async-proxy
 // (TMA) accesses to the same addresses
 __device__ __forceinline__ void fence_proxy_async() {

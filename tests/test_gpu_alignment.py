@@ -227,7 +227,6 @@ def _offs(elem, names=("in", "out")):
 
 
 C64_IO = _offs(8)
-MOVED_IN = ({"in": 8}, {"in": 8, "out": 8})     # moved input: the plain pass-after-pass schedule
 TSUM_IO = _offs({"in": 8, "out": 4})     # float32 out: +4, +12
 
 L666 = {"PBK_LEVELS": "6,6,6"}
@@ -247,8 +246,6 @@ ROWS = [
         {**L886, "PBK_TMA": "1"}, ("last:tma-r16", ":timesum")),
     Row("dedisp-timesum-perpol-tma", dedisp(2 ** 20, 32, 2, 1, 8, (1000, 2 ** 20 - 3000)),
         TSUM_IO, {**L886, "PBK_TMA": "1"}, ("last:tma-r16", ":timesum")),
-    Row("dedisp-timesum-warp", dedisp(2 ** 20, 32, 2, 2, 64, (12345, 2 ** 20 - 777)), TSUM_IO,
-        {**L886, "PBK_TMA": "1", "PBK_TSUMW": "1"}, ("last:tmaw-r16", ":timesum")),
     Row("dedisp-unfused-sum", dedisp(2 ** 16, 16, 2, 2, 64, (4100, 2 ** 16 - 1000)), TSUM_IO,
         {"PBK_NO_FUSED_SUM": "1"}, ()),
     Row("dedisp-evenodd-odd-crop", dedisp(2 ** 16, 1, 1, crop=(3, 2 ** 16 - 5)), C64_IO, {},
@@ -269,10 +266,6 @@ ROWS = [
         ("generic",)),
     Row("dedisp-bluestein", dedisp(4233, 3, 2, 1, 1, (4, 4200)), _offs({"in": 8, "out": 4}), {},
         ("BLUESTEIN",)),
-    Row("dedisp-l2pipe", dedisp(2 ** 20, 64, 2, crop=(77, 2 ** 20 - 101)), MOVED_IN,
-        {"PBK_LEVELS": "6,8,6", "PBK_L2PIPE": "1"}, ("l2pipe",)),
-    Row("dedisp-l2chunks", dedisp(2 ** 18, 32, 2), MOVED_IN,
-        {**L666, "PBK_L2_CHUNK_MB": "1"}, ("l2chunks",)),
 ]
 
 

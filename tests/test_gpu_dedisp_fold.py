@@ -3,7 +3,7 @@
 oracle and against the two steps it replaces.
 
 ROWS lists shapes that reach every route of the fold: the time sum fused into the last inverse
-pass on the TMA, LDG and warp-private kernels (the group sums go straight into profile[bin]), and
+pass on the TMA and LDG kernels (the group sums go straight into profile[bin]), and
 the plans that run their normal execution into a plan-owned buffer and fold that (no time sum, a
 factor too large to fuse, Bluestein lengths, one single-pol column, PBK_NO_FUSED_SUM=1), with
 complex64 and raw int8 / u4 input.  At these sizes the fold call itself takes its two-step
@@ -57,8 +57,6 @@ ROWS = [
         "tma-r16:W=32"),
     Row(2 ** 20, 32, 2, 1, 8, (1000, 2 ** 20 - 3000), "c64", {**L886, "PBK_TMA": "0"},
         "fast-r16"),
-    Row(2 ** 20, 32, 2, 2, 64, (12345, 2 ** 20 - 777), "c64",
-        {**L886, "PBK_TMA": "1", "PBK_TSUMW": "1"}, "tmaw-r16"),
     Row(2 ** 16, 16, 2, 1, 1, (100, 2 ** 16 - 50), "c64", {}, None),            # no time sum
     Row(2 ** 16, 64, 2, 2, 1024, (0, 2 ** 16), "c64", {}, None),               # factor too large
     Row(3 * 2 ** 14, 8, 2, 2, 16, (77, 3 * 2 ** 14 - 99), "c64", {}, None),    # Bluestein
@@ -185,8 +183,7 @@ def test_fold_matches_oracle_and_two_steps(row, monkeypatch):
 
 
 @pytest.mark.parametrize("out_kind, ds, nbin", [(1, 4, 2048), (2, 2, 4096)])
-@pytest.mark.parametrize("env", [{}, {"PBK_TMA": "0"}, {"PBK_TMA": "1", "PBK_TSUMW": "1"}],
-                         ids=["tma", "ldg", "warp"])
+@pytest.mark.parametrize("env", [{}, {"PBK_TMA": "0"}], ids=["tma", "ldg"])
 def test_fused_fold_route(out_kind, ds, nbin, env, monkeypatch):
     """cfg2 geometry with an intensity of >= 256 MiB and <= 512 rows per bin: the fold call adds
     the group sums of the time-summing pass straight into the profile.  Counts equal the float64
@@ -196,7 +193,7 @@ def test_fused_fold_route(out_kind, ds, nbin, env, monkeypatch):
     row = Row(2 ** 22, 64, 2, out_kind, ds, (4097, 2 ** 22 - 1001), "c64", env, ":timesum")
     plan = _plan(row, monkeypatch)
     desc = plan.describe().split(";")[-1]
-    assert ":timesum" in desc and ("tmaw-r16" in desc) == ("PBK_TSUMW" in env), desc
+    assert ":timesum" in desc, desc
     rows, relems = plan.out_rows, plan.row_elems
     assert rows * relems * 4 >= 256 << 20 and rows <= 512 * nbin
     g = torch.Generator(device="cuda")

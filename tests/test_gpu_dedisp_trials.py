@@ -110,8 +110,6 @@ ROWS = [
         env={**L886, "PBK_TMA": "1"}, route=("tma-r16", ":timesum")),
     Row("unfused-sum", 2 ** 16, 16, 2, 2, 64, (4100, 2 ** 16 - 1000),
         env={"PBK_NO_FUSED_SUM": "1"}, route=("TRIALS",), not_route=(":timesum",)),
-    Row("l2chunks-ignored", 2 ** 18, 32, 2, crop=(9, 2 ** 18 - 9),
-        env={**L666, "PBK_L2_CHUNK_MB": "1"}, route=("TRIALS",), not_route=("l2chunks",)),
     Row("many-trials", 2 ** 16, 16, 2, 1, crop=(11, 2 ** 16 - 13),
         route=("TRIALS:ndm=7",), dms=(DM, 0.0, -0.3, 2.0, -1.25, 7.5, 1e-3)),
     # trials batched along gridDim.y (small blocks: fewer tiles than resident CTAs)
@@ -187,8 +185,6 @@ def test_trials_route(row, monkeypatch):
 
     # single-DM plans into aligned arrays: the bits every trial must reproduce
     singles = [L.DedispPlan(dm=dm, **_desc_kw(L, row, freqs)) for dm in dms]
-    if "PBK_L2_CHUNK_MB" in row.env:
-        assert "l2chunks" in singles[0].describe()
     one = singles[0].out_array()
     ref = []
     for p in singles:

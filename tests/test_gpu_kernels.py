@@ -1248,46 +1248,6 @@ def test_tma_passes_are_bit_identical_to_ldg_passes(monkeypatch, n, C, P, out_ki
     assert torch.equal(outs[0], outs[1]), descs[1]
 
 
-@pytest.mark.parametrize("n, C, P, out_kind, ds, crop, levels", [
-    (20, 32, 2, 2, 64, (12345, 2 ** 20 - 777), "8,6,6"),   # Stokes I, ragged crop
-    (20, 32, 2, 1, 8, (1000, 2 ** 20 - 3000), "8,6,6"),    # per-pol intensity
-    (21, 64, 1, 1, 4, None, "8,7,6"),                      # single pol
-])
-def test_warp_private_time_sum_is_bit_identical(monkeypatch, n, C, P, out_kind, ds, crop, levels):
-    """PBK_TSUMW=1: the time-summing last pass with warp-private columns (csrc/pbk_tsumw.cuh: both
-    radix-16 stages of a column inside one warp, a rank-5 swizzled TMA box, no group barrier) must
-    give the bits of the thread-group kernel.  Opt-in: it is slower on B200
-    (profiles/r02_tsum_warp_private.log)."""
-    import torch
-    L = _lib()
-    N = 2 ** n
-    sr, fcen = 6.25e6, 600e6
-    freqs = fcen + sr * (np.arange(C) + 0.5 - C / 2)
-    g = torch.Generator(device="cuda")
-    g.manual_seed(n * 7 + C)
-    x = torch.randn((N, C, P, 2), device="cuda", dtype=torch.float32, generator=g)
-    monkeypatch.setenv("PBK_LEVELS", levels)
-    monkeypatch.setenv("PBK_TMA", "1")
-    outs, descs = [], []
-    for warp in ("0", "1"):
-        monkeypatch.setenv("PBK_TSUMW", warp)
-        plan = L.DedispPlan(nsamp=N, nchan=C, npol=P, dm=3.0, sample_rate_hz=sr, ref_freq_hz=fcen,
-                            chan_freq_hz=freqs, crop=crop or (0, N), out_kind=out_kind,
-                            downsample=ds)
-        nout = plan.out_rows * plan.row_elems * plan.elem_bytes
-        out = torch.zeros(nout, device="cuda", dtype=torch.uint8)
-        for _ in range(2):
-            out.zero_()
-            plan.exec_device(x.data_ptr(), out.data_ptr(), None,
-                             torch.cuda.current_stream().cuda_stream)
-        torch.cuda.synchronize()
-        outs.append(out.clone())
-        descs.append(plan.describe())
-        plan.destroy()
-    assert "tmaw-r16" not in descs[0] and "tmaw-r16" in descs[1], descs
-    assert torch.equal(outs[0], outs[1]), descs[1]
-
-
 def test_plan_execution_replays_from_a_cuda_graph():
     """A plan execution only enqueues kernels (and one memset for the fused time sum) on the
     caller's stream: it can be captured into a CUDA graph -- programmatic dependent launches
@@ -1323,37 +1283,3 @@ def test_plan_execution_replays_from_a_cuda_graph():
         del graph
         plan.destroy()
 
-
-def test_l2_pipeline_of_the_middle_passes_is_bit_identical(monkeypatch):
-    """PBK_L2PIPE=1: FWD(level 2) -> MID(level 3) -> INV(level 2) as one persistent, ticket-ordered
-    kernel with per-block completion counters (csrc/pbk_l2pipe.cuh) must give exactly the output
-    of three launches (same per-tile arithmetic).  Opt-in: on B200 it is not faster
-    (profiles/r02_l2pipe_real_kernels.log)."""
-    import torch
-    L = _lib()
-    for (n, C, P, out_kind, ds, crop) in [(20, 64, 2, 0, 1, (77, 2 ** 20 - 101)),
-                                          (20, 64, 1, 1, 1, None), (21, 32, 2, 2, 16, None)]:
-        N = 2 ** n
-        sr, fcen = 6.25e6, 600e6
-        freqs = fcen + sr * (np.arange(C) + 0.5 - C / 2)
-        g = torch.Generator(device="cuda")
-        g.manual_seed(n + C)
-        x = torch.randn((N, C, P, 2), device="cuda", dtype=torch.float32, generator=g)
-        monkeypatch.setenv("PBK_LEVELS", f"{n - 14},8,6")
-        outs, descs = [], []
-        for pipe in ("0", "1"):
-            monkeypatch.setenv("PBK_L2PIPE", pipe)
-            plan = L.DedispPlan(nsamp=N, nchan=C, npol=P, dm=3.0, sample_rate_hz=sr,
-                                ref_freq_hz=fcen, chan_freq_hz=freqs, crop=crop or (0, N),
-                                out_kind=out_kind, downsample=ds)
-            nout = plan.out_rows * plan.row_elems * plan.elem_bytes
-            out = torch.zeros(nout, device="cuda", dtype=torch.uint8)
-            for _ in range(2):
-                plan.exec_device(x.data_ptr(), out.data_ptr(), None,
-                                 torch.cuda.current_stream().cuda_stream)
-            torch.cuda.synchronize()
-            outs.append(out.clone())
-            descs.append(plan.describe())
-            plan.destroy()
-        assert "l2pipe" in descs[1] and "l2pipe" not in descs[0], descs
-        assert torch.equal(outs[0], outs[1]), descs[1]
