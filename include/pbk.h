@@ -389,6 +389,37 @@ int pbk_boxcar_search(const void* in, int64_t nser, int64_t rows, int64_t ncols,
                       int32_t stats_given, void* snr, void* start, void* width, int32_t on_device,
                       int32_t device, void* stream);
 
+/* Spectral kurtosis RFI flagging (builder-defined; Nita & Gary 2010): in (nsamp, nchan, npol) of
+ * in_dtype PBK_C64, PBK_I8X2 or PBK_F32 (detected power, a filterbank), C-contiguous; column
+ * (c, p) is one series.  Per block b of the m rows [b m, (b+1) m), nblk = floor(nsamp / m), and
+ * per column, with p = re^2 + im^2 (voltages) or p = x (float32), widened to float64:
+ *   S1 = sum p, S2 = sum p^2 -- int64 for int8 input (exact), float64 in a fixed order otherwise;
+ *   SK = F (m S2 / (S1 S1) - 1) in float64 in exactly this order without contraction,
+ *       F = (m nd + 1) / (m - 1), NaN when S1 == 0 (an all-zero block);
+ *   sk[b, c, p] = (float)SK, float32 (nblk, nchan, npol);
+ *   mask[b, c] = 1 when the SK of any p is not inside [lo, hi] (NaN is flagged), uint8 (nblk, nchan).
+ * nd is the number of raw voltage powers summed into each value of in: 1 for voltages, e.g. 2 for
+ * Stokes I or downsample * freq_sum for pbk_detect output.  The int8 route is bit for bit the
+ * float64 definition; no atomics, so every execution is bit for bit reproducible.
+ * out: NULL (estimate only), == in (the m x npol elements of every flagged cell are set to zero in
+ * place and nothing else is written), or a separate array of in's type and shape (a copy of in with
+ * the flagged cells zeroed; the estimate pass writes the copy as it reads).  The tail rows
+ * nblk m .. nsamp - 1 are never estimated, flagged or zeroed; they are copied when out != in.
+ * A zero is 0 + 0i, (0, 0) or 0.0f.  sk and mask may each be NULL.
+ * u4 / u2 input returns PBK_ERR_UNSUPPORTED: a 2-bit code has no zero, and a u4 zero is code 8,
+ * so zeroing would need a decoded output.  m < 2, nd not finite or <= 0, lo or hi NaN, lo > hi,
+ * nchan or npol < 1, nsamp < 0, a NULL in when nsamp > 0, all three outputs NULL, another in_dtype,
+ * and device arrays not aligned to their element size (8, 2 or 4 bytes for in and out, 4 for sk)
+ * return PBK_ERR_INVALID.  Element offsets are 64-bit; nchan * npol above INT32_MAX, and more than
+ * INT32_MAX CTAs in either launch (nblk * splits * ceil(nchan npol / 32) or nblk * nchan / 256)
+ * return PBK_ERR_UNSUPPORTED.  nblk == 0 estimates nothing and copies in to a separate out.
+ * on_device = 1 only enqueues on `stream` (the partial sums are a stream-ordered allocation, the
+ * tail a device-to-device copy) and can be captured into a graph; 0 copies in, runs, copies out
+ * and synchronises. */
+int pbk_spectral_kurtosis(const void* in, void* out, int64_t nsamp, int64_t nchan, int64_t npol,
+                          int32_t in_dtype, int64_t m, double nd, double lo, double hi, void* sk,
+                          void* mask, int32_t on_device, int32_t device, void* stream);
+
 /* ---- polarisation -------------------------------------------------------------------------
  * pbk_stokes:    (A, B) complex64 pol pairs -> [I, Q, U, V] float32 (core.py:930-966; basis
  *                linear when circular == 0).  npairs = nsamp * nchan.

@@ -30,6 +30,7 @@
 #include "pbk_misc.cuh"
 #include "pbk_incoh.cuh"
 #include "pbk_search.cuh"
+#include "pbk_sk.cuh"
 
 using namespace pbk;
 
@@ -2822,6 +2823,125 @@ extern "C" int pbk_boxcar_search(const void* in, int64_t nser, int64_t rows, int
     CUDA_TRY(device_to_host(start, d_start, ob, st));
     CUDA_TRY(device_to_host(width, d_width, ob, st));
     if (!stats_given) CUDA_TRY(device_to_host(stats, d_stats, sb, st));
+  }
+  return PBK_OK;
+}
+
+// ------------------------------------------------------------------------------------------
+// spectral kurtosis: per-block estimate, flags and zeroing of flagged cells (pbk_sk.cuh)
+// ------------------------------------------------------------------------------------------
+extern "C" int pbk_spectral_kurtosis(const void* in, void* out, int64_t nsamp, int64_t nchan,
+                                     int64_t npol, int32_t in_dtype, int64_t m, double nd,
+                                     double lo, double hi, void* sk, void* mask, int32_t on_device,
+                                     int32_t device, void* stream) {
+  namespace pk = pbk_sk;
+  if (in_dtype == PBK_U4X2 || in_dtype == PBK_U2X2)
+    return fail(PBK_ERR_UNSUPPORTED, "spectral kurtosis of u4 / u2 input: a zeroed sample has no code");
+  if (in_dtype != PBK_C64 && in_dtype != PBK_I8X2 && in_dtype != PBK_F32)
+    return fail(PBK_ERR_INVALID, "in_dtype must be PBK_C64, PBK_I8X2 or PBK_F32");
+  if (m < 2) return fail(PBK_ERR_INVALID, "m = %lld: at least 2 samples per block", (long long)m);
+  if (!std::isfinite(nd) || nd <= 0.0) return fail(PBK_ERR_INVALID, "nd must be finite and > 0");
+  if (std::isnan(lo) || std::isnan(hi) || lo > hi)
+    return fail(PBK_ERR_INVALID, "thresholds must satisfy lo <= hi");
+  if (nchan < 1 || npol < 1 || nsamp < 0)
+    return fail(PBK_ERR_INVALID, "bad shape (nchan and npol must be >= 1, nsamp >= 0)");
+  if (!out && !sk && !mask) return fail(PBK_ERR_INVALID, "no output: out, sk and mask are NULL");
+  if (nsamp > 0 && !in) return fail(PBK_ERR_INVALID, "in is NULL");
+  const int esize = in_dtype == PBK_C64 ? 8 : in_dtype == PBK_I8X2 ? 2 : 4;
+  if (on_device && ((((uintptr_t)in | (uintptr_t)out) & (esize - 1)) || ((uintptr_t)sk & 3)))
+    return fail(PBK_ERR_INVALID, "device arrays must be aligned to their element size");
+  if (nchan > INT_MAX || npol > INT_MAX || nchan * npol > INT_MAX)
+    return fail(PBK_ERR_UNSUPPORTED, "nchan * npol must be at most INT32_MAX");
+  const long long W = nchan * npol;
+  if (nsamp > LLONG_MAX / 8 / W) return fail(PBK_ERR_UNSUPPORTED, "input too large");
+  const long long nblk = nsamp / m;
+  const size_t rowb = (size_t)W * esize, ib = (size_t)nsamp * rowb;
+  const bool copy = out && out != in;
+  if (nblk == 0) {   // nothing to estimate: a separate output is a copy of the input
+    if (copy && ib) {
+      if (!on_device) {
+        std::memcpy(out, in, ib);
+        return PBK_OK;
+      }
+      CUDA_TRY(cudaSetDevice(device));
+      CUDA_TRY(cudaMemcpyAsync(out, in, ib, cudaMemcpyDeviceToDevice,
+                               reinterpret_cast<cudaStream_t>(stream)));
+    }
+    return PBK_OK;
+  }
+  // the estimate grid: (block, split, column group).  The lanes, the splits and so the order of
+  // every sum follow from the shape alone; arrays aligned to vw elements only take wider loads.
+  const int vw = pk::vector_width(esize);
+  const long long vn = W % vw == 0 ? vw : 1;
+  const int CW = pk::columns_per_cta(W / vn);
+  const long long tpc = pk::kThreads / CW, ngn = (W / vn + CW - 1) / CW;
+  const long long want = (pk::kTargetCtas + nblk * ngn - 1) / (nblk * ngn);
+  const long long most = std::max<long long>(1, m / (tpc * pk::kMinRowsPerLane));
+  long long nsplit = std::max<long long>(1, std::min(want, most));
+  const long long chunk = (m + nsplit - 1) / nsplit;
+  nsplit = (m + chunk - 1) / chunk;
+  const long long ncells = nblk * nchan, fgrid = (ncells + pk::kThreads - 1) / pk::kThreads;
+  if (nblk * nsplit * ((W + CW - 1) / CW) > INT_MAX || fgrid > INT_MAX)
+    return fail(PBK_ERR_UNSUPPORTED, "too many blocks for one launch");
+
+  CUDA_TRY(cudaSetDevice(device));
+  cudaStream_t st = on_device ? reinterpret_cast<cudaStream_t>(stream) : cudaStreamPerThread;
+  const size_t skb = (size_t)ncells * npol * 4, mb = (size_t)ncells;
+  DevBuf di, dsk, dm;
+  const void* x = in;
+  void* d_sk = sk;
+  void* d_mask = mask;
+  void* zap = out;          // the array whose flagged cells are zeroed
+  void* cp = copy ? out : nullptr;
+  if (!on_device) {
+    // host route: zero in place in a device copy of the input, then copy the whole array out
+    CUDA_TRY(cudaMalloc(&di.p, ib));
+    CUDA_TRY(host_to_device(di.p, in, ib, st));
+    if (sk) CUDA_TRY(cudaMalloc(&dsk.p, skb));
+    if (mask) CUDA_TRY(cudaMalloc(&dm.p, mb));
+    x = di.p, d_sk = dsk.p, d_mask = dm.p;
+    zap = out ? di.p : nullptr;
+    cp = nullptr;
+  } else if (copy && (size_t)nsamp > (size_t)nblk * m) {   // the tail rows are never estimated
+    const size_t off = (size_t)nblk * m * rowb;
+    CUDA_TRY(cudaMemcpyAsync(static_cast<char*>(out) + off, static_cast<const char*>(in) + off,
+                             ib - off, cudaMemcpyDeviceToDevice, st));
+  }
+  const bool vec = vn > 1 && (((uintptr_t)x | (uintptr_t)zap | (uintptr_t)cp) % (vw * esize)) == 0;
+  const long long ngroups = vec ? ngn : (W + CW - 1) / CW;
+  const unsigned pgrid = (unsigned)(nblk * nsplit * ngroups);
+  // the partial sums and the flags live in a stream-ordered allocation
+  const size_t partb = (size_t)nblk * nsplit * W * 16;
+  void* part = nullptr;
+  CUDA_TRY(cudaMallocAsync(&part, partb + (size_t)ncells, st));
+  unsigned char* flags = static_cast<unsigned char*>(part) + partb;
+  pk::PartArgs pa{};
+  pa.in = x, pa.out = cp, pa.part = part, pa.flags = flags;
+  pa.W = W, pa.m = m, pa.chunk = chunk, pa.nchan = nchan, pa.npol = npol;
+  pa.nsplit = (int)nsplit, pa.ngroups = (int)ngroups;
+  pk::FinArgs fa{};
+  fa.part = part;
+  fa.sk = reinterpret_cast<float*>(d_sk);
+  fa.mask = reinterpret_cast<unsigned char*>(d_mask);
+  fa.flags = flags;
+  fa.ncells = ncells, fa.nchan = nchan, fa.npol = npol, fa.W = W;
+  fa.nsplit = (int)nsplit;
+  fa.mf = (double)m;
+  fa.f = ((double)m * nd + 1.0) / ((double)m - 1.0);
+  fa.lo = lo, fa.hi = hi;
+  cudaError_t e = pk::launch_pass(esize, false, vec, CW, pa, pgrid, st);
+  if (e == cudaSuccess) e = pk::launch_finalize(esize, fa, (unsigned)fgrid, st);
+  if (e == cudaSuccess && zap) {
+    pa.out = zap;
+    e = pk::launch_pass(esize, true, vec, CW, pa, pgrid, st);
+  }
+  cudaError_t ef = cudaFreeAsync(part, st);
+  if (e != cudaSuccess) return fail(PBK_ERR_CUDA, "spectral kurtosis launch: %s", cudaGetErrorString(e));
+  CUDA_TRY(ef);
+  if (!on_device) {
+    if (sk) CUDA_TRY(device_to_host(sk, d_sk, skb, st));
+    if (mask) CUDA_TRY(device_to_host(mask, d_mask, mb, st));
+    if (out) CUDA_TRY(device_to_host(out, di.p, ib, st));
   }
   return PBK_OK;
 }

@@ -24,7 +24,8 @@ from .device import DeviceArray
 
 __all__ = ["default_device", "dedisperse", "chirp", "detect", "shift_channels", "phase_ramp", "mix", "analytic_decimate", "stokes", "pol_basis",
            "downsample", "fft", "stft", "istft", "stft_detect", "stft_fold", "fold",
-           "dedisperse_fold", "dedisperse_trials", "incoherent_trials", "boxcar_search", "predict_phase",
+           "dedisperse_fold", "dedisperse_trials", "incoherent_trials", "boxcar_search", "spectral_kurtosis",
+           "predict_phase",
            "clear_plan_cache",
            "pinned_results"]
 
@@ -772,6 +773,90 @@ def boxcar_search(data, widths, window, stats=None, device=None):
                                       int(given), L.ptr(snr), L.ptr(start), L.ptr(width), 0, dev,
                                       None))
     return snr, start, width, st
+
+
+_SK_DTYPES = {np.dtype(np.complex64): L.PBK_C64, np.dtype(np.float32): L.PBK_F32}
+_SK_ZAP = (None, "copy", "inplace")
+
+
+def spectral_kurtosis(data, m, *, lo, hi, nd=1.0, zap=None, raw=None, device=None):
+    """Spectral kurtosis per block of ``m`` samples of every column, and the zeroing of flagged
+    (block, channel) cells (pbk_spectral_kurtosis).
+
+    ``data`` is (nsamp, nchan, ...) complex64 voltages or float32 detected power, or with
+    ``raw="int8"`` (nsamp, nchan, ..., 2) int8 (re, im) pairs; numpy or DeviceArray.  Per block
+    ``b`` of rows ``[b m, (b+1) m)`` and column, ``SK = F (m S2 / S1^2 - 1)`` with
+    ``F = (m nd + 1) / (m - 1)`` and S1, S2 the sums of the power and its square (NaN for an
+    all-zero block); cell (b, c) is flagged when the SK of any trailing index is outside
+    ``[lo, hi]``.  ``zap``: None (estimate only), "copy" (a copy with flagged cells zeroed) or
+    "inplace" (flagged cells of ``data`` are zeroed and nothing else is written; ``data`` must be
+    C-contiguous).  Tail rows past ``nblk m`` are never flagged.
+
+    Returns ``(sk, mask, out)`` on the side of the bus of ``data``: (nblk, nchan, ...) float32,
+    (nblk, nchan) uint8 (1 = flagged) and the zapped array (``data`` itself for "inplace", None
+    without zapping).  complex128 is refused rather than narrowed."""
+    if zap not in _SK_ZAP:
+        raise ValueError(f"zap must be one of {_SK_ZAP}, got {zap!r}")
+    if raw is not None and raw != "int8":
+        raise ValueError(f'raw must be None or "int8", got {raw!r}')
+    from . import _dask
+    if _dask.is_dask(data):
+        raise TypeError("spectral_kurtosis takes numpy or DeviceArray data, not dask")
+    shape = tuple(data.shape)
+    dt = np.dtype(data.dtype)
+    if raw == "int8":
+        if dt != np.int8 or len(shape) < 3 or shape[-1] != 2:
+            raise TypeError("raw='int8' takes (nsamp, nchan, ..., 2) int8 data")
+        body, in_dtype = shape[:-1], L.PBK_I8X2
+    else:
+        if dt not in _SK_DTYPES:
+            raise TypeError(f"spectral_kurtosis takes complex64, float32 or raw int8 data, got {dt}")
+        body, in_dtype = shape, _SK_DTYPES[dt]
+    if len(body) < 2:
+        raise ValueError("spectral_kurtosis takes (nsamp, nchan, ...) data")
+    m = int(m)
+    if m < 2:
+        raise ValueError(f"m = {m}: at least 2 samples per block")
+    if not float(lo) <= float(hi):
+        raise ValueError(f"thresholds must satisfy lo <= hi, got ({lo}, {hi})")
+    nsamp, nchan = body[0], body[1]
+    trailing = body[2:]
+    npol = int(np.prod(trailing, dtype=np.int64)) if trailing else 1
+    nblk = nsamp // m
+    sk_shape, mask_shape = (nblk, nchan) + trailing, (nblk, nchan)
+    args = (nsamp, nchan, npol, in_dtype, m, float(nd), float(lo), float(hi))
+    if _is_dev(data):
+        if zap == "inplace":
+            if not data.tensor.is_contiguous():
+                raise ValueError("zap='inplace' needs a C-contiguous array")
+            x = data
+        else:
+            x = data.contiguous()
+        dev = x.device
+        sk = DeviceArray.empty(sk_shape, np.float32, dev)
+        mask = DeviceArray.empty(mask_shape, np.uint8, dev)
+        out = x if zap == "inplace" else (DeviceArray.empty(shape, dt, dev) if zap else None)
+        if nblk or (zap == "copy" and nsamp):   # an empty tensor may have a NULL pointer
+            L.check(L.lib().pbk_spectral_kurtosis(
+                L.ptr(x.ptr), None if out is None else L.ptr(out.ptr), *args,
+                L.ptr(sk.ptr) if nblk else None, L.ptr(mask.ptr) if nblk else None, 1, dev,
+                ctypes.c_void_p(_stream())))
+        return sk, mask, out
+    if zap == "inplace":
+        if not (isinstance(data, np.ndarray) and data.flags.c_contiguous and data.flags.writeable):
+            raise ValueError("zap='inplace' needs a writeable C-contiguous numpy array")
+        x = data
+    else:
+        x = np.ascontiguousarray(data)
+    dev = default_device() if device is None else device
+    sk = _result(sk_shape, np.float32)
+    mask = _result(mask_shape, np.uint8)
+    out = x if zap == "inplace" else (_result(shape, dt) if zap else None)
+    if nblk or (zap == "copy" and nsamp):
+        L.check(L.lib().pbk_spectral_kurtosis(L.ptr(x), None if out is None else L.ptr(out), *args,
+                                              L.ptr(sk) if nblk else None,
+                                              L.ptr(mask) if nblk else None, 0, dev, None))
+    return sk, mask, out
 
 
 def phase_ramp(data, shift_samples=None, zero_lo=None, zero_hi=None, device=None):
