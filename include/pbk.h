@@ -363,6 +363,37 @@ int pbk_incoh_trials_plan_create(int64_t nsamp_in, int64_t nchan, int64_t npol, 
 int pbk_incoh_trials_exec_device(pbk_plan* plan, const void* d_in, void* d_out, void* stream);
 int pbk_incoh_trials_exec_host(pbk_plan* plan, const void* in, void* out);
 
+/* Fast dispersion measure transform (FDMT; builder-defined, DESIGN.md 5.4h, numpy statement in
+ * tests/fdmt_oracle.py): every integer delay trial d in [d_min, max_delay] of a (nsamp, nchan,
+ * npol) float32 filterbank with ascending channels over [f_lo_hz, f_hi_hz), in about
+ * ceil(log2 nchan) passes.  Trial d sums exactly d + nchan samples per column along a track of
+ * d samples of sweep from f_hi to f_lo; out is a contiguous (ndm, rows, npol) float32 array with
+ * ndm = max_delay - d_min + 1, and out[k, j, :] is trial d_min + k arriving at ref_freq_hz
+ * t_lo + j samples after the input starts (pbk_fdmt_plan_geometry).  Every output is a fixed
+ * tree of float32 adds: executions are bit for bit reproducible, integer-valued input sums
+ * exactly, and a chunked plan equals an unchunked one.
+ * The plan builds the tree and its index tables once in float64 (uploaded, counted in
+ * pbk_plan_info's workspace bytes with the two state buffers).  The state is about
+ * (max_delay + nchan) * nsamp * npol floats per level; when two levels exceed
+ * max_workspace_bytes (0: a fifth of the device's memory) the output rows are split into chunks,
+ * each an independent transform of its input slice.  pbk_plan_describe shows
+ * "FDMT:C=..:P=..:D=..:levels=..:fused=k:T=..:smem=..:chunks=..:rows=..", where k merges run
+ * inside the first kernel (PBK_FDMT_FUSED=k forces it).
+ * nsamp, nchan or npol < 1, f_lo_hz <= 0, f_hi_hz <= f_lo_hz, ref_freq_hz <= 0, max_delay < 0,
+ * d_min < 0 or > max_delay, and a NULL pointer return PBK_ERR_INVALID; nsamp, nchan, npol or
+ * nsamp + max_delay beyond INT32_MAX, state rows beyond 32-bit indices and a workspace cap that
+ * holds no chunk return PBK_ERR_UNSUPPORTED.  rows == 0 (nsamp too short for the sweep) is a valid
+ * plan whose executions are no-ops, as for pbk_incoh_trials.
+ * Execution: device pointers need 4-byte alignment (PBK_ERR_INVALID otherwise); _exec_device only
+ * enqueues kernels on `stream` (no synchronisation, no atomics) and can be captured into a graph;
+ * _exec_host copies in, runs, copies out and synchronises.  The input is never written. */
+int pbk_fdmt_plan_create(int64_t nsamp, int64_t nchan, int64_t npol, double f_lo_hz,
+                         double f_hi_hz, double ref_freq_hz, int64_t max_delay, int64_t d_min,
+                         int64_t max_workspace_bytes, int32_t device, pbk_plan** plan);
+int pbk_fdmt_plan_geometry(const pbk_plan* plan, int32_t* ndm, int64_t* rows, int64_t* t_lo);
+int pbk_fdmt_exec_device(pbk_plan* plan, const void* d_in, void* d_out, void* stream);
+int pbk_fdmt_exec_host(pbk_plan* plan, const void* in, void* out);
+
 /* Single-pulse search of a stack of time series (builder-defined): x (nser, rows, ncols) float32,
  * C-contiguous, series (s, c) = x[s, :, c] -- e.g. the (ndm, rows, 1[*P]) plane of
  * pbk_incoh_trials_* or the (ndm, rows, nchan[*P]) output of a trial plan.

@@ -20,6 +20,7 @@ EXPORTS = [
     "pbk_dedisp_exec_device", "pbk_dedisp_fold_exec_device", "pbk_dedisp_trials_plan_create",
     "pbk_plan_trials", "pbk_dedisp_exec_blocks_device", "pbk_plan_blocks_per_launch",
     "pbk_incoh_trials_plan_create", "pbk_incoh_trials_exec_device", "pbk_incoh_trials_exec_host",
+    "pbk_fdmt_plan_create", "pbk_fdmt_plan_geometry", "pbk_fdmt_exec_device", "pbk_fdmt_exec_host",
     "pbk_boxcar_search", "pbk_spectral_kurtosis",
     "pbk_fft_plan_create", "pbk_stft_plan_create", "pbk_stft_plan_create_raw",
     "pbk_stft_detect_plan_create", "pbk_stft_fold_exec_device",
@@ -94,6 +95,13 @@ def lib():
                                                    i32, ctypes.POINTER(vp)]
         L.pbk_incoh_trials_exec_device.argtypes = [vp, vp, vp, vp]
         L.pbk_incoh_trials_exec_host.argtypes = [vp, vp, vp]
+        L.pbk_fdmt_plan_create.argtypes = [i64, i64, i64, ctypes.c_double, ctypes.c_double,
+                                           ctypes.c_double, i64, i64, i64, i32,
+                                           ctypes.POINTER(vp)]
+        L.pbk_fdmt_plan_geometry.argtypes = [vp, ctypes.POINTER(i32), ctypes.POINTER(i64),
+                                             ctypes.POINTER(i64)]
+        L.pbk_fdmt_exec_device.argtypes = [vp, vp, vp, vp]
+        L.pbk_fdmt_exec_host.argtypes = [vp, vp, vp]
         L.pbk_dedisp_out_shape.argtypes = [vp] + [ctypes.POINTER(i64)] * 3
         L.pbk_dedisp_exec_host.argtypes = [vp, vp, vp, vp]
         L.pbk_dedisp_exec_device.argtypes = [vp, vp, vp, vp, vp]
@@ -367,6 +375,38 @@ class IncohTrialsPlan(Plan):
         n = ctypes.c_int32(0)
         check(lib().pbk_plan_blocks_per_launch(self.handle, ctypes.byref(n)))
         return n.value
+
+
+class FdmtPlan(Plan):
+    """Fast dispersion measure transform (pbk_fdmt_plan_create): every delay trial
+    ``d_min..max_delay`` of (nsamp, nchan, npol) float32 input as a contiguous (ndm, rows, npol)
+    float32 plane whose row j arrives at ``ref_freq_hz`` ``t_lo + j`` samples after the input
+    starts."""
+
+    def __init__(self, *, nsamp, nchan, npol, f_lo_hz, f_hi_hz, ref_freq_hz, max_delay, d_min=0,
+                 max_workspace_bytes=0, device=0):
+        h = ctypes.c_void_p(0)
+        check(lib().pbk_fdmt_plan_create(
+            int(nsamp), int(nchan), int(npol), float(f_lo_hz), float(f_hi_hz), float(ref_freq_hz),
+            int(max_delay), int(d_min), int(max_workspace_bytes), int(device), ctypes.byref(h)))
+        super().__init__(h)
+        self.nsamp, self.nchan, self.npol = int(nsamp), int(nchan), int(npol)
+        self.device = device
+        ndm, rows, t_lo = ctypes.c_int32(0), ctypes.c_int64(0), ctypes.c_int64(0)
+        check(lib().pbk_fdmt_plan_geometry(self.handle, ctypes.byref(ndm), ctypes.byref(rows),
+                                           ctypes.byref(t_lo)))
+        self.ndm, self.rows, self.t_lo = ndm.value, rows.value, t_lo.value
+
+    def out_array(self):
+        return np.empty((self.ndm, self.rows, self.npol), dtype=np.float32)
+
+    def exec_host(self, x, out):
+        check(lib().pbk_fdmt_exec_host(self.handle, ptr(x), ptr(out)))
+        return out
+
+    def exec_device(self, d_in, d_out, stream=0):
+        check(lib().pbk_fdmt_exec_device(self.handle, ptr(d_in), ptr(d_out),
+                                         ctypes.c_void_p(stream)))
 
 
 class RampPlan(Plan):

@@ -31,6 +31,7 @@
 #include "pbk_incoh.cuh"
 #include "pbk_search.cuh"
 #include "pbk_sk.cuh"
+#include "pbk_fdmt.cuh"
 
 using namespace pbk;
 
@@ -93,7 +94,7 @@ extern "C" int pbk_device_mem_info(int device, size_t* free_bytes, size_t* total
 // plan
 // ------------------------------------------------------------------------------------------
 enum Role { ROLE_USER_IN = 0, ROLE_SCRATCH = 1, ROLE_USER_OUT = 2, ROLE_TMPF = 3 };
-enum PlanKind { PLAN_DEDISP = 0, PLAN_FFT = 1, PLAN_INCOH = 2 };
+enum PlanKind { PLAN_DEDISP = 0, PLAN_FFT = 1, PLAN_INCOH = 2, PLAN_FDMT = 3 };
 
 struct Pass {
   int mode = MODE_FWD;
@@ -190,6 +191,8 @@ struct pbk_plan {
   size_t incoh_smem = 0;
   int* d_incoh = nullptr;       // perm, off, lo and ext tables
   size_t incoh_bytes = 0;
+  // FDMT plans (pbk_fdmt_plan_create)
+  struct FdmtPlan* fdmt = nullptr;
 };
 
 static void prof_mark(pbk_plan* pl, int idx, cudaStream_t st) {
@@ -2251,6 +2254,11 @@ extern "C" int pbk_plan_profile_read(pbk_plan* pl, int32_t slot, float* ms, int3
   return PBK_OK;
 }
 
+struct FdmtPlan;
+static void fdmt_destroy(FdmtPlan* f);
+static size_t fdmt_bytes(const FdmtPlan* f);
+static int fdmt_describe(const FdmtPlan* f, char* buf, size_t n);
+
 extern "C" void pbk_plan_destroy(pbk_plan* pl) {
   if (!pl) return;
   cudaSetDevice(pl->device);
@@ -2271,6 +2279,7 @@ extern "C" void pbk_plan_destroy(pbk_plan* pl) {
   cudaFree(pl->d_foldbuf);
   cudaFree(pl->d_stage);
   cudaFree(pl->d_incoh);
+  fdmt_destroy(pl->fdmt);
   cudaFree(pl->h_din);
   cudaFree(pl->h_dout);
   cudaFree(pl->h_dchirp);
@@ -2286,7 +2295,7 @@ extern "C" int pbk_plan_info(const pbk_plan* pl, int32_t* launches, int64_t* wor
                 (pl->work_bytes > pl->scratch_bytes ? pl->work_bytes - pl->scratch_bytes : 0) +
                 pl->blk_bytes * ((pl->blk_scratch[0] ? 1 : 0) + (pl->blk_scratch[1] ? 1 : 0)) +
                 pl->tmpf_bytes + pl->fold_bytes +
-                pl->stage_bytes + pl->incoh_bytes);
+                pl->stage_bytes + pl->incoh_bytes + fdmt_bytes(pl->fdmt));
   if (levels) *levels = pl->nlevels;
   if (level_log2)
     for (int i = 0; i < 3; ++i) level_log2[i] = pl->level_log2[i];
@@ -2297,6 +2306,7 @@ extern "C" int pbk_plan_describe(const pbk_plan* pl, char* buf, size_t n) {
   if (!pl || !buf || n == 0) return fail(PBK_ERR_INVALID, "NULL argument");
   size_t off = 0;
   buf[0] = 0;
+  if (pl->kind == PLAN_FDMT) return fdmt_describe(pl->fdmt, buf, n);
   if (pl->kind == PLAN_INCOH) {
     const pbk_incoh::Args& a = pl->incoh;
     snprintf(buf, n, "INCOH:ndm=%d:C=%d:P=%d:rows=%d:KD=%d:TT=%d:CC=%d:smem=%zu:tiles=%u", pl->ndm,
@@ -2501,6 +2511,308 @@ extern "C" int pbk_incoh_trials_exec_host(pbk_plan* pl, const void* in, void* ou
   cudaStream_t st = cudaStreamPerThread;
   CUDA_TRY(host_to_device(pl->h_din, in, pl->in_bytes, st));
   if ((rc = pbk_incoh_trials_exec_device(pl, pl->h_din, pl->h_dout, st)) != PBK_OK) return rc;
+  CUDA_TRY(device_to_host(out, pl->h_dout, pl->out_bytes, st));
+  return PBK_OK;
+}
+
+// ------------------------------------------------------------------------------------------
+// fast dispersion measure transform (pbk_fdmt.cuh, tables from pbk_fdmt_tables.cu)
+// ------------------------------------------------------------------------------------------
+// Shared memory of one fused CTA is at most this much, so that two CTAs fit an SM.
+static constexpr size_t kFdmtSmemCap = 100 * 1024;
+
+struct FdmtPlan {
+  pbk_fdmt::Tables t;
+  long long nsamp = 0, D = 0, d_min = 0;
+  int C = 0, P = 0, k = 0, T = 0;
+  size_t smem = 0;
+  int bufB_floats = 0;
+  long long J = 0;              // output rows per chunk
+  int nchunks = 0;
+  long long stride = 0;         // floats per state row
+  size_t buf_bytes = 0;         // each state buffer
+  float* buf[2] = {nullptr, nullptr};
+  int* d_tab = nullptr;         // row0, row0_off, nnodes, ent_off, then int4 entries and last
+  size_t tab_bytes = 0;
+  std::vector<long long> ent_off;   // per level, in int4 entries
+  long long last_off = 0;
+  int row0_off_at = 0, nnodes_at = 0, ent_off_at = 0, ent_at = 0;   // int offsets in d_tab
+};
+
+static void fdmt_destroy(FdmtPlan* f) {
+  if (!f) return;
+  cudaFree(f->buf[0]);
+  cudaFree(f->buf[1]);
+  cudaFree(f->d_tab);
+  delete f;
+}
+
+static size_t fdmt_bytes(const FdmtPlan* f) {
+  return f ? f->tab_bytes + f->buf_bytes * ((f->buf[0] ? 1 : 0) + (f->buf[1] ? 1 : 0)) : 0;
+}
+
+static int fdmt_describe(const FdmtPlan* f, char* buf, size_t n) {
+  snprintf(buf, n, "FDMT:C=%d:P=%d:D=%lld:levels=%d:fused=%d:T=%d:smem=%zu:chunks=%d:rows=%lld",
+           f->C, f->P, f->D, f->t.L, f->k, f->T, f->smem, f->nchunks, f->t.rows);
+  return PBK_OK;
+}
+
+// Shared floats of the fused kernel at fusion depth k and tile T over every level-k node, and the
+// offset of its second buffer; 0 when some node's subtree cannot be held.
+static size_t fdmt_fused_smem(const pbk_fdmt::Tables& t, int k, int T, int P, int* bufB) {
+  if (k == 0) { *bufB = 0; return 0; }
+  long long a_max = 0, b_max = 0;
+  for (int n = 0; n < t.nnodes[k]; ++n) {
+    const long long H = t.row0[k][n + 1] - t.row0[k][n] - 1, WT = T + H;
+    long long rm = 0;
+    for (int l = 0; l <= k; ++l) {
+      const int s = k - l;
+      rm = std::max<long long>(rm, t.row0[l][std::min((n + 1) << s, t.nnodes[l])] - t.row0[l][n << s]);
+    }
+    const int ca = n << k, cb = std::min((n + 1) << k, t.C);
+    long long nl = 1;
+    for (int c = ca; c < cb; ++c) nl = std::max<long long>(nl, t.row0[0][c + 1] - t.row0[0][c]);
+    a_max = std::max(a_max, rm * WT * P);
+    b_max = std::max(b_max, std::max(rm * WT * P, (WT + nl - 1) * (cb - ca) * P));
+    if (a_max + b_max > (long long)(kFdmtSmemCap / sizeof(float))) return 0;
+  }
+  a_max = (a_max + 3) & ~3LL;
+  *bufB = (int)a_max;
+  return (size_t)(a_max + b_max) * sizeof(float);
+}
+
+// Largest tile (a multiple of 32, at most 2048 times) that fits at depth k; 0 if none.
+static int fdmt_tile(const pbk_fdmt::Tables& t, int k, int P, long long wlen) {
+  if (k == 0) return 1024;
+  int best = 0, b;
+  for (int T = 32; T <= 2048 && T < wlen + 32; T += 32)
+    if (fdmt_fused_smem(t, k, T, P, &b)) best = T; else break;
+  return best;
+}
+
+extern "C" int pbk_fdmt_plan_create(int64_t nsamp, int64_t nchan, int64_t npol, double f_lo_hz,
+                                    double f_hi_hz, double ref_freq_hz, int64_t max_delay,
+                                    int64_t d_min, int64_t max_workspace_bytes, int32_t device,
+                                    pbk_plan** out) {
+  if (!out) return fail(PBK_ERR_INVALID, "NULL pointer");
+  *out = nullptr;
+  if (nsamp < 1 || nchan < 1 || npol < 1)
+    return fail(PBK_ERR_INVALID, "bad shape (nsamp, nchan and npol must be >= 1)");
+  if (!(f_lo_hz > 0) || !(f_hi_hz > f_lo_hz) || !std::isfinite(f_hi_hz))
+    return fail(PBK_ERR_INVALID, "need 0 < f_lo < f_hi");
+  if (!(ref_freq_hz > 0) || !std::isfinite(ref_freq_hz))
+    return fail(PBK_ERR_INVALID, "ref_freq must be positive and finite");
+  if (max_delay < 0 || d_min < 0 || d_min > max_delay)
+    return fail(PBK_ERR_INVALID, "need 0 <= d_min <= max_delay");
+  if (max_workspace_bytes < 0) return fail(PBK_ERR_INVALID, "negative workspace cap");
+  if (nsamp > INT_MAX || nchan > INT_MAX || npol > INT_MAX || max_delay >= INT_MAX - nsamp)
+    return fail(PBK_ERR_UNSUPPORTED, "nsamp, nchan, npol and nsamp + max_delay must fit 32-bit indices");
+  CUDA_TRY(cudaSetDevice(device));    // before anything is allocated: nothing to free on failure
+  FdmtPlan* f = new FdmtPlan();
+  auto drop = [&](int code) { fdmt_destroy(f); return code; };
+  const int C = (int)nchan, P = (int)npol;
+  if (pbk_fdmt::build_tables(nsamp, C, f_lo_hz, f_hi_hz, ref_freq_hz, max_delay, d_min, &f->t))
+    return drop(fail(PBK_ERR_UNSUPPORTED, "state rows or shifts beyond 32-bit indices"));
+  const pbk_fdmt::Tables& t = f->t;
+  f->nsamp = nsamp, f->D = max_delay, f->d_min = d_min, f->C = C, f->P = P;
+  const long long ndm = max_delay - d_min + 1, rows = t.rows;
+  // rows of the largest state level the passes keep (levels k .. max(L - 1, 0))
+  const int kmax = std::max(t.L - 1, 0);
+  auto state_rows = [&](int k) {
+    long long m = 0;
+    for (int l = k; l <= kmax; ++l) m = std::max<long long>(m, t.row0[l].back());
+    return m;
+  };
+  // fusion depth: 0, the leaves alone, which was fastest on every workload measured (DESIGN.md
+  // 5.4h: the shared-memory merges pay a halo of the node's largest row per tile and run two CTAs
+  // per SM); PBK_FDMT_FUSED=k forces k merges in the first kernel (developer knob)
+  const long long spread = (long long)t.s_max - t.s_min;
+  const long long wfull = std::min<long long>(nsamp, rows + spread + max_delay);
+  int k = 0, T = fdmt_tile(t, 0, P, wfull);
+  if (const char* e = getenv("PBK_FDMT_FUSED")) {
+    k = atoi(e);
+    if (k < 0 || k > kmax) return drop(fail(PBK_ERR_INVALID, "PBK_FDMT_FUSED=%d: 0..%d", k, kmax));
+    T = fdmt_tile(t, k, P, wfull);
+    if (!T) return drop(fail(PBK_ERR_UNSUPPORTED, "PBK_FDMT_FUSED=%d does not fit shared memory", k));
+  }
+  f->k = k, f->T = T;
+  f->smem = fdmt_fused_smem(t, k, T, P, &f->bufB_floats);
+  // time chunks: the largest J whose two state levels fit the cap (0: 1/5 of the device)
+  size_t cap = (size_t)max_workspace_bytes;
+  if (cap == 0) {
+    size_t fr = 0, tot = 0;
+    const cudaError_t ce = cudaMemGetInfo(&fr, &tot);
+    if (ce != cudaSuccess)
+      return drop(fail(PBK_ERR_CUDA, "FDMT plan: %s", cudaGetErrorString(ce)));
+    cap = tot / 5;
+  }
+  const int nbuf = t.L - 1 > k ? 2 : 1;
+  const long long srows = state_rows(k);
+  auto bytes_of = [&](long long J) {
+    const long long w = std::min<long long>(nsamp, J + spread + max_delay);
+    const long long stride = (w * P + 3) & ~3LL;
+    return (double)nbuf * srows * stride * sizeof(float);
+  };
+  long long J = std::max(rows, 1LL);
+  if (bytes_of(J) > (double)cap) {
+    long long lo = 0, hi = J;
+    while (hi - lo > 1) {
+      const long long mid = (lo + hi) / 2;
+      if (bytes_of(mid) <= (double)cap) lo = mid; else hi = mid;
+    }
+    J = lo;
+  }
+  if (J < 1) return drop(fail(PBK_ERR_UNSUPPORTED, "workspace cap %zu bytes holds no chunk (%.0f bytes needed)", cap, bytes_of(1)));
+  f->nchunks = rows > 0 ? (int)((rows + J - 1) / J) : 0;
+  f->J = f->nchunks ? (rows + f->nchunks - 1) / f->nchunks : 0;
+  {
+    const long long w = std::min<long long>(nsamp, f->J + spread + max_delay);
+    f->stride = (w * P + 3) & ~3LL;
+    if (w * P > INT_MAX) return drop(fail(PBK_ERR_UNSUPPORTED, "a state row beyond 32-bit indices"));
+  }
+  // tables: int header then int4 entries
+  std::vector<int> hdr;
+  std::vector<int> row0_off(t.L + 1), ent_off_i(t.L + 1, 0);
+  for (int l = 0; l <= t.L; ++l) {
+    row0_off[l] = (int)hdr.size();
+    hdr.insert(hdr.end(), t.row0[l].begin(), t.row0[l].end());
+  }
+  f->row0_off_at = (int)hdr.size();
+  hdr.insert(hdr.end(), row0_off.begin(), row0_off.end());
+  f->nnodes_at = (int)hdr.size();
+  hdr.insert(hdr.end(), t.nnodes.begin(), t.nnodes.end());
+  f->ent_off_at = (int)hdr.size();
+  f->ent_off.assign(t.L + 1, 0);
+  long long ne = 0;
+  for (int l = 1; l <= t.L; ++l) f->ent_off[l] = ne, ne += (long long)t.ent[l].size();
+  f->last_off = ne;
+  if (ne + (long long)t.last.size() > INT_MAX) return drop(fail(PBK_ERR_UNSUPPORTED, "tables beyond 32-bit indices"));
+  for (int l = 0; l <= t.L; ++l) ent_off_i[l] = (int)f->ent_off[l];
+  hdr.insert(hdr.end(), ent_off_i.begin(), ent_off_i.end());
+  while (hdr.size() % 4) hdr.push_back(0);
+  f->ent_at = (int)hdr.size();
+  std::vector<int4> ents;
+  ents.reserve(ne + t.last.size());
+  for (int l = 1; l <= t.L; ++l)
+    for (const pbk_fdmt::Entry& e : t.ent[l]) ents.push_back(make_int4(e.l, e.u, e.h, e.s));
+  for (const pbk_fdmt::Entry& e : t.last) ents.push_back(make_int4(e.l, e.u, e.h, e.s));
+  f->tab_bytes = hdr.size() * sizeof(int) + ents.size() * sizeof(int4);
+  pbk_plan* pl = new pbk_plan();
+  pl->kind = PLAN_FDMT;
+  pl->device = device;
+  pl->ndm = (int)ndm;
+  pl->fdmt = f;
+  auto cleanup = [&](int code) { pbk_plan_destroy(pl); return code; };
+  cudaError_t e = cudaMalloc(&f->d_tab, f->tab_bytes);
+  if (e == cudaSuccess)
+    e = cudaMemcpy(f->d_tab, hdr.data(), hdr.size() * sizeof(int), cudaMemcpyHostToDevice);
+  if (e == cudaSuccess && !ents.empty())
+    e = cudaMemcpy(f->d_tab + f->ent_at, ents.data(), ents.size() * sizeof(int4), cudaMemcpyHostToDevice);
+  if (rows > 0) {
+    f->buf_bytes = (size_t)srows * f->stride * sizeof(float);
+    for (int b = 0; b < nbuf && e == cudaSuccess; ++b) e = cudaMalloc(&f->buf[b], f->buf_bytes);
+  }
+  if (e == cudaSuccess && f->smem)
+    e = cudaFuncSetAttribute(pbk_fdmt::fdmt_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             (int)kFdmtSmemCap);   // the cap, never less: other plans share it
+  if (e != cudaSuccess)
+    return cleanup(fail(e == cudaErrorMemoryAllocation ? PBK_ERR_NOMEM : PBK_ERR_CUDA,
+                        "FDMT plan: %s", cudaGetErrorString(e)));
+  pl->launches = f->nchunks * (1 + std::max(t.L - 1 - k, 0) + 1);
+  pl->in_bytes = (size_t)nsamp * C * P * sizeof(float);
+  pl->out_bytes = (size_t)ndm * rows * P * sizeof(float);
+  *out = pl;
+  return PBK_OK;
+}
+
+extern "C" int pbk_fdmt_plan_geometry(const pbk_plan* pl, int32_t* ndm, int64_t* rows,
+                                      int64_t* t_lo) {
+  if (!pl || pl->kind != PLAN_FDMT) return fail(PBK_ERR_INVALID, "not an FDMT plan");
+  if (!ndm || !rows || !t_lo) return fail(PBK_ERR_INVALID, "NULL argument");
+  *ndm = pl->ndm;
+  *rows = pl->fdmt->t.rows;
+  *t_lo = pl->fdmt->t.t_lo;
+  return PBK_OK;
+}
+
+extern "C" int pbk_fdmt_exec_device(pbk_plan* pl, const void* d_in, void* d_out, void* stream) {
+  if (!pl || pl->kind != PLAN_FDMT) return fail(PBK_ERR_INVALID, "not an FDMT plan");
+  if (!d_in || !d_out) return fail(PBK_ERR_INVALID, "NULL data pointer");
+  if (((uintptr_t)d_in | (uintptr_t)d_out) & 3)
+    return fail(PBK_ERR_INVALID, "float32 arrays must be 4-byte aligned");
+  const FdmtPlan& f = *pl->fdmt;
+  const pbk_fdmt::Tables& t = f.t;
+  if (t.rows == 0) return PBK_OK;
+  CUDA_TRY(cudaSetDevice(pl->device));
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  const int P = f.P, kmax = std::max(t.L - 1, 0);
+  const int4* ents = reinterpret_cast<const int4*>(f.d_tab + f.ent_at);
+  for (int ch = 0; ch < f.nchunks; ++ch) {
+    const long long ja = ch * f.J, jn = std::min(f.J, t.rows - ja);
+    // window: root times [t_lo + ja + s_min - D, t_lo + ja + jn + s_max), clipped at 0
+    const long long ws = std::max(0LL, t.t_lo + ja + t.s_min - f.D);
+    const long long we = t.t_lo + ja + jn + t.s_max;
+    const int wlen = (int)(we - ws);
+    pbk_fdmt::FusedArgs fa{};
+    fa.x = reinterpret_cast<const float*>(d_in);
+    fa.out = f.buf[0];
+    fa.xrow = (long long)f.C * P;
+    fa.ws = ws;
+    fa.stride = f.stride;
+    fa.wlen = wlen;
+    fa.P = P, fa.k = f.k, fa.T = f.T, fa.nnodes = t.nnodes[f.k];
+    fa.row0 = f.d_tab;
+    fa.row0_off = f.d_tab + f.row0_off_at;
+    fa.nnodes_l = f.d_tab + f.nnodes_at;
+    fa.ent = ents;
+    fa.ent_off = f.d_tab + f.ent_off_at;
+    fa.bufB_floats = f.bufB_floats;
+    const long long ntiles = (wlen + f.T - 1) / f.T;
+    pbk_fdmt::fdmt_fused_kernel<<<(unsigned)(ntiles * fa.nnodes), dim3(32, pbk_fdmt::kFusedThreads / 32), f.smem, st>>>(fa);
+    const int n = wlen * P;
+    const unsigned gy = (unsigned)std::min<long long>((n + pbk_fdmt::kPassFloats - 1) / pbk_fdmt::kPassFloats, 65535);
+    int cur = 0;
+    for (int l = f.k + 1; l <= kmax; ++l) {
+      pbk_fdmt::PassArgs pa{};
+      pa.src = f.buf[cur];
+      pa.dst = f.buf[cur ^ 1];
+      pa.ent = ents + f.ent_off[l];
+      pa.stride = f.stride;
+      pa.n = n;
+      pa.P = P;
+      pbk_fdmt::fdmt_pass_kernel<<<dim3((unsigned)t.row0[l].back(), gy), pbk_fdmt::kThreads, 0, st>>>(pa);
+      cur ^= 1;
+    }
+    pbk_fdmt::LastArgs la{};
+    la.src = f.buf[cur];
+    la.out = reinterpret_cast<float*>(d_out);
+    la.ent = ents + f.last_off;
+    la.stride = f.stride;
+    la.rows = t.rows;
+    la.base = t.t_lo + ja - ws;
+    la.ja = ja;
+    la.n = (int)(jn * P);
+    la.P = P;
+    const unsigned ly = (unsigned)std::min<long long>((la.n + pbk_fdmt::kThreads - 1) / pbk_fdmt::kThreads, 65535);
+    pbk_fdmt::fdmt_last_kernel<<<dim3((unsigned)pl->ndm, ly), pbk_fdmt::kThreads, 0, st>>>(la);
+  }
+  cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess) return fail(PBK_ERR_CUDA, "FDMT launch: %s", cudaGetErrorString(e));
+  return PBK_OK;
+}
+
+extern "C" int pbk_fdmt_exec_host(pbk_plan* pl, const void* in, void* out) {
+  if (!pl || pl->kind != PLAN_FDMT) return fail(PBK_ERR_INVALID, "not an FDMT plan");
+  if (!in || !out) return fail(PBK_ERR_INVALID, "NULL data pointer");
+  if (pl->fdmt->t.rows == 0) return PBK_OK;
+  std::lock_guard<std::mutex> lock(pl->mu);
+  CUDA_TRY(cudaSetDevice(pl->device));
+  int rc;
+  if ((rc = ensure_buf(&pl->h_din, pl->in_bytes)) != PBK_OK) return rc;
+  if ((rc = ensure_buf(&pl->h_dout, pl->out_bytes)) != PBK_OK) return rc;
+  cudaStream_t st = cudaStreamPerThread;
+  CUDA_TRY(host_to_device(pl->h_din, in, pl->in_bytes, st));
+  if ((rc = pbk_fdmt_exec_device(pl, pl->h_din, pl->h_dout, st)) != PBK_OK) return rc;
   CUDA_TRY(device_to_host(out, pl->h_dout, pl->out_bytes, st));
   return PBK_OK;
 }

@@ -24,7 +24,7 @@ from .device import DeviceArray
 
 __all__ = ["default_device", "dedisperse", "chirp", "detect", "shift_channels", "phase_ramp", "mix", "analytic_decimate", "stokes", "pol_basis",
            "downsample", "fft", "stft", "istft", "stft_detect", "stft_fold", "fold",
-           "dedisperse_fold", "dedisperse_trials", "incoherent_trials", "boxcar_search", "spectral_kurtosis",
+           "dedisperse_fold", "dedisperse_trials", "incoherent_trials", "fdmt", "boxcar_search", "spectral_kurtosis",
            "predict_phase",
            "clear_plan_cache",
            "pinned_results"]
@@ -857,6 +857,49 @@ def spectral_kurtosis(data, m, *, lo, hi, nd=1.0, zap=None, raw=None, device=Non
                                               L.ptr(sk) if nblk else None,
                                               L.ptr(mask) if nblk else None, 0, dev, None))
     return sk, mask, out
+
+
+def fdmt(data, f_lo_hz, f_hi_hz, max_delay, *, d_min=0, ref_freq_hz=None, max_workspace_bytes=0,
+         device=None):
+    """Fast dispersion measure transform of a filterbank at every delay trial
+    ``d_min..max_delay`` (pbk_fdmt_plan_create; definition in DESIGN.md 5.4h).
+
+    ``data`` is (nsamp, nchan, ...) float32, numpy or DeviceArray, channels ascending over
+    ``[f_lo_hz, f_hi_hz)``; trial d has d samples of sweep from ``f_hi_hz`` down to ``f_lo_hz``.
+    Returns ``(out, t_lo)``: ``out`` is (ndm, rows, ...) float32 on the input's side of the bus,
+    and its row j arrives at ``ref_freq_hz`` (default: the band's centre) ``t_lo + j`` samples
+    after the input starts.  Plans are cached by their arguments."""
+    shape = tuple(data.shape)
+    if len(shape) < 2:
+        raise ValueError("fdmt takes (nsamp, nchan, ...) data")
+    if np.dtype(data.dtype) != np.float32:
+        raise TypeError(f"fdmt takes float32 data, got {np.dtype(data.dtype)}")
+    nsamp, nchan = shape[0], shape[1]
+    npol = int(np.prod(shape[2:], dtype=np.int64)) if len(shape) > 2 else 1
+    f_lo, f_hi = float(f_lo_hz), float(f_hi_hz)
+    ref = 0.5 * (f_lo + f_hi) if ref_freq_hz is None else float(ref_freq_hz)
+    dev = data.device if _is_dev(data) else (default_device() if device is None else device)
+    key = ("fdmt", nsamp, nchan, npol, f_lo, f_hi, ref, int(max_delay), int(d_min),
+           int(max_workspace_bytes), dev)
+    ctx = _use_plan(key, lambda: L.FdmtPlan(nsamp=nsamp, nchan=nchan, npol=npol, f_lo_hz=f_lo,
+                                            f_hi_hz=f_hi, ref_freq_hz=ref, max_delay=max_delay,
+                                            d_min=d_min, max_workspace_bytes=max_workspace_bytes,
+                                            device=dev))
+    with ctx as plan:
+        out_shape = (plan.ndm, plan.rows) + shape[2:]
+        if _is_dev(data):
+            x = data.contiguous()
+            out = DeviceArray.empty(out_shape, np.float32, x.device)
+            if plan.rows:                  # an empty tensor may have a NULL pointer
+                with ctx.lock:
+                    plan.exec_device(x.ptr, out.ptr, _stream())
+            return out, plan.t_lo
+        x = np.ascontiguousarray(data)
+        out = _result(out_shape, np.float32)
+        if plan.rows:
+            with ctx.lock:
+                plan.exec_host(x, out)
+        return out, plan.t_lo
 
 
 def phase_ramp(data, shift_samples=None, zero_lo=None, zero_hi=None, device=None):

@@ -6,6 +6,7 @@ sm_100a passes in libpbk (the chirp is generated in registers and never stored).
 """
 
 import math
+from typing import NamedTuple
 
 import numpy as np
 
@@ -17,6 +18,7 @@ from ..core import BasebandSignal, IntensitySignal, RadioSignal
 
 __all__ = ["DispersionMeasure", "DM", "coherent_dedispersion", "incoherent_dedispersion",
            "dedisperse_detect", "dedisperse_trials", "incoherent_dedispersion_trials",
+           "fdmt_dedispersion_trials", "FDMTTrials",
            "overlap_save_dedispersion"]
 
 #: s MHz^2 cm^3 / pc -- dedispersion.py:30
@@ -354,6 +356,61 @@ def incoherent_dedispersion_trials(z, DMs, /, *, ref_freq=None):
     if z.start_time is not None:
         kw["start_time"] = z.start_time + t_lo / z.sample_rate
     return [IntensitySignal.like(z, x[k], **kw) for k in range(len(DMs))]
+
+
+class FDMTTrials(NamedTuple):
+    """Result of :func:`fdmt_dedispersion_trials`: ``DMs`` (float64, pc / cm^3) and one
+    ``IntensitySignal`` per DM in ``trials``."""
+    DMs: np.ndarray
+    trials: list
+
+
+def fdmt_dedispersion_trials(z, DM_max, /, *, DM_min=0, ref_freq=None):
+    """Dedisperse a filterbank at every DM step from ``DM_min`` to ``DM_max`` with the fast
+    dispersion measure transform (FDMT) on the GPU (builder-defined; kernels.fdmt, DESIGN.md
+    5.4h).
+
+    The band is ``[f_lo, f_hi) = [z.min_freq, z.max_freq)`` in ``z.nchan`` equal channels,
+    whatever ``freq_align``.  With ``u = DispersionMeasure(1).sample_delay(f_lo, f_hi,
+    sample_rate)`` the band's sweep per unit DM in samples, the trials are the integer sweeps
+    ``d = ceil(DM_min * u) .. ceil(DM_max * u)`` and ``DMs[k] = d_k / u``.  Trial k sums exactly
+    ``d_k + nchan`` samples of every column along its track.
+
+    Returns ``FDMTTrials(DMs, trials)``: ``trials[k]`` is an ``IntensitySignal`` of shape
+    ``(rows, 1, ...)``, shaped and annotated as :func:`incoherent_dedispersion_trials` makes them
+    (the band as one channel at ``center_freq``, ``start_time`` shifted by ``t_lo`` samples), and
+    its row j arrives at ``ref_freq`` (default ``center_freq``).  The trials are views of one
+    stacked array on ``z``'s side of the bus.  ``z`` must hold float32 numpy or DeviceArray data;
+    other dtypes and dask arrays raise ``TypeError``.
+    """
+    if not isinstance(z, RadioSignal):
+        raise TypeError("Signal must be a RadioSignal object.")
+    if _dask.is_dask(z.data):
+        raise TypeError("fdmt_dedispersion_trials takes numpy or DeviceArray data (a dask "
+                        "array: compute it first)")
+    if np.dtype(z.dtype) != np.float32:
+        raise TypeError(f"fdmt_dedispersion_trials needs float32 data, got {z.dtype} "
+                        "(complex and float64 signals are not supported)")
+    f_lo, f_hi = _hz(z.min_freq), _hz(z.max_freq)
+    per_dm = DispersionMeasure(1).sample_delay(z.min_freq, z.max_freq, z.sample_rate)
+    dm_max, dm_min = _as_dm(DM_max).value, _as_dm(DM_min).value
+    if not 0 <= dm_min <= dm_max:
+        raise ValueError("need 0 <= DM_min <= DM_max")
+    D = int(np.ceil(dm_max * per_dm))
+    d_min = int(np.ceil(dm_min * per_dm))
+    ref = _hz(z.center_freq if ref_freq is None else ref_freq)
+    x, t_lo = kernels.fdmt(z.data, f_lo, f_hi, D, d_min=d_min, ref_freq_hz=ref)
+    DMs = np.arange(d_min, D + 1, dtype=np.float64) / per_dm
+    trailing = tuple(z.shape[2:])
+    shape = (len(DMs), x.shape[1], 1) + trailing
+    if isinstance(x, kernels.DeviceArray):
+        x = kernels.DeviceArray(x.tensor.reshape(shape))
+    else:
+        x = x.reshape(shape)
+    kw = {"chan_bw": z.chan_bw * z.nchan, "center_freq": z.center_freq, "freq_align": "center"}
+    if z.start_time is not None:
+        kw["start_time"] = z.start_time + t_lo / z.sample_rate
+    return FDMTTrials(DMs, [IntensitySignal.like(z, x[k], **kw) for k in range(len(DMs))])
 
 
 def _block_schedule(nsamp, block_len, start, stop, downsample):
